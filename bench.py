@@ -18,6 +18,9 @@ rank's shard of the clip (frames resident in HBM):
 
 `--impl reference` times the reference's CPU path (the oracle; the C++ binary cannot be built
 offline: no OpenCV SDK) on the same config and prints the same JSON shape.
+
+`--dump-outputs DIR` writes the stabilized frames of the last timed step (see `dump_outputs`).  The clip is
+generated from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -123,6 +126,33 @@ def ncu_traffic(stage, frames_per_launch):
         return None if v is None else float(v) * frames_per_launch / float(t.get("frames_per_launch", 256))
     except Exception:
         return None
+
+
+DUMP_BYTES = 64 * 10 ** 6        # --dump-outputs: all files together
+DUMP_PIXELS = 4096               # pixels per call in frames_sampled.npy
+DUMP_SEED = 0
+
+
+def sample_pixels(h, w, n):
+    """Flat indices (y * w + x) of the n pixels of frames_sampled.npy: drawn once with DUMP_SEED, sorted."""
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(h * w, n, replace=False))
+
+
+def dump_outputs(directory, out):
+    """Writes what the timed path returned in its last step, `out` = the uint8 [ncalls, H, W, 3] device tensor of
+    stabilized frames, as float32 .npy files of DUMP_BYTES at most:
+      frame_last.npy      [H, W, 3]              the last call's frame, complete
+      frames_sampled.npy  [ncalls, n, 3]         every call's frame at the n pixels sample_pixels(H, W, n) picks,
+                                                 the same pixels in every call (n = DUMP_PIXELS unless the budget is less)"""
+    import torch
+    ncalls, h, w, _ = out.shape
+    last = out[-1].cpu().numpy().astype(np.float32)
+    n = min(DUMP_PIXELS, h * w, (DUMP_BYTES - last.nbytes - 1024) // (ncalls * 3 * 4))
+    idx = torch.from_numpy(sample_pixels(h, w, n)).to(out.device)
+    sampled = out.reshape(ncalls, h * w, 3).index_select(1, idx).cpu().numpy().astype(np.float32)
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "frame_last.npy"), last)
+    np.save(os.path.join(directory, "frames_sampled.npy"), sampled)
 
 
 class ClockSampler:
@@ -339,6 +369,8 @@ def run_ours(args):
     barrier()
     ms = e0.elapsed_time(e1)
     launches = lib.vstab_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out[:ncalls])
     # one more pass outside the timed region, with the per-call checksums (the warp's checksum variant is a few % slower)
     last_run.update(off.run(n_total, mode, LOCK_CALL, device_frames=frames, device_halo=halo, device_out=out))
     stages = off.stage_times()
@@ -853,7 +885,13 @@ def main():
     ap.add_argument("--no-c5-probe", action="store_true")
     ap.add_argument("--parity-frames", type=int, default=160, help="frames of the bounded parity run against the oracle")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the stabilized frames of the last timed step (rank 0's "
+                                                          "calls) to DIR as float32 .npy files, 64 MB at most")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c2"):
+        ap.error("--dump-outputs writes the frames of the default workload's GPU path (--impl ours --workload c2)")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -50,6 +50,15 @@ struct ImageView {
     size_t step{0};
 };
 
+// A YUV 4:2:0 frame (NV12 / I420): base pointer and where its planes are (vstab_yuv_layout, e.g. from
+// vstab_yuv_layout_packed for ffmpeg rawvideo, or offsets/steps of an NVDEC surface).
+struct YuvView {
+    uint8_t* data{nullptr};
+    vstab_yuv_layout layout{};
+    int rows{0};
+    int cols{0};
+};
+
 // Owning image returned by stabilizeFrame (the reference returns a fresh cv::Mat).
 struct Image {
     std::vector<uint8_t> pixels;
@@ -85,6 +94,13 @@ public:
     // Same, into a caller-owned buffer (e.g. pinned memory from vstab_host_alloc).
     void stabilizeFrame(const ImageView& frame, const ImageView& out) {
         check(vstab_stabilize_frame(h_, frame.data, frame.rows, frame.cols, frame.step, out.data, out.step));
+    }
+
+    // stabilizeFrame on YUV frames: `in` is converted to BGR on the device, the BGR output to `out`'s format before it leaves
+    // (out == BGR2YUV_I420(stabilizeFrame(YUV2BGR(in))), see vstab.h).  Throws like stabilizeFrame.
+    void stabilizeFrameYuv(const YuvView& in, const YuvView& out) {
+        if (out.rows != in.rows || out.cols != in.cols) throw std::invalid_argument("stabilizeFrameYuv: output size differs from input size");
+        check(vstab_stabilize_frame_yuv(h_, in.data, &in.layout, in.rows, in.cols, out.data, &out.layout));
     }
 
 #ifdef VSTAB_WITH_OPENCV

@@ -87,6 +87,35 @@ vstab_status vstab_stabilize_frame_device(vstab_t* s, const uint8_t* d_bgr, int 
                                           size_t step, uint8_t* d_out_bgr, size_t out_step);
 vstab_status vstab_synchronize(vstab_t* s);
 
+/* ---- YUV 4:2:0 frames (what video decoders produce and encoders take) ---------------------------------------------
+ * NV12 (NVDEC's output: a Y plane and one interleaved U,V plane) and I420 (ffmpeg's yuv420p: Y, U, V planes), 8-bit,
+ * BT.601 limited range.  The stabilizer stores and processes BGR either way: a YUV input frame is converted on the device
+ * when it arrives, a BGR output frame is converted on the device before it leaves, each conversion exactly OpenCV's
+ * (cvtColor COLOR_YUV2BGR_NV12 / _I420 and COLOR_BGR2YUV_I420; NV12 output = I420's chroma interleaved U,V).  So for every
+ * call c:  out_yuv[c] == BGR2YUV_I420(stabilizeFrame(YUV2BGR(in_yuv))[c]) -- call 0 returns the converted copy of its
+ * input converted back, not the caller's input bytes.  Only 1.5 bytes per pixel cross the host link instead of 3.
+ * rows and cols must be even. */
+typedef enum vstab_pixel_format { VSTAB_PIX_NV12 = 1, VSTAB_PIX_I420 = 2 } vstab_pixel_format;
+/* plane k of a frame starts at base + offset[k] with rows step[k] bytes apart: k = 0 Y (rows x cols), NV12: k = 1 U,V
+ * interleaved (rows/2 x cols bytes), k = 2 unused; I420: k = 1 U, k = 2 V (rows/2 x cols/2 each).  Covers ffmpeg's
+ * data[] / linesize[] within one allocation and NVDEC's pitched surface with the chroma plane at pitch * rows. */
+typedef struct vstab_yuv_layout {
+    int format;                     /* vstab_pixel_format */
+    size_t offset[3];
+    size_t step[3];
+} vstab_yuv_layout;
+/* The tight rawvideo layout of a rows x cols frame (what `ffmpeg -f rawvideo -pix_fmt nv12|yuv420p` reads and writes)
+ * into *out; returns the frame's size in bytes, or 0 for an unknown format, odd or non-positive sizes.  Host only. */
+size_t vstab_yuv_layout_packed(int format, int rows, int cols, vstab_yuv_layout* out);
+/* vstab_stabilize_frame / _device with YUV frames: `in` / `out` are frame base pointers, the layouts say where their planes
+ * are (input and output formats are independent).  Same synchronicity as the BGR pair; BGR and YUV calls may be mixed on one
+ * instance (the window holds BGR frames either way).  VSTAB_ERR_INVALID_ARGUMENT: NULL pointers or layouts, an unknown
+ * format, odd rows or cols, a step below its plane's row bytes; the frame size checks are those of the BGR calls. */
+vstab_status vstab_stabilize_frame_yuv(vstab_t* s, const uint8_t* in, const vstab_yuv_layout* in_layout, int rows, int cols,
+                                       uint8_t* out, const vstab_yuv_layout* out_layout);
+vstab_status vstab_stabilize_frame_yuv_device(vstab_t* s, const uint8_t* d_in, const vstab_yuv_layout* in_layout, int rows,
+                                              int cols, uint8_t* d_out, const vstab_yuv_layout* out_layout);
+
 /* static bool Stabilizer::decomposeHomography(H, params_out, rot_center)
  * include/stabilizer.hpp:227, src/stabilizer.cpp:1435-1533.
  * returns 1 (true) / 0 (false: degenerate, out untouched) / -1 (bad argument,
@@ -291,6 +320,14 @@ typedef struct vstab_offline_report {   /* device time per phase on this rank, m
     long frames, calls;
 } vstab_offline_report;
 vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offline_cfg* cfg, vstab_offline_report* report /* or NULL */);
+/* YUV 4:2:0 frames for vstab_offline_run_host and vstab_offline_run (see vstab_yuv_layout above; NULL = BGR, the default):
+ * `in` describes every source frame (HOST and DEVICE sources; the simulator source ignores it), `out` every output frame
+ * (`out` / `host_out` / `d_out`).  While a layout is set the corresponding `step` / `out_step` arguments are ignored; frame
+ * strides still apply and must cover the layout's planes.  Frames are converted on the device when they arrive and before
+ * they leave; the clip is processed as BGR, so per-call checksums are those of the BGR outputs.  The device-pointer
+ * building blocks (estimate, render, register, reference_capture) take BGR only.  VSTAB_ERR_INVALID_ARGUMENT for a
+ * layout that does not fit the instance's frame size. */
+vstab_status vstab_offline_set_yuv(vstab_offline_t* o, const vstab_yuv_layout* in, const vstab_yuv_layout* out);
 /* the checksum the warp kernel accumulates, of a host frame (tests) */
 uint64_t vstab_frame_checksum(const uint8_t* bgr, int rows, int cols, size_t step);
 
@@ -321,6 +358,12 @@ vstab_status vstab_k_warp(int device, const uint8_t* bgr, int rows, int cols, si
  * darkened, blurred gray background; both images rows x cols BGR with the same step. */
 vstab_status vstab_k_copy_feathered(int device, const uint8_t* fg, const uint8_t* bg, int rows, int cols, size_t step,
                                     const double H[9], uint8_t* out, size_t out_step);
+/* K15 alone: cvtColor(YUV2BGR_NV12 / _I420) and cvtColor(BGR2YUV_I420) (+ NV12 interleave) of one frame.  The YUV side is a
+ * frame base pointer and its layout; bgr_to_yuv writes only the bytes of the layout's planes. */
+vstab_status vstab_k_yuv_to_bgr(int device, const uint8_t* yuv, const vstab_yuv_layout* layout, int rows, int cols,
+                                uint8_t* bgr, size_t step);
+vstab_status vstab_k_bgr_to_yuv(int device, const uint8_t* bgr, int rows, int cols, size_t step, uint8_t* yuv,
+                                const vstab_yuv_layout* layout);
 
 /* ORB / SIFT registration path (src/stabilizer.cpp:448-477 preprocessing, :483-491 + :605-606 ORB
  * detectAndCompute, :647-673 Hamming 2-NN + ratio test).  kps_out: 6 floats per keypoint

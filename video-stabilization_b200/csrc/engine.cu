@@ -218,6 +218,102 @@ bool device_ok(int device, std::string& err) {
     return true;
 }
 
+// ---- YUV 4:2:0 frames (vstab_yuv_layout): plane geometry, checks, device staging, plane copies -------------------------
+inline int yuv_nplanes(int fmt) { return fmt == VSTAB_PIX_NV12 ? 2 : 3; }
+inline size_t yuv_row_bytes(int fmt, int k, int cols) { return k == 0 || fmt == VSTAB_PIX_NV12 ? (size_t)cols : (size_t)cols / 2; }
+inline int yuv_rows(int k, int rows) { return k == 0 ? rows : rows / 2; }
+
+// end of the last plane byte of a frame laid out as *L, or 0 (and `err`) when the layout does not describe a rows x cols frame
+size_t yuv_extent(const vstab_yuv_layout* L, int rows, int cols, std::string& err) {
+    if (!L) { err = "null YUV layout"; return 0; }
+    if (L->format != VSTAB_PIX_NV12 && L->format != VSTAB_PIX_I420) { err = "unknown pixel format " + std::to_string(L->format); return 0; }
+    if (rows < 2 || cols < 2 || (rows & 1) || (cols & 1)) {
+        err = "YUV 4:2:0 frames need even rows and cols. Rows: " + std::to_string(rows) + ", Cols: " + std::to_string(cols);
+        return 0;
+    }
+    size_t end = 0;
+    for (int k = 0; k < yuv_nplanes(L->format); ++k) {
+        const size_t rb = yuv_row_bytes(L->format, k, cols);
+        if (L->step[k] < rb) { err = "row step of YUV plane " + std::to_string(k) + " smaller than its " + std::to_string(rb) + " bytes"; return 0; }
+        const size_t e = L->offset[k] + L->step[k] * (size_t)(yuv_rows(k, rows) - 1) + rb;
+        if (e > end) end = e;
+    }
+    return end;
+}
+
+size_t yuv_packed(int fmt, int rows, int cols, vstab_yuv_layout* out) {
+    const size_t y = (size_t)rows * cols, c = y / 4;
+    *out = vstab_yuv_layout{};
+    out->format = fmt;
+    out->step[0] = (size_t)cols;
+    out->offset[1] = y;
+    if (fmt == VSTAB_PIX_NV12) {
+        out->step[1] = (size_t)cols;
+    } else {
+        out->step[1] = out->step[2] = (size_t)cols / 2;
+        out->offset[2] = y + c;
+    }
+    return y + 2 * c;
+}
+
+// Layout of the library's own YUV staging buffers: the packed one when cols % 8 == 0 (then every plane and frame offset is a
+// multiple of 8 and the conversions take their word paths; 1080p, 4K), otherwise rows padded to 16 bytes.
+vstab_yuv_layout yuv_staging_layout(int fmt, int rows, int cols, size_t* frame_bytes) {
+    vstab_yuv_layout L;
+    size_t bytes = yuv_packed(fmt, rows, cols, &L);
+    if (cols % 8) {
+        size_t off = 0;
+        for (int k = 0; k < yuv_nplanes(fmt); ++k) {
+            L.offset[k] = off;
+            L.step[k] = align_up(yuv_row_bytes(fmt, k, cols), 16);
+            off += L.step[k] * (size_t)yuv_rows(k, rows);
+        }
+        bytes = off;
+    }
+    *frame_bytes = bytes;
+    return L;
+}
+
+size_t yuv_staging_bytes(int rows, int cols) {            // one frame, either format
+    size_t a = 0, b = 0;
+    yuv_staging_layout(VSTAB_PIX_NV12, rows, cols, &a);
+    yuv_staging_layout(VSTAB_PIX_I420, rows, cols, &b);
+    return a > b ? a : b;
+}
+
+YuvPlanes yuv_planes_of(const vstab_yuv_layout& L) {
+    YuvPlanes p{};
+    p.off_y = L.offset[0]; p.step_y = L.step[0];
+    p.off_u = L.offset[1]; p.step_u = L.step[1];
+    if (L.format == VSTAB_PIX_NV12) { p.off_v = L.offset[1] + 1; p.step_v = L.step[1]; p.cstep = 2; }
+    else { p.off_v = L.offset[2]; p.step_v = L.step[2]; p.cstep = 1; }
+    return p;
+}
+
+bool same_planes(const vstab_yuv_layout& a, const vstab_yuv_layout& b) {
+    if (a.format != b.format) return false;
+    for (int k = 0; k < yuv_nplanes(a.format); ++k)
+        if (a.offset[k] != b.offset[k] || a.step[k] != b.step[k]) return false;
+    return true;
+}
+
+// n frames between two layouts of the same format, one cudaMemcpy2DAsync per plane and frame -- or ONE copy when both sides
+// are tightly packed rawvideo (no bytes between planes or frames that the copy could clobber)
+cudaError_t yuv_copy(uint8_t* dst, const vstab_yuv_layout& dl, size_t dst_fs, const uint8_t* src, const vstab_yuv_layout& sl,
+                     size_t src_fs, long n, int rows, int cols, cudaMemcpyKind kind, cudaStream_t q) {
+    vstab_yuv_layout P;
+    const size_t packed = yuv_packed(dl.format, rows, cols, &P);
+    if (same_planes(dl, P) && same_planes(sl, P) && (n == 1 || (dst_fs == packed && src_fs == packed)))
+        return cudaMemcpyAsync(dst, src, packed * (size_t)n, kind, q);
+    for (long i = 0; i < n; ++i)
+        for (int k = 0; k < yuv_nplanes(dl.format); ++k) {
+            const cudaError_t e = cudaMemcpy2DAsync(dst + (size_t)i * dst_fs + dl.offset[k], dl.step[k], src + (size_t)i * src_fs + sl.offset[k],
+                                                    sl.step[k], yuv_row_bytes(dl.format, k, cols), yuv_rows(k, rows), kind, q);
+            if (e != cudaSuccess) return e;
+        }
+    return cudaSuccess;
+}
+
 }  // namespace
 
 // =====================================================================================
@@ -282,6 +378,9 @@ struct vstab {
     bool trail = false;                     // copyFeathered branch of stabilizeFrame (:1303-1307)
     bool partial_fix = false;               // TRANSLATION_/ROTATION_LOCK fed with the accumulated lock (hpp:23 @todo)
     DevBuf trail_bg, trail_ws;              // trail_background_ (:129) and K14 scratch
+    // YUV calls with host buffers: the input planes are uploaded here (copy_stream) and converted into the ring, the
+    // presented BGR frame is converted here (out_stream) and downloaded.  One frame each: every use is ordered by its stream.
+    DevBuf yuv_in, yuv_out;
     DevBuf feat_ws, feat_gray, nn_x, nn_y, ref_kps, ref_desc, cur_kps, cur_desc, orb_counts, m_idx, m_d0, m_d1, m_good,
         m_ref, m_cur, m_status, lock_fit, lock_h, lock_tap;
     std::string err;
@@ -557,14 +656,52 @@ static vstab_status stream_output(vstab* s, long n, uint8_t* d_out, size_t out_p
     return VSTAB_OK;
 }
 
-// One stabilizeFrame call; `kind` selects how frame pixels move (host<->device or device<->device).
+// YUV input frame -> BGR ring slot on q: device frames are converted where they are, host frames uploaded first
+static vstab_status stream_yuv_in(vstab* s, const uint8_t* in, const vstab_yuv_layout& L, bool host, uint8_t* slot, cudaStream_t q) {
+    auto set_err = [&](const std::string& e) { s->err = e; };
+    Geometry& g = s->g;
+    if (!host) {
+        launch_yuv420_to_bgr(in, yuv_planes_of(L), 0, 1, g.rows, g.cols, slot, g.pitch, 0, q);
+    } else {
+        size_t fb = 0;
+        const vstab_yuv_layout S = yuv_staging_layout(L.format, g.rows, g.cols, &fb);
+        if (!s->yuv_in.p) CK(s->yuv_in.alloc(yuv_staging_bytes(g.rows, g.cols)));
+        CK(yuv_copy(s->yuv_in.as<uint8_t>(), S, fb, in, L, 0, 1, g.rows, g.cols, cudaMemcpyHostToDevice, q));
+        launch_yuv420_to_bgr(s->yuv_in.as<uint8_t>(), yuv_planes_of(S), fb, 1, g.rows, g.cols, slot, g.pitch, 0, q);
+    }
+    CK(cudaGetLastError());
+    return VSTAB_OK;
+}
+
+// presented BGR frame -> YUV output frame on out_stream: into device memory directly, or through staging to host memory
+static vstab_status stream_yuv_out(vstab* s, const uint8_t* bgr, size_t pitch, uint8_t* out, const vstab_yuv_layout& L, bool host) {
+    auto set_err = [&](const std::string& e) { s->err = e; };
+    Geometry& g = s->g;
+    cudaStream_t q = s->out_stream;
+    if (!host) {
+        launch_bgr_to_yuv420(bgr, pitch, 0, 1, g.rows, g.cols, out, yuv_planes_of(L), 0, q);
+    } else {
+        size_t fb = 0;
+        const vstab_yuv_layout S = yuv_staging_layout(L.format, g.rows, g.cols, &fb);
+        if (!s->yuv_out.p) CK(s->yuv_out.alloc(yuv_staging_bytes(g.rows, g.cols)));
+        launch_bgr_to_yuv420(bgr, pitch, 0, 1, g.rows, g.cols, s->yuv_out.as<uint8_t>(), yuv_planes_of(S), fb, q);
+        CK(yuv_copy(out, L, 0, s->yuv_out.as<uint8_t>(), S, fb, 1, g.rows, g.cols, cudaMemcpyDeviceToHost, q));
+    }
+    CK(cudaGetLastError());
+    return VSTAB_OK;
+}
+
+// One stabilizeFrame call; `kind` selects how frame pixels move (host<->device or device<->device).  in_yuv / out_yuv:
+// layouts of YUV frames (null: BGR with `step` / `out_step`).
 static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols, size_t step, uint8_t* out,
-                                size_t out_step, cudaMemcpyKind in_kind, cudaMemcpyKind out_kind, bool host_wait) {
+                                size_t out_step, cudaMemcpyKind in_kind, cudaMemcpyKind out_kind, bool host_wait,
+                                const vstab_yuv_layout* in_yuv = nullptr, const vstab_yuv_layout* out_yuv = nullptr) {
     auto set_err = [&](const std::string& e) { s->err = e; };
     Geometry& g = s->g;
     uint8_t* slot = s->ring.as<uint8_t>() + (size_t)(s->n % s->W) * g.frame_bytes;
     const size_t row_bytes = (size_t)cols * 3;
     const bool device_out = out_kind == cudaMemcpyDeviceToDevice;
+    const bool direct_out = device_out && !out_yuv;     // the warp writes the caller's BGR buffer itself
     const bool out_first = s->n > 0 && s->F >= 1;      // output chain does not need this call's transform
     static const bool trace = getenv("VSTAB_TRACE") != nullptr;
     static const bool prepare_ok = !(getenv("VSTAB_PREPARE") && atoi(getenv("VSTAB_PREPARE")) == 0);
@@ -587,10 +724,12 @@ static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols,
         return s->ev_fit[(c - lag) & 7];
     };
     auto output_into = [&](long c, int slot, cudaStream_t q, bool ahead) -> vstab_status {
-        uint8_t* dst = device_out ? out : s->dout_at(slot);
-        return stream_output(s, c, dst, device_out ? out_step : g.pitch, s->wp_at(slot), q, ahead);
+        uint8_t* dst = direct_out ? out : s->dout_at(slot);
+        return stream_output(s, c, dst, direct_out ? out_step : g.pitch, s->wp_at(slot), q, ahead);
     };
+    // YUV outputs are converted from whichever BGR half is presented (an output prepared one call ahead did not know the layout)
     auto copy_out = [&](int slot) -> vstab_status {
+        if (out_yuv) return stream_yuv_out(s, s->dout_at(slot), g.pitch, out, *out_yuv, !device_out);
         if (!device_out)
             CK(cudaMemcpy2DAsync(out, out_step, s->dout_at(slot), g.pitch, row_bytes, rows, out_kind, s->out_stream));
         return VSTAB_OK;
@@ -600,7 +739,7 @@ static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols,
     bool in_call_chain = false;                                               // ev_chain: that chain's lock state is final
     if (out_first) {
         const long p = s->n - (long)s->F > 0 ? s->n - (long)s->F : 0;
-        if (s->pre_valid && s->pre_call == s->n && s->pre_epoch == s->epoch && !device_out) {
+        if (s->pre_valid && s->pre_call == s->n && s->pre_epoch == s->epoch && !direct_out) {
             s->out_slot ^= 1;                                          // prepared during the previous call
             s->last_presented = p;
             if (s->mode == VSTAB_ACCUMULATED_FULL_LOCK || (s->partial_fix && (s->mode == VSTAB_TRANSLATION_LOCK || s->mode == VSTAB_ROTATION_LOCK))) {
@@ -627,7 +766,12 @@ static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols,
     cudaStream_t up = s->copy_stream;
     if (s->n > 0) CK(cudaStreamWaitEvent(up, s->ev_out, 0));
     s->mark(0, up);
-    CK(cudaMemcpy2DAsync(slot, g.pitch, in, step, row_bytes, rows, in_kind, up));
+    if (in_yuv) {
+        vstab_status sy = stream_yuv_in(s, in, *in_yuv, in_kind == cudaMemcpyHostToDevice, slot, up);
+        if (sy != VSTAB_OK) return sy;
+    } else {
+        CK(cudaMemcpy2DAsync(slot, g.pitch, in, step, row_bytes, rows, in_kind, up));
+    }
     s->mark(1, up);
     CK(cudaEventRecord(s->ev_in, up));
     vstab_status st = stream_estimate(s);
@@ -636,7 +780,12 @@ static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols,
         if (s->n == 0) {
             // call 0 returns the input frame itself (:1181)
             CK(cudaStreamWaitEvent(s->out_stream, s->ev_in, 0));
-            CK(cudaMemcpy2DAsync(out, out_step, slot, g.pitch, row_bytes, rows, out_kind, s->out_stream));
+            if (out_yuv) {
+                st = stream_yuv_out(s, slot, g.pitch, out, *out_yuv, !device_out);
+                if (st != VSTAB_OK) return st;
+            } else {
+                CK(cudaMemcpy2DAsync(out, out_step, slot, g.pitch, row_bytes, rows, out_kind, s->out_stream));
+            }
             s->last_presented = 0;
         } else {
             CK(cudaStreamWaitEvent(s->out_stream, s->ev_fit[s->n & 7], 0));   // future == 0: needs T[n] of this call
@@ -878,6 +1027,40 @@ vstab_status vstab_stabilize_frame_device(vstab_t* s, const uint8_t* d_bgr, int 
                        cudaMemcpyDeviceToDevice, false);
 }
 
+size_t vstab_yuv_layout_packed(int format, int rows, int cols, vstab_yuv_layout* out) {
+    std::string err;
+    vstab_yuv_layout L;
+    if (!out || rows <= 0 || cols <= 0 || (format != VSTAB_PIX_NV12 && format != VSTAB_PIX_I420)) return 0;
+    const size_t bytes = yuv_packed(format, rows, cols, &L);
+    if (!yuv_extent(&L, rows, cols, err)) return 0;             // odd sizes
+    *out = L;
+    return bytes;
+}
+
+static vstab_status stream_yuv_call(vstab_t* s, const uint8_t* in, const vstab_yuv_layout* in_layout, int rows, int cols,
+                                    uint8_t* out, const vstab_yuv_layout* out_layout, bool device) {
+    if (!s) return VSTAB_ERR_INVALID_ARGUMENT;
+    vstab_status st = stream_check_args(s, in, rows, cols, (size_t)cols * 3, out, (size_t)cols * 3);
+    if (st != VSTAB_OK) return st;
+    if (!yuv_extent(in_layout, rows, cols, s->err) || !yuv_extent(out_layout, rows, cols, s->err)) return VSTAB_ERR_INVALID_ARGUMENT;
+    auto set_err = [&](const std::string& e) { s->err = e; };
+    CK(cudaSetDevice(s->device));
+    if (!s->inited) { st = stream_init(s, rows, cols); if (st != VSTAB_OK) return st; }
+    const cudaMemcpyKind in_kind = device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+    const cudaMemcpyKind out_kind = device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    return stream_call(s, in, rows, cols, 0, out, 0, in_kind, out_kind, !device, in_layout, out_layout);
+}
+
+vstab_status vstab_stabilize_frame_yuv(vstab_t* s, const uint8_t* in, const vstab_yuv_layout* in_layout, int rows, int cols,
+                                       uint8_t* out, const vstab_yuv_layout* out_layout) {
+    return stream_yuv_call(s, in, in_layout, rows, cols, out, out_layout, false);
+}
+
+vstab_status vstab_stabilize_frame_yuv_device(vstab_t* s, const uint8_t* d_in, const vstab_yuv_layout* in_layout, int rows,
+                                              int cols, uint8_t* d_out, const vstab_yuv_layout* out_layout) {
+    return stream_yuv_call(s, d_in, in_layout, rows, cols, d_out, out_layout, true);
+}
+
 int vstab_decompose_homography(const double H[9], double cx, double cy, vstab_hparams* out) {
     if (!H || !out) return -1;
     HParams hp;
@@ -999,7 +1182,12 @@ struct vstab_offline {
     int rank = 0, world = 1;
     DevBuf job_chunk, job_out;
     size_t job_chunk_frames = 0;
-    std::vector<cudaEvent_t> host_events;         // vstab_offline_run_host: upload / render / download marks per chunk
+    std::vector<cudaEvent_t> host_events;         // vstab_offline_run_host: upload / render / download / conversion marks per chunk
+    // YUV frames of run_host / run (vstab_offline_set_yuv), and run_host's double-buffered staging (2 x max_batch frames each)
+    bool yuv_in = false, yuv_out = false;
+    vstab_yuv_layout yin{}, yout{};
+    DevBuf ystage_in, ystage_out;
+    size_t ystage_frames = 0;
     std::string err;
     void set_err(const std::string& e) { err = e; }
 };
@@ -1434,7 +1622,12 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
     auto set_err = [&](const std::string& e) { o->err = e; };
     Geometry& g = o->g;
     const size_t row_bytes = (size_t)g.cols * 3;
-    if (step < row_bytes || out_step < row_bytes) { o->err = "row step smaller than 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
+    const bool yin = o->yuv_in, yout = o->yuv_out;
+    if ((!yin && step < row_bytes) || (!yout && out_step < row_bytes)) { o->err = "row step smaller than 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
+    if ((yin && frame_stride < yuv_extent(&o->yin, g.rows, g.cols, o->err)) ||
+        (yout && out_frame_stride < yuv_extent(&o->yout, g.rows, g.cols, o->err))) {
+        o->err = "frame stride smaller than the extent of the YUV layout's planes"; return VSTAB_ERR_INVALID_ARGUMENT;
+    }
     CK(cudaSetDevice(o->device));
     if (!o->copy_in) CK(cudaStreamCreateWithFlags(&o->copy_in, cudaStreamNonBlocking));
     if (!o->copy_out) CK(cudaStreamCreateWithFlags(&o->copy_out, cudaStreamNonBlocking));
@@ -1449,10 +1642,21 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
     uint8_t* clip = o->clip.as<uint8_t>();
     double* T = o->clipT.as<double>();
     unsigned long long* sums = o->clipSums.as<unsigned long long>();
+    // YUV frames cross the link in staging buffers of two halves of B frames: upload(k) -> convert(k) into the clip, and
+    // render(k) -> convert(k) -> download(k), the halves alternating with k
+    size_t sfb_in = 0, sfb_out = 0;
+    const vstab_yuv_layout S_in = yin ? yuv_staging_layout(o->yin.format, g.rows, g.cols, &sfb_in) : vstab_yuv_layout{};
+    const vstab_yuv_layout S_out = yout ? yuv_staging_layout(o->yout.format, g.rows, g.cols, &sfb_out) : vstab_yuv_layout{};
+    if ((yin || yout) && o->ystage_frames < (size_t)B) {
+        const size_t sb = yuv_staging_bytes(g.rows, g.cols) * 2 * (size_t)B;
+        CK(o->ystage_in.alloc(sb));
+        CK(o->ystage_out.alloc(sb));
+        o->ystage_frames = (size_t)B;
+    }
     const long nchunks = (n_total + B - 1) / B;
     // per-chunk events live in the instance (created once, reused by every call, destroyed with it)
     std::vector<cudaEvent_t>& ev = o->host_events;
-    while (ev.size() < (size_t)nchunks * 3) {
+    while (ev.size() < (size_t)nchunks * 4) {
         cudaEvent_t e = nullptr;
         if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) { o->err = "cudaEventCreate failed"; return VSTAB_ERR_CUDA; }
         ev.push_back(e);
@@ -1461,6 +1665,7 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
     cudaEvent_t* ev_up = ev.data();                 // chunk k uploaded
     cudaEvent_t* ev_rd = ev.data() + nchunks;       // chunk k rendered
     cudaEvent_t* ev_dn = ev.data() + 2 * nchunks;   // chunk k downloaded
+    cudaEvent_t* ev_cv = ev.data() + 3 * nchunks;   // YUV input: chunk k converted (its staging half is free again)
     vstab_status st = VSTAB_OK;
     const bool in_contig = step == g.pitch && frame_stride == g.frame_bytes;
     const bool out_contig = out_step == g.pitch && out_frame_stride == g.frame_bytes;
@@ -1476,7 +1681,12 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
     for (long k = 0; k < nchunks && st == VSTAB_OK; ++k) {
         const long f0 = k * B, n = (n_total - f0 < B) ? n_total - f0 : B;
         const long seen = f0 + n;                                       // frames uploaded and estimated so far
-        if (in_contig) {            // tightly packed frames: one large copy per chunk
+        uint8_t* stg_in = o->ystage_in.as<uint8_t>() + (size_t)(k & 1) * B * sfb_in;
+        if (yin) {
+            if (k >= 2) cudaStreamWaitEvent(o->copy_in, ev_cv[k - 2], 0);
+            if (yuv_copy(stg_in, S_in, sfb_in, frames + (size_t)f0 * frame_stride, o->yin, frame_stride, n, g.rows, g.cols,
+                         cudaMemcpyHostToDevice, o->copy_in) != cudaSuccess) { o->err = "upload failed"; st = VSTAB_ERR_CUDA; }
+        } else if (in_contig) {     // tightly packed frames: one large copy per chunk
             if (cudaMemcpyAsync(clip + (size_t)f0 * g.frame_bytes, frames + (size_t)f0 * frame_stride, (size_t)n * g.frame_bytes,
                                 cudaMemcpyHostToDevice, o->copy_in) != cudaSuccess) { o->err = "upload failed"; st = VSTAB_ERR_CUDA; }
         } else {
@@ -1489,6 +1699,11 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
         if (st != VSTAB_OK) break;
         cudaEventRecord(ev_up[k], o->copy_in);
         cudaStreamWaitEvent(o->stream, ev_up[k], 0);
+        if (yin) {
+            launch_yuv420_to_bgr(stg_in, yuv_planes_of(S_in), sfb_in, (int)n, g.rows, g.cols, clip + (size_t)f0 * g.frame_bytes,
+                                 g.pitch, g.frame_bytes, o->stream);
+            cudaEventRecord(ev_cv[k], o->stream);
+        }
         st = vstab_offline_estimate(o, clip + (size_t)f0 * g.frame_bytes, g.frame_bytes, g.pitch, (int)n, f0,
                                     f0 > 0 ? clip + (size_t)(f0 - 1) * g.frame_bytes : nullptr, T + (size_t)f0 * 9,
                                     sums + (size_t)f0 * 3);
@@ -1502,9 +1717,15 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
         st = vstab_offline_render(o, clip, g.frame_bytes, g.pitch, 0, (int)n, f0, T, seen, rmode, lock_call, sums, ob,
                                   g.frame_bytes, g.pitch);
         if (st != VSTAB_OK) break;
+        uint8_t* stg_out = o->ystage_out.as<uint8_t>() + (size_t)(k & 1) * B * sfb_out;      // free: ev_dn[k - 2] above
+        if (yout)
+            launch_bgr_to_yuv420(ob, g.pitch, g.frame_bytes, (int)n, g.rows, g.cols, stg_out, yuv_planes_of(S_out), sfb_out, o->stream);
         cudaEventRecord(ev_rd[k], o->stream);
         cudaStreamWaitEvent(o->copy_out, ev_rd[k], 0);
-        if (out_contig) {
+        if (yout) {
+            if (yuv_copy(out + (size_t)f0 * out_frame_stride, o->yout, out_frame_stride, stg_out, S_out, sfb_out, n, g.rows, g.cols,
+                         cudaMemcpyDeviceToHost, o->copy_out) != cudaSuccess) { o->err = "download failed"; st = VSTAB_ERR_CUDA; }
+        } else if (out_contig) {
             if (cudaMemcpyAsync(out + (size_t)f0 * out_frame_stride, ob, (size_t)n * g.frame_bytes, cudaMemcpyDeviceToHost,
                                 o->copy_out) != cudaSuccess) { o->err = "download failed"; st = VSTAB_ERR_CUDA; }
         } else {
@@ -1522,6 +1743,16 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
     cleanup();
     if (st == VSTAB_OK && cudaGetLastError() != cudaSuccess) { o->err = "CUDA failure in vstab_offline_run_host"; st = VSTAB_ERR_CUDA; }
     return st;
+}
+
+extern "C" vstab_status vstab_offline_set_yuv(vstab_offline_t* o, const vstab_yuv_layout* in, const vstab_yuv_layout* out) {
+    if (!o) return VSTAB_ERR_INVALID_ARGUMENT;
+    if ((in && !yuv_extent(in, o->g.rows, o->g.cols, o->err)) || (out && !yuv_extent(out, o->g.rows, o->g.cols, o->err)))
+        return VSTAB_ERR_INVALID_ARGUMENT;
+    o->yuv_in = in != nullptr; o->yuv_out = out != nullptr;
+    o->yin = in ? *in : vstab_yuv_layout{};
+    o->yout = out ? *out : vstab_yuv_layout{};
+    return VSTAB_OK;
 }
 
 extern "C" void vstab_offline_set_timing(vstab_offline_t* o, int enable) { if (o) o->timer.enabled = enable != 0; }
@@ -1726,13 +1957,20 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     const long N = cfg->n_total;
     const int mode = cfg->mode;
     const bool sim = cfg->source == VSTAB_SRC_SIMULATOR;
-    const bool resident = cfg->source == VSTAB_SRC_DEVICE;
+    const bool dev_src = cfg->source == VSTAB_SRC_DEVICE;
+    const bool yin = o->yuv_in && !sim, yout = o->yuv_out;
+    // a YUV device shard is staged through the chunk ring like a host one (converted instead of copied)
+    const bool resident = dev_src && !yin;
     const bool feature_lock = mode == VSTAB_ORB_FULL_LOCK || mode == VSTAB_SIFT_FULL_LOCK;
     if (mode < 0 || mode > 5) { o->err = "Stabilizer: Invalid stabilization mode"; return VSTAB_ERR_INVALID_ARGUMENT; }
     if (sim && (!cfg->d_texture || !cfg->poses || cfg->tex_rows < 1 || cfg->tex_cols < 1)) { o->err = "simulator source needs d_texture and poses"; return VSTAB_ERR_INVALID_ARGUMENT; }
     const size_t row_bytes = (size_t)g.cols * 3;
-    if (!sim && (!cfg->host_frames || cfg->step < row_bytes)) { o->err = "host / device source needs frames with step >= 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
-    if ((cfg->host_out || cfg->d_out) && cfg->out_step < row_bytes) { o->err = "out_step smaller than 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
+    if (!sim && (!cfg->host_frames || (!yin && cfg->step < row_bytes))) { o->err = "host / device source needs frames with step >= 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
+    if ((cfg->host_out || cfg->d_out) && !yout && cfg->out_step < row_bytes) { o->err = "out_step smaller than 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
+    if ((yin && cfg->frame_stride < yuv_extent(&o->yin, g.rows, g.cols, o->err)) ||
+        (yout && (cfg->host_out || cfg->d_out) && cfg->out_frame_stride < yuv_extent(&o->yout, g.rows, g.cols, o->err))) {
+        o->err = "frame stride smaller than the extent of the YUV layout's planes"; return VSTAB_ERR_INVALID_ARGUMENT;
+    }
     if (cfg->host_out && cfg->d_out) { o->err = "give host_out or d_out, not both"; return VSTAB_ERR_INVALID_ARGUMENT; }
     if ((mode == VSTAB_ACCUMULATED_FULL_LOCK || feature_lock) && cfg->lock_call < (long)o->F) {
         o->err = "lock modes must be set at a call index >= future (SURVEY B.6)"; return VSTAB_ERR_STATE;
@@ -1762,7 +2000,7 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     const long ring_chunks = fused ? fp.ring_chunks : 1;
     const long ring_frames = ring_chunks * B;                       // + one slot for the halo frame of the first chunk
     DevBuf& chunk = o->job_chunk; DevBuf& outc = o->job_out;
-    if (!(resident && cfg->d_out) && o->job_chunk_frames < (size_t)ring_frames + 1) {
+    if (!(resident && cfg->d_out && !yout) && o->job_chunk_frames < (size_t)ring_frames + 1) {
         CK(chunk.alloc(g.frame_bytes * ((size_t)ring_frames + 1) + 64));
         CK(outc.alloc(g.frame_bytes * (size_t)B + 64));
         o->job_chunk_frames = (size_t)ring_frames + 1;
@@ -1777,6 +2015,14 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     CK(cudaMemsetAsync(checks.p, 0, sizeof(unsigned long long) * (size_t)(n_calls > 0 ? n_calls : 1), q));
     uint8_t* cb = chunk.as<uint8_t>();
     const size_t fb = g.frame_bytes;
+    // YUV: host frames are uploaded into a staging buffer of the stream that fetches them (q, and qs in the fused pass) and
+    // converted into the chunk slots; YUV outputs are converted from the BGR output chunk, into d_out or a download staging
+    size_t sfb_in = 0, sfb_out = 0;
+    const vstab_yuv_layout S_in = yin ? yuv_staging_layout(o->yin.format, g.rows, g.cols, &sfb_in) : vstab_yuv_layout{};
+    const vstab_yuv_layout S_out = yout ? yuv_staging_layout(o->yout.format, g.rows, g.cols, &sfb_out) : vstab_yuv_layout{};
+    DevBuf ystage_q, ystage_qs, ystage_o;
+    if (yin && !dev_src) { CK(ystage_q.alloc(sfb_in * (size_t)B)); CK(ystage_qs.alloc(sfb_in * (size_t)B)); }
+    if (yout && cfg->host_out) CK(ystage_o.alloc(sfb_out * (size_t)B));
     // resident shard: frame f of the clip lives at dframe(f); no staging
     auto dframe = [&](long f) -> const uint8_t* { return f == pl.first - 1 ? cfg->host_halo : cfg->host_frames + (size_t)(f - pl.first) * cfg->frame_stride; };
     const size_t src_fs = resident ? cfg->frame_stride : fb, src_step = resident ? cfg->step : g.pitch;
@@ -1800,6 +2046,23 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
         if (sim) {
             launch_render(cfg->d_texture, cfg->tex_rows, cfg->tex_cols, poses_d.as<RenderPose>() + f0, (int)n, g.cols, g.rows, cfg->focal,
                           cb + (size_t)slot * fb, g.pitch, fb, q, rays_d.as<double>(), tex4_d.as<unsigned>());
+        } else if (yin) {
+            if (f0 < pl.first - 1 || f0 + n > pl.last) { o->err = "internal: frame outside the rank's shard"; return VSTAB_ERR_STATE; }
+            for (long i = 0; i < n;) {
+                const long f = f0 + i;
+                const bool halo = f == pl.first - 1;
+                const long m = halo ? 1 : n - i;                    // the halo frame alone, then one contiguous run
+                const uint8_t* src = halo ? cfg->host_halo : cfg->host_frames + (size_t)(f - pl.first) * cfg->frame_stride;
+                uint8_t* dst = cb + (size_t)(slot + i) * fb;
+                if (dev_src) {
+                    launch_yuv420_to_bgr(src, yuv_planes_of(o->yin), cfg->frame_stride, (int)m, g.rows, g.cols, dst, g.pitch, fb, q);
+                } else {
+                    uint8_t* stg = (q == o->stream ? ystage_q : ystage_qs).as<uint8_t>();
+                    CK(yuv_copy(stg, S_in, sfb_in, src, o->yin, cfg->frame_stride, m, g.rows, g.cols, cudaMemcpyHostToDevice, q));
+                    launch_yuv420_to_bgr(stg, yuv_planes_of(S_in), sfb_in, (int)m, g.rows, g.cols, dst, g.pitch, fb, q);
+                }
+                i += m;
+            }
         } else {
             for (long i = 0; i < n; ++i) {
                 const long f = f0 + i;
@@ -1852,15 +2115,29 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
             vstab_status s2;
             if (ring == 0 && (s2 = fetch(p_lo, p_hi - p_lo + 1, 0, qw)) != VSTAB_OK) return s2;
             clock.begin(PH_RENDER, qw);
-            uint8_t* dst = cfg->d_out ? cfg->d_out + (size_t)(c - pl.call_first) * cfg->out_frame_stride : outc.as<uint8_t>();
+            const bool direct = cfg->d_out && !yout;                // warp straight into the caller's BGR buffer
+            uint8_t* dst = direct ? cfg->d_out + (size_t)(c - pl.call_first) * cfg->out_frame_stride : outc.as<uint8_t>();
             const long base = ring > 0 ? pl.first : p_lo;          // frame held by slot 0 (ring: modulo `ring`)
             s2 = offline_render_impl(o, resident ? dframe(p_lo) : cb, src_fs, src_step, base, (int)n, c, T_all.as<double>(), N, mode,
                                      cfg->lock_call, sums.as<unsigned long long>() + (size_t)(base - pl.first) * 3, dst,
-                                     cfg->d_out ? cfg->out_frame_stride : fb, cfg->d_out ? cfg->out_step : g.pitch,
+                                     direct ? cfg->out_frame_stride : fb, direct ? cfg->out_step : g.pitch,
                                      cfg->checksums ? checks.as<unsigned long long>() + (c - pl.call_first) : nullptr, ring, qw);
             clock.end(qw);
             if (s2 != VSTAB_OK) return s2;
-            if (cfg->host_out) {
+            uint8_t* yuv_dst = cfg->d_out ? cfg->d_out : cfg->host_out;
+            if (yout && yuv_dst) {
+                uint8_t* d = yuv_dst + (size_t)(c - pl.call_first) * cfg->out_frame_stride;
+                if (cfg->d_out) {
+                    launch_bgr_to_yuv420(outc.as<uint8_t>(), g.pitch, fb, (int)n, g.rows, g.cols, d, yuv_planes_of(o->yout),
+                                         cfg->out_frame_stride, qw);
+                } else {
+                    launch_bgr_to_yuv420(outc.as<uint8_t>(), g.pitch, fb, (int)n, g.rows, g.cols, ystage_o.as<uint8_t>(),
+                                         yuv_planes_of(S_out), sfb_out, qw);
+                    CK(yuv_copy(d, o->yout, cfg->out_frame_stride, ystage_o.as<uint8_t>(), S_out, sfb_out, n, g.rows, g.cols,
+                                cudaMemcpyDeviceToHost, qw));
+                }
+                CK(cudaGetLastError());
+            } else if (cfg->host_out) {
                 for (long i = 0; i < n; ++i)
                     CK(cudaMemcpy2DAsync(cfg->host_out + (size_t)(c - pl.call_first + i) * cfg->out_frame_stride, cfg->out_step,
                                          outc.as<uint8_t>() + (size_t)i * fb, g.pitch, row_bytes, g.rows, cudaMemcpyDeviceToHost, qw));
@@ -2174,6 +2451,44 @@ extern "C" vstab_status vstab_k_warp(int device, const uint8_t* bgr, int rows, i
     launch_warp(src.as<uint8_t>(), pitch, 0, 0, wp.as<WarpParams>(), 1, cols, rows, dst.as<uint8_t>(), pitch, 0, 0);
     CK(cudaGetLastError());
     CK(cudaMemcpy2D(out, out_step, dst.p, pitch, (size_t)cols * 3, rows, cudaMemcpyDeviceToHost));
+    return VSTAB_OK;
+}
+
+// K15 alone.  The YUV frame is mirrored on the device byte for byte over its extent (padding and gaps included), so the
+// kernels run on the caller's layout -- padded steps, planes apart, unaligned offsets -- and the caller sees exactly which
+// bytes bgr_to_yuv writes.
+extern "C" vstab_status vstab_k_yuv_to_bgr(int device, const uint8_t* yuv, const vstab_yuv_layout* layout, int rows, int cols,
+                                           uint8_t* bgr, size_t step) {
+    auto set_err = [&](const std::string& e) { g_err = e; };
+    if (!yuv || !bgr || step < (size_t)cols * 3) { g_err = "null pointer or row step smaller than 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
+    const size_t extent = yuv_extent(layout, rows, cols, g_err);
+    if (!extent) return VSTAB_ERR_INVALID_ARGUMENT;
+    if (!device_ok(device, g_err)) return VSTAB_ERR_CUDA;
+    const size_t pitch = align_up((size_t)cols * 3, 16);
+    DevBuf src, dst;
+    CK(src.alloc(extent)); CK(dst.alloc(pitch * rows));
+    CK(cudaMemcpy(src.p, yuv, extent, cudaMemcpyHostToDevice));
+    launch_yuv420_to_bgr(src.as<uint8_t>(), yuv_planes_of(*layout), 0, 1, rows, cols, dst.as<uint8_t>(), pitch, 0, 0);
+    CK(cudaGetLastError());
+    CK(cudaMemcpy2D(bgr, step, dst.p, pitch, (size_t)cols * 3, rows, cudaMemcpyDeviceToHost));
+    return VSTAB_OK;
+}
+
+extern "C" vstab_status vstab_k_bgr_to_yuv(int device, const uint8_t* bgr, int rows, int cols, size_t step, uint8_t* yuv,
+                                           const vstab_yuv_layout* layout) {
+    auto set_err = [&](const std::string& e) { g_err = e; };
+    if (!yuv || !bgr || step < (size_t)cols * 3) { g_err = "null pointer or row step smaller than 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
+    const size_t extent = yuv_extent(layout, rows, cols, g_err);
+    if (!extent) return VSTAB_ERR_INVALID_ARGUMENT;
+    if (!device_ok(device, g_err)) return VSTAB_ERR_CUDA;
+    const size_t pitch = align_up((size_t)cols * 3, 16);
+    DevBuf src, dst;
+    CK(src.alloc(pitch * rows)); CK(dst.alloc(extent));
+    CK(cudaMemcpy2D(src.p, pitch, bgr, step, (size_t)cols * 3, rows, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(dst.p, yuv, extent, cudaMemcpyHostToDevice));
+    launch_bgr_to_yuv420(src.as<uint8_t>(), pitch, 0, 1, rows, cols, dst.as<uint8_t>(), yuv_planes_of(*layout), 0, 0);
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(yuv, dst.p, extent, cudaMemcpyDeviceToHost));
     return VSTAB_OK;
 }
 

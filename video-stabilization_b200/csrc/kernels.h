@@ -134,6 +134,19 @@ void launch_warp(const uint8_t* frames, size_t pitch, size_t frame_stride, long 
                  uint8_t* out, size_t out_pitch, size_t out_frame_stride, cudaStream_t st,
                  unsigned long long* check = nullptr /* [nout], pre-zeroed: per-frame output checksum (warp.cu) */);
 
+// ---------------------------------------------------------------- K15 YUV 4:2:0 <-> BGR (cv::cvtColor, bit-exact)
+// the planes of one 4:2:0 frame relative to its base pointer; chroma sample k of a row is at off_u / off_v + k * cstep
+struct YuvPlanes {
+    size_t off_y, off_u, off_v;
+    size_t step_y, step_u, step_v;
+    int cstep;                   // 2: NV12 (one interleaved U,V plane, off_v = off_u + 1), 1: I420
+};
+// rows, cols even; frames `*_frame_stride` bytes apart (grid.z)
+void launch_yuv420_to_bgr(const uint8_t* yuv, const YuvPlanes& L, size_t yuv_frame_stride, int nframes, int rows, int cols,
+                          uint8_t* bgr, size_t pitch, size_t frame_stride, cudaStream_t st);
+void launch_bgr_to_yuv420(const uint8_t* bgr, size_t pitch, size_t frame_stride, int nframes, int rows, int cols, uint8_t* yuv,
+                          const YuvPlanes& L, size_t yuv_frame_stride, cudaStream_t st);
+
 // ---------------------------------------------------------------- K14 feathered trail compositing (copyFeathered)
 size_t trail_workspace_bytes(int w, int h, size_t frame_bytes);
 // out = copyFeathered(frames[slot], bg, wp->Hs) (src/stabilizer.cpp:1051-1155); src_slot < 0: the slot named by *wp

@@ -19,6 +19,7 @@ ACCUMULATED_FULL_LOCK, ORB_FULL_LOCK, SIFT_FULL_LOCK, TRANSLATION_LOCK, ROTATION
 
 OK, ERR_INVALID_ARGUMENT, ERR_SIZE_CHANGED, ERR_CUDA, ERR_UNSUPPORTED, ERR_STATE, ERR_NCCL = range(7)
 SRC_HOST, SRC_SIMULATOR, SRC_DEVICE = 0, 1, 2
+PIX_NV12, PIX_I420 = 1, 2
 
 TAP_GRAY, TAP_PYR1, TAP_PYR2, TAP_PYR3, TAP_PREV_PTS, TAP_LK_PTS, TAP_LK_STATUS, TAP_NEW_PTS, TAP_T, TAP_M, \
     TAP_H_STABILIZE, TAP_H_SCALED, TAP_BORDER, TAP_EIG, TAP_INLIERS, TAP_CHANNEL_SUMS, TAP_LOCK_H, TAP_ORB_COUNTS, \
@@ -36,6 +37,15 @@ class HParams(C.Structure):
     """struct HomographyParameters, include/stabilizer.hpp:44-57"""
     _fields_ = [("s", C.c_double), ("theta", C.c_double), ("k", C.c_double), ("delta", C.c_double),
                 ("t", C.c_double * 2), ("v", C.c_double * 2)]
+
+
+class YuvLayout(C.Structure):          # vstab_yuv_layout: plane k at base + offset[k], rows step[k] bytes apart
+    _fields_ = [("format", C.c_int), ("offset", C.c_size_t * 3), ("step", C.c_size_t * 3)]
+
+    @classmethod
+    def make(cls, fmt: int, offsets, steps):
+        off, st = list(offsets) + [0] * (3 - len(offsets)), list(steps) + [0] * (3 - len(steps))
+        return cls(int(fmt), (C.c_size_t * 3)(*off), (C.c_size_t * 3)(*st))
 
 
 class NcclId(C.Structure):
@@ -81,6 +91,12 @@ SYMBOLS = {
     "vstab_stabilize_frame": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_size_t, _vp, C.c_size_t]),
     "vstab_stabilize_frame_device": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_size_t, _vp, C.c_size_t]),
     "vstab_synchronize": (C.c_int, [_vp]),
+    "vstab_yuv_layout_packed": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.POINTER(YuvLayout)]),
+    "vstab_stabilize_frame_yuv": (C.c_int, [_vp, _vp, C.POINTER(YuvLayout), C.c_int, C.c_int, _vp, C.POINTER(YuvLayout)]),
+    "vstab_stabilize_frame_yuv_device": (C.c_int, [_vp, _vp, C.POINTER(YuvLayout), C.c_int, C.c_int, _vp, C.POINTER(YuvLayout)]),
+    "vstab_offline_set_yuv": (C.c_int, [_vp, C.POINTER(YuvLayout), C.POINTER(YuvLayout)]),
+    "vstab_k_yuv_to_bgr": (C.c_int, [C.c_int, _vp, C.POINTER(YuvLayout), C.c_int, C.c_int, _vp, C.c_size_t]),
+    "vstab_k_bgr_to_yuv": (C.c_int, [C.c_int, _vp, C.c_int, C.c_int, C.c_size_t, _vp, C.POINTER(YuvLayout)]),
     "vstab_decompose_homography": (C.c_int, [_f64p, C.c_double, C.c_double, C.POINTER(HParams)]),
     "vstab_compose_homography": (None, [C.POINTER(HParams), C.c_double, C.c_double, _f64p]),
     "vstab_last_error": (C.c_char_p, [_vp]),
@@ -197,6 +213,22 @@ def frame_checksum(img: np.ndarray) -> int:
         return int(t.sum(dtype=np.uint64))
 
 
+def yuv_layout_packed(fmt: int, rows: int, cols: int):
+    """The tight rawvideo layout of a rows x cols NV12 / I420 frame -> (YuvLayout, frame bytes).  Host only."""
+    L = YuvLayout()
+    n = load_library().vstab_yuv_layout_packed(int(fmt), int(rows), int(cols), C.byref(L))
+    if n == 0:
+        raise ValueError(f"no 4:2:0 layout for format {fmt} at {rows}x{cols} (formats PIX_NV12 / PIX_I420, even sizes)")
+    return L, int(n)
+
+
+def _yuv_frame_rows(frame: np.ndarray) -> int:
+    """rows of a packed 4:2:0 frame array [rows * 3 // 2, cols]"""
+    if not isinstance(frame, np.ndarray) or frame.dtype != np.uint8 or frame.ndim != 2 or frame.shape[0] % 3:
+        raise ValueError("a packed 4:2:0 frame is a uint8 array [rows * 3 // 2, cols]")
+    return frame.shape[0] * 2 // 3
+
+
 @dataclass
 class HomographyParameters:
     s: float = 1.0
@@ -256,6 +288,32 @@ class Stabilizer:
         _check(self._lib.vstab_stabilize_frame(self._h, _ptr(frame), frame.shape[0], frame.shape[1],
                                                frame.strides[0], _ptr(out), out.strides[0]), self._h)
         return out
+
+    def stabilize_frame_yuv(self, frame: np.ndarray, fmt: int, out: np.ndarray | None = None,
+                            out_fmt: int | None = None) -> np.ndarray:
+        """stabilize_frame on a packed NV12 / I420 frame [rows * 3 // 2, cols] (ffmpeg rawvideo); returns the output as a
+        packed frame of `out_fmt` (default: `fmt`).  Equals to_yuv(stabilize_frame(from_yuv(frame))) call by call."""
+        rows = _yuv_frame_rows(frame)
+        cols = frame.shape[1]
+        out_fmt = fmt if out_fmt is None else out_fmt
+        frame = np.ascontiguousarray(frame)
+        if out is None:
+            out = np.empty_like(frame)
+        elif (not isinstance(out, np.ndarray) or out.shape != frame.shape or out.dtype != np.uint8 or not out.flags.c_contiguous
+              or not out.flags.writeable):
+            raise ValueError("out must be a writeable C-contiguous uint8 array of the frame's shape")
+        # the library checks formats and sizes (odd sizes have no packed layout: pass one it rejects with its own message)
+        lin, lout = (YuvLayout.make(f, [0, 0, 0], [cols] * 3) for f in (fmt, out_fmt))
+        if rows > 0 and cols > 0 and rows % 2 == 0 and cols % 2 == 0 and fmt in (PIX_NV12, PIX_I420) and out_fmt in (PIX_NV12, PIX_I420):
+            lin, lout = yuv_layout_packed(fmt, rows, cols)[0], yuv_layout_packed(out_fmt, rows, cols)[0]
+        _check(self._lib.vstab_stabilize_frame_yuv(self._h, _ptr(frame), C.byref(lin), rows, cols, _ptr(out), C.byref(lout)), self._h)
+        return out
+
+    def stabilize_frame_yuv_ptr(self, src_ptr: int, layout: YuvLayout, rows: int, cols: int, dst_ptr: int,
+                                out_layout: YuvLayout, device: bool = False) -> None:
+        """YUV call on raw frame base pointers (host, or device with device=True: asynchronous, see synchronize())."""
+        fn = self._lib.vstab_stabilize_frame_yuv_device if device else self._lib.vstab_stabilize_frame_yuv
+        _check(fn(self._h, _vp(src_ptr), C.byref(layout), rows, cols, _vp(dst_ptr), C.byref(out_layout)), self._h)
 
     def stabilize_frame_ptr(self, src_ptr: int, rows: int, cols: int, step: int, dst_ptr: int, dst_step: int,
                             device: bool = False) -> None:
@@ -395,6 +453,34 @@ def k_warp(bgr: np.ndarray, H: np.ndarray, border, device: int = 0):
     out = np.empty_like(bgr)
     _check(lib.vstab_k_warp(device, _ptr(bgr), bgr.shape[0], bgr.shape[1], bgr.strides[0], H.ctypes.data_as(_f64p),
                             _ptr(b), _ptr(out), out.strides[0]))
+    return out
+
+
+def k_yuv_to_bgr(yuv: np.ndarray, layout, rows: int | None = None, cols: int | None = None, device: int = 0) -> np.ndarray:
+    """cvtColor(YUV2BGR_NV12 / _I420) on the GPU (K15).  `layout`: PIX_NV12 / PIX_I420 for a packed frame
+    [rows * 3 // 2, cols], or a YuvLayout of the frame whose base is yuv's first byte (then rows, cols are required)."""
+    lib = load_library()
+    yuv = np.ascontiguousarray(yuv)
+    if not isinstance(layout, YuvLayout):
+        rows, cols = _yuv_frame_rows(yuv), yuv.shape[1]
+        layout = yuv_layout_packed(layout, rows, cols)[0]
+    out = np.empty((rows, cols, 3), np.uint8)
+    _check(lib.vstab_k_yuv_to_bgr(device, _ptr(yuv), C.byref(layout), rows, cols, _ptr(out), out.strides[0]))
+    return out
+
+
+def k_bgr_to_yuv(bgr: np.ndarray, layout, out: np.ndarray | None = None, device: int = 0) -> np.ndarray:
+    """cvtColor(BGR2YUV_I420) on the GPU (K15; NV12 = its chroma interleaved U,V).  `layout`: PIX_NV12 / PIX_I420 returns a
+    packed frame [rows * 3 // 2, cols]; a YuvLayout writes its planes into `out` (a C-contiguous buffer holding the frame)."""
+    lib = load_library()
+    bgr = np.ascontiguousarray(bgr)
+    rows, cols = bgr.shape[:2]
+    if not isinstance(layout, YuvLayout):
+        layout = yuv_layout_packed(layout, rows, cols)[0]
+        out = np.zeros((rows * 3 // 2, cols), np.uint8)
+    elif out is None or not out.flags.c_contiguous or not out.flags.writeable:
+        raise ValueError("a YuvLayout needs a writeable C-contiguous `out` buffer")
+    _check(lib.vstab_k_bgr_to_yuv(device, _ptr(bgr), rows, cols, bgr.strides[0], _ptr(out), C.byref(layout)))
     return out
 
 

@@ -19,7 +19,7 @@ from __future__ import annotations
 import ctypes as C
 
 from . import (ACCUMULATED_FULL_LOCK, GLOBAL_SMOOTHING, SRC_DEVICE, SRC_HOST, SRC_SIMULATOR, NcclId, OfflineCfg, OfflineReport,  # noqa: F401
-               ShardPlan, _vp, load_library)
+               ShardPlan, YuvLayout, _vp, load_library, yuv_layout_packed)
 from . import _check as _check_any
 
 
@@ -89,6 +89,20 @@ class OfflineStabilizer:
         assert t.is_cuda and t.dtype == self._torch.uint8 and t.dim() == 4 and t.shape[1:] == (self.rows, self.cols, 3)
         assert t.stride(3) == 1 and t.stride(2) == 3
 
+    def _yuv_frames_ok(self, t):
+        """packed 4:2:0 frames [n, rows * 3 // 2, cols] (the frame stride may be larger than a frame)"""
+        assert t.dtype == self._torch.uint8 and t.dim() == 3 and tuple(t.shape[1:]) == (self.rows * 3 // 2, self.cols)
+        assert t.stride(2) == 1 and t.stride(1) == self.cols
+
+    def set_yuv(self, in_fmt=None, out_fmt=None):
+        """NV12 / I420 frames for run_host and run (vstab_offline_set_yuv): PIX_NV12 / PIX_I420 for packed frames
+        [n, rows * 3 // 2, cols], a YuvLayout for any other layout, None for BGR (the default).  The clip is processed as
+        BGR: checksums are those of the BGR outputs."""
+        def lay(f):
+            return None if f is None else f if isinstance(f, YuvLayout) else yuv_layout_packed(f, self.rows, self.cols)[0]
+        self._yuv = (lay(in_fmt), lay(out_fmt))
+        _check(self._lib.vstab_offline_set_yuv(self._h, *(C.byref(x) if x is not None else None for x in self._yuv)), self._h)
+
     def estimate(self, frames, first: int, halo, T_out, sums_out=None):
         """T_out[i] <- transform frame (first+i-1) -> (first+i); sums_out[i] <- channel byte sums."""
         self._frames_ok(frames)
@@ -131,6 +145,12 @@ class OfflineStabilizer:
         _check(self._lib.vstab_offline_run_host(self._h, _vp(frames_ptr), frame_stride, step, n_total, mode, lock_call,
                                                 _vp(out_ptr), out_frame_stride, out_step), self._h)
 
+    def _yuv_in(self):
+        return getattr(self, "_yuv", (None, None))[0] is not None
+
+    def _yuv_out(self):
+        return getattr(self, "_yuv", (None, None))[1] is not None
+
     # ---- the whole sharded job in the library (vstab_offline_run: NCCL all-gather inside) ---------------------
     def comm_init(self, rank: int, world: int, group=None):
         """Join the library-side NCCL communicator of the job: rank 0 makes the id, torch.distributed (any backend)
@@ -161,7 +181,7 @@ class OfflineStabilizer:
         tensor [n_local, rows, cols, 3], + `host_halo` [rows, cols, 3] on ranks > 0).  Returns a dict with the report,
         `checksums` (uint64 numpy, one per call of this rank) and optionally `T` [n_total, 3, 3].
         `device_frames` / `device_halo` / `device_out`: the shard, its halo frame and the outputs as CUDA tensors
-        (resident in HBM, no staging copies)."""
+        (resident in HBM, no staging copies).  After set_yuv, frames and outputs are packed 4:2:0 [n, rows * 3 // 2, cols]."""
         import numpy as np
         cfg = OfflineCfg()
         cfg.n_total, cfg.mode, cfg.lock_call = n_total, mode, lock_call
@@ -174,7 +194,7 @@ class OfflineStabilizer:
             cfg.poses, cfg.focal = poses.ctypes.data_as(C.POINTER(C.c_double)), float(focal)
             keep.append(poses)
         elif device_frames is not None:
-            self._frames_ok(device_frames)
+            (self._yuv_frames_ok if self._yuv_in() else self._frames_ok)(device_frames)
             cfg.source = SRC_DEVICE
             cfg.host_frames, cfg.frame_stride, cfg.step = device_frames.data_ptr(), device_frames.stride(0), device_frames.stride(1)
             cfg.host_halo = device_halo.data_ptr() if device_halo is not None else None
@@ -192,7 +212,7 @@ class OfflineStabilizer:
             cfg.out_frame_stride, cfg.out_step = (host_out.stride(0), host_out.stride(1)) if hasattr(host_out, "data_ptr") \
                 else (host_out.strides[0], host_out.strides[1])
         if device_out is not None:
-            self._frames_ok(device_out)
+            (self._yuv_frames_ok if self._yuv_out() else self._frames_ok)(device_out)
             assert device_out.shape[0] >= c1 - c0
             cfg.d_out, cfg.out_frame_stride, cfg.out_step = device_out.data_ptr(), device_out.stride(0), device_out.stride(1)
         sums = np.zeros(max(c1 - c0, 1), np.uint64)

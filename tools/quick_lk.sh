@@ -1,6 +1,6 @@
 #!/bin/bash
 # Quick check on the GPU box: per-stage times of the LK + warp path (256 frames per launch) and the kernel / pipeline parity tests.
-# usage (from the repo root): gpurun -- 'bash tools/lk_exp.sh'; prefix environment switches (DESIGN.md section 6) to A/B a kernel variant.
+# usage (from the repo root, on a machine with a B200): bash tools/quick_lk.sh
 cd "$(dirname "$0")/.."
 python bench.py --steps 6 --warmup 3 --frames-per-gpu 256 --batch 256 --no-cpu-baseline --no-e2e --no-mode-probes 2>/dev/null | python -c "
 import json,sys

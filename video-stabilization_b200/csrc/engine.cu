@@ -42,10 +42,6 @@ int device_sm_count() {
     }
     return n;
 }
-bool graphs_enabled() {
-    static const bool on = !(getenv("VSTAB_GRAPHS") && atoi(getenv("VSTAB_GRAPHS")) == 0);
-    return on;
-}
 GraphCache::~GraphCache() {
     for (auto& e : entries) {
         if (e.exec) cudaGraphExecDestroy(e.exec);
@@ -99,6 +95,8 @@ inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
     } while (0)
 
 thread_local std::string g_err;   // for entry points without an instance
+// a SIFT matcher launch (launch_l2_match / launch_l2_nn_batch) returned false
+constexpr const char* kL2MapErr = "SIFT matcher: cuTensorMapEncodeTiled (the driver's tensor-map encoder) is missing or rejected the descriptor arrays";
 void nccl_comm_destroy(void* comm);
 
 // VSTAB_GUARD=1 (tests): every device buffer of the library is allocated between two 4 KB guard bands filled with a pattern;
@@ -181,7 +179,6 @@ struct Geometry {
         // 1 row 0.51, 2 0.43, 3-4 0.41, 8 0.45; 4K -> 360 (6 source rows per destination row): 2 rows 85 % of the HBM roofline,
         // 4 rows 76 % -- so about 12 source rows per CTA.
         plan.rows_per_band = wh >= 360 ? ((long)r >= 5L * wh ? 2 : 4) : 1;
-        if (const char* e = getenv("VSTAB_INGEST_ROWS")) { if (atoi(e) > 0) plan.rows_per_band = atoi(e); }
         plan.nbands = (wh + plan.rows_per_band - 1) / plan.rows_per_band;
         std::vector<int4> hx(ww), hy(wh);
         build_ingest_tables(c, ww, plan.mode, hx.data());
@@ -562,11 +559,13 @@ static vstab_status stream_feature_lock(vstab* s, long p, cudaStream_t q, int sl
                                  counts + 1, s->cur_kps.as<OrbKeypoint>(), kOrbMaxKp, 0.6f, s->m_idx.as<int>(), s->m_d0.as<int>(),
                                  s->m_d1.as<int>(), s->m_good.as<uint8_t>(), s->m_ref.as<float2>(), s->m_cur.as<float2>(),
                                  s->m_status.as<uint8_t>(), counts + 2, q);                        // :647-673, :711-716
-        else
-            launch_l2_match(s->ref_desc.as<uint8_t>(), counts + 0, s->ref_kps.as<OrbKeypoint>(), s->cur_desc.as<uint8_t>(),
-                            counts + 1, s->cur_kps.as<OrbKeypoint>(), kOrbMaxKp, s->m_d1.p, s->m_idx.as<int>(), s->m_d0.as<int>(),
-                            s->m_good.as<uint8_t>(), s->m_ref.as<float2>(), s->m_cur.as<float2>(), s->m_status.as<uint8_t>(),
-                            counts + 2, q);                                                        // :675-708, :711-716
+        else if (!launch_l2_match(s->ref_desc.as<uint8_t>(), counts + 0, s->ref_kps.as<OrbKeypoint>(), s->cur_desc.as<uint8_t>(),
+                                  counts + 1, s->cur_kps.as<OrbKeypoint>(), kOrbMaxKp, s->m_d1.p, s->m_idx.as<int>(), s->m_d0.as<int>(),
+                                  s->m_good.as<uint8_t>(), s->m_ref.as<float2>(), s->m_cur.as<float2>(), s->m_status.as<uint8_t>(),
+                                  counts + 2, q)) {                                               // :675-708, :711-716
+            s->err = kL2MapErr;
+            return VSTAB_ERR_CUDA;
+        }
         launch_fit_large(s->m_ref.as<float2>(), s->m_cur.as<float2>(), s->m_status.as<uint8_t>(), counts + 2, 5.0,
                          g.ww / 2.0, g.wh / 2.0, Tfit, Tfit + 9, fitc, q);                         // :734-758
         launch_lock_update(Tfit, fitc, counts + 0, counts + 1, counts + 2, 0, lock_h, lock_tap, q);  // :784-787
@@ -622,8 +621,7 @@ static vstab_status stream_output(vstab* s, long n, uint8_t* d_out, size_t out_p
     a.cx = (double)(float)(g.ww / 2.0); a.cy = (double)(float)(g.wh / 2.0);                            // Point2f centre
     launch_smooth(a, n, 1, wp, q);                                                                     // :1234-1296
     if (!prepared_ahead) s->mark(8, q);
-    static const bool lookahead = !(getenv("VSTAB_LOOKAHEAD") && atoi(getenv("VSTAB_LOOKAHEAD")) == 0);
-    if (feature_lock && lookahead && s->F >= 2 && s->has_reference) {
+    if (feature_lock && s->F >= 2 && s->has_reference) {
         // registration of the next call's presentation frame, beside this call's warp and download.  Only with
         // future >= 2: that frame (n + 1 - F <= n - 1) is then already in the ring; with future == 1 it is the frame
         // this very call uploads AFTER its output chain was enqueued, so its registration stays inside call n + 1
@@ -704,7 +702,6 @@ static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols,
     const bool direct_out = device_out && !out_yuv;     // the warp writes the caller's BGR buffer itself
     const bool out_first = s->n > 0 && s->F >= 1;      // output chain does not need this call's transform
     static const bool trace = getenv("VSTAB_TRACE") != nullptr;
-    static const bool prepare_ok = !(getenv("VSTAB_PREPARE") && atoi(getenv("VSTAB_PREPARE")) == 0);
     auto now_us = [] { return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
     const double tr0 = trace ? now_us() : 0.0;
     double tr1 = 0.0;
@@ -800,7 +797,7 @@ static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols,
     }
     // the next call's output, beside this call's download (see pre_stream)
     const bool lk_mode = s->mode != VSTAB_ORB_FULL_LOCK && s->mode != VSTAB_SIFT_FULL_LOCK;
-    if (prepare_ok && host_wait && !device_out && s->F >= 1 && lk_mode && !s->trail) {
+    if (host_wait && !device_out && s->F >= 1 && lk_mode && !s->trail) {
         const long c = s->n + 1;
         if (in_call_chain) CK(cudaStreamWaitEvent(s->pre_stream, s->ev_chain, 0));
         CK(cudaStreamWaitEvent(s->pre_stream, fit_event(c), 0));
@@ -1156,8 +1153,6 @@ struct vstab_offline {
     DevBuf clip, outbuf, clipT, clipSums;
     size_t clip_frames = 0;
     cudaStream_t copy_in = nullptr, copy_out = nullptr;
-    cudaStream_t gftt_stream = nullptr;           // corner detection beside the pyramid build (VSTAB_OVERLAP=1)
-    cudaEvent_t ev_ingest = nullptr, ev_corners = nullptr;
     // ORB / SIFT registration (offline): reference set, per-launch scratch, gathered registrations
     OrbPlan* orb = nullptr;
     SiftPlan* sift = nullptr;
@@ -1288,10 +1283,8 @@ vstab_status vstab_offline_register(vstab_offline_t* o, const uint8_t* d_frames,
     // lanes: the ORB front end is ~44 small dependent launches per frame, SIFT at 4K mostly large ones (and 1.1 GB of pyramid per
     // lane).  Measured on B200, complete offline pass, frames/s with 1 / 2 / 3 / 4 / 8 lanes: ORB 1080p 1950 / - / 2834 / 2981 / 3117,
     // SIFT 4K 442 / 511 / 531 / - / 563.
-    static const int lanes_env = getenv("VSTAB_REG_LANES") ? atoi(getenv("VSTAB_REG_LANES")) : 0;
-    int K = lanes_env > 0 ? lanes_env : (is_orb ? 8 : 4);
+    int K = is_orb ? 8 : 4;
     if (K > n) K = n;
-    if (K > 8) K = 8;
     while ((int)o->lanes.size() < K - 1) {
         auto* L = new (std::nothrow) vstab_offline::RegLane();
         if (!L) { o->err = "out of memory"; return VSTAB_ERR_CUDA; }
@@ -1343,8 +1336,8 @@ vstab_status vstab_offline_register(vstab_offline_t* o, const uint8_t* d_frames,
                                  m_ref, m_cur, m_status, counts + 2, ql);
         } else {
             launch_sift(L ? L->sift : o->sift, feat_gray, cur_kps, cur_desc, counts + 1, ql);
-            launch_l2_match(ref_desc, nref, ref_kps, cur_desc, counts + 1, cur_kps, kOrbMaxKp, m_d1, m_idx, m_d0, m_good, m_ref, m_cur,
-                            m_status, counts + 2, ql);
+            if (!launch_l2_match(ref_desc, nref, ref_kps, cur_desc, counts + 1, cur_kps, kOrbMaxKp, m_d1, m_idx, m_d0, m_good, m_ref,
+                                 m_cur, m_status, counts + 2, ql)) { o->err = kL2MapErr; return VSTAB_ERR_CUDA; }
         }
         launch_fit_large(m_ref, m_cur, m_status, counts + 2, 5.0, g.ww / 2.0, g.wh / 2.0, Tfit, Tfit + 9, fitc, ql);
         launch_reg_store(Tfit, fitc, nref, counts + 1, counts + 2, d_reg + (size_t)i * 10, ql);
@@ -1403,9 +1396,6 @@ void vstab_offline_destroy(vstab_offline_t* o) {
     if (!o) return;
     cudaSetDevice(o->device);
     if (o->stream) { cudaStreamSynchronize(o->stream); cudaStreamDestroy(o->stream); }
-    if (o->gftt_stream) { cudaStreamSynchronize(o->gftt_stream); cudaStreamDestroy(o->gftt_stream); }
-    if (o->ev_ingest) cudaEventDestroy(o->ev_ingest);
-    if (o->ev_corners) cudaEventDestroy(o->ev_corners);
     if (o->copy_in) { cudaStreamSynchronize(o->copy_in); cudaStreamDestroy(o->copy_in); }
     if (o->copy_out) { cudaStreamSynchronize(o->copy_out); cudaStreamDestroy(o->copy_out); }
     if (o->orb) orb_plan_destroy(o->orb);
@@ -1470,40 +1460,14 @@ extern "C" vstab_status vstab_offline_estimate(vstab_offline_t* o, const uint8_t
     const int npairs = nslots - 1;
     float2* corners = o->corners.as<float2>() + (size_t)s0 * kMaxCorners;
     int* ccount = o->ccount.as<int>() + s0;
-    // Corner detection only needs the gray level 0 that ingest wrote, the tracker needs corners AND pyramid: with
-    // VSTAB_OVERLAP=1 the two run side by side on two streams (the top-k / greedy kernel is one latency-bound CTA per
-    // frame and leaves most issue slots to the pyramid kernels); stage times then are overlapping wall intervals.
-    static const bool overlap = getenv("VSTAB_OVERLAP") && atoi(getenv("VSTAB_OVERLAP")) != 0;
-    cudaStream_t qg = q;
-    if (overlap && npairs > 0) {
-        if (!o->gftt_stream) {
-            CK(cudaStreamCreateWithFlags(&o->gftt_stream, cudaStreamNonBlocking));
-            CK(cudaEventCreateWithFlags(&o->ev_ingest, cudaEventDisableTiming));
-            CK(cudaEventCreateWithFlags(&o->ev_corners, cudaEventDisableTiming));
-        }
-        qg = o->gftt_stream;
-        CK(cudaEventRecord(o->ev_ingest, q));
-        CK(cudaStreamWaitEvent(qg, o->ev_ingest, 0));
-    }
-    if (npairs > 0 && qg != q) {
-        o->timer.begin(ST_GFTT, qg);
-        launch_gftt(pyr + (size_t)s0 * g.pd.frame_bytes, g.pd.frame_bytes, g.ww, g.wh, npairs, 0.01, g.min_distance,
-                    kMaxCorners, o->gws, corners, ccount, nullptr, qg);
-        o->timer.end(ST_GFTT, qg);
-        CK(cudaEventRecord(o->ev_corners, qg));
-    }
     o->timer.begin(ST_PYRAMID, q);
     launch_pyramid(g.pd, pyr + (size_t)s0 * g.pd.frame_bytes, nslots, q);
     o->timer.end(ST_PYRAMID, q);
     if (npairs > 0) {
-        if (qg != q) {
-            CK(cudaStreamWaitEvent(q, o->ev_corners, 0));
-        } else {
-            o->timer.begin(ST_GFTT, q);
-            launch_gftt(pyr + (size_t)s0 * g.pd.frame_bytes, g.pd.frame_bytes, g.ww, g.wh, npairs, 0.01, g.min_distance,
-                        kMaxCorners, o->gws, corners, ccount, nullptr, q);
-            o->timer.end(ST_GFTT, q);
-        }
+        o->timer.begin(ST_GFTT, q);
+        launch_gftt(pyr + (size_t)s0 * g.pd.frame_bytes, g.pd.frame_bytes, g.ww, g.wh, npairs, 0.01, g.min_distance,
+                    kMaxCorners, o->gws, corners, ccount, nullptr, q);
+        o->timer.end(ST_GFTT, q);
         o->timer.begin(ST_LK, q);
         launch_lk(pyr + (size_t)s0 * g.pd.frame_bytes, pyr + (size_t)(s0 + 1) * g.pd.frame_bytes, g.pd.frame_bytes,
                   g.pd.frame_bytes, g.pd, corners, ccount, npairs, o->lkpts.as<float2>(), o->lkstat.as<uint8_t>(), q);
@@ -1993,8 +1957,7 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     // nothing else, so the calls whose windows are complete are warped right behind the estimation, from a ring of the last
     // ceil((F-1)/B) + 3 chunks -- every frame is rendered / uploaded once instead of twice.  The calls whose windows reach
     // into a neighbour's shard (the first P-1 and the last F-1 of a rank in a world > 1) wait for the all-gather as before.
-    static const bool fuse_ok = !(getenv("VSTAB_OFFLINE_FUSED") && atoi(getenv("VSTAB_OFFLINE_FUSED")) == 0);
-    const bool fused = fuse_ok && !resident && mode == VSTAB_GLOBAL_SMOOTHING;
+    const bool fused = !resident && mode == VSTAB_GLOBAL_SMOOTHING;
     vstab_fused_plan fp;
     vstab_offline_fused_plan(N, world, rank, o->P, o->F, B, &fp);
     const long ring_chunks = fused ? fp.ring_chunks : 1;
@@ -2638,9 +2601,9 @@ extern "C" vstab_status vstab_k_l2match(int device, const uint8_t* ref, int nref
     CK(cudaMemcpy(a.p, ref, (size_t)128 * nref, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(b.p, cur, (size_t)128 * ncur, cudaMemcpyHostToDevice));
     CK(cudaMemcpy(na.p, &nref, 4, cudaMemcpyHostToDevice)); CK(cudaMemcpy(nb.p, &ncur, 4, cudaMemcpyHostToDevice));
-    launch_l2_match(a.as<uint8_t>(), na.as<int>(), ka.as<OrbKeypoint>(), b.as<uint8_t>(), nb.as<int>(), kb.as<OrbKeypoint>(),
-                    kOrbMaxKp, scr.p, bi.as<int>(), bd.as<int>(), gd.as<uint8_t>(), rp.as<float2>(), cp.as<float2>(),
-                    stt.as<uint8_t>(), nm.as<int>(), 0);
+    if (!launch_l2_match(a.as<uint8_t>(), na.as<int>(), ka.as<OrbKeypoint>(), b.as<uint8_t>(), nb.as<int>(), kb.as<OrbKeypoint>(),
+                         kOrbMaxKp, scr.p, bi.as<int>(), bd.as<int>(), gd.as<uint8_t>(), rp.as<float2>(), cp.as<float2>(),
+                         stt.as<uint8_t>(), nm.as<int>(), 0)) { g_err = kL2MapErr; return VSTAB_ERR_CUDA; }
     CK(cudaGetLastError());
     CK(cudaDeviceSynchronize());
     CK(cudaMemcpy(best_idx, bi.p, 4 * (size_t)nref, cudaMemcpyDeviceToHost));
@@ -2670,12 +2633,13 @@ extern "C" vstab_status vstab_k_l2match_batch(int device, const uint8_t* ref, in
         off += (size_t)128 * ncur[f];
     }
     CK(cudaMemcpy(na.p, &nref, 4, cudaMemcpyHostToDevice)); CK(cudaMemcpy(nb.p, ncur, 4 * (size_t)nframes, cudaMemcpyHostToDevice));
+    if (!launch_l2_nn_batch(a.as<uint8_t>(), na.as<int>(), b.as<uint8_t>(), nb.as<int>(), kOrbMaxKp, nframes, scr.p, bi.as<int>(),
+                            bd.as<int>(), 0)) { g_err = kL2MapErr; return VSTAB_ERR_CUDA; }                     // warm-up
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0)); CK(cudaEventCreate(&e1));
     const int R = reps > 0 ? reps : 1;
-    launch_l2_nn_batch(a.as<uint8_t>(), na.as<int>(), b.as<uint8_t>(), nb.as<int>(), kOrbMaxKp, nframes, scr.p, bi.as<int>(), bd.as<int>(), 0);   // warm-up
     CK(cudaEventRecord(e0, 0));
-    for (int r = 0; r < R; ++r)
+    for (int r = 0; r < R; ++r)              // the same descriptor arrays as the warm-up: their tensor maps are made again
         launch_l2_nn_batch(a.as<uint8_t>(), na.as<int>(), b.as<uint8_t>(), nb.as<int>(), kOrbMaxKp, nframes, scr.p, bi.as<int>(), bd.as<int>(), 0);
     CK(cudaEventRecord(e1, 0));
     CK(cudaDeviceSynchronize());

@@ -12,7 +12,6 @@
 //   pass C  greedy min-distance suppression in sorted order on a cell grid held in shared
 //           memory, one warp per frame, 32 candidates per step with ballot/shuffle conflict
 //           resolution -- the accepted set and its order equal the sequential OpenCV loop.
-#include <cstdlib>
 #include <type_traits>
 #include <cub/block/block_radix_sort.cuh>
 #include <cub/device/device_segmented_radix_sort.cuh>
@@ -33,6 +32,7 @@ constexpr int kGreedySmemMax = 200 * 1024;
 // three eigenvalue rows (horizontal neighbours by shuffle).  Each gray row is read once per strip (+4 halo
 // columns, +4 halo rows per segment); every f32 product is converted to f64 once.
 constexpr int kStripW = 28, kSegH = 90, kEigWarps = 4;   // (segment height 45 / 60 / 90 / 120 / 180: 0.663 / 0.655 / 0.646 / 0.658 / 0.670 ms)
+constexpr int kEigPrefetchRows = 4;                      // eig_kernel's `pf`: L1 prefetch distance in rows
 
 struct D3 { double xx, xy, yy; };
 
@@ -539,16 +539,16 @@ void launch_gftt(const uint8_t* gray, size_t gray_frame_stride, int w, int h, in
                  float2* pts, int* counts, float* eig_out, cudaStream_t st) {
     if (nframes <= 0) return;
     if (max_corners > kMaxCorners) max_corners = kMaxCorners;
-    static const bool allow_fused = !(getenv("VSTAB_GFTT_FUSED") && atoi(getenv("VSTAB_GFTT_FUSED")) == 0);
     const size_t grid_bytes = (size_t)ws.ncells * kCellCap * sizeof(unsigned short);
     typedef TkShape<1024, 8> Big;
     typedef TkShape<512, 8> Small;
     const size_t fused_smem = sizeof(Big::Scratch) + grid_bytes;
     const size_t small_smem = sizeof(Small::Scratch) + grid_bytes;
-    const bool fused = allow_fused && fused_smem <= (size_t)220 * 1024;
+    // the unfused schedule (clamp, cub sort, greedy_kernel) serves cell grids that do not fit beside the top-k scratch:
+    // small working heights, where min_distance is 1 and a cell is one pixel
+    const bool fused = fused_smem <= (size_t)220 * 1024;
     // batches larger than one wave of single-CTA SMs: the half-size shape when two of its CTAs fit an SM
     // (227 KB shared memory per SM, 1 KB reserved per CTA, + the static histogram)
-    static const int small_ok = getenv("VSTAB_TOPK_SMALL") ? atoi(getenv("VSTAB_TOPK_SMALL")) : 1;
     static PerDeviceOnce once;
     once.run([] {
         cudaFuncSetAttribute(greedy_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kGreedySmemMax);
@@ -556,7 +556,7 @@ void launch_gftt(const uint8_t* gray, size_t gray_frame_stride, int w, int h, in
         cudaFuncSetAttribute(topk_greedy_kernel<512, 8, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024);
     });
     const int num_sms = device_sm_count();
-    const bool use_small = fused && small_ok && nframes > num_sms && small_smem <= (size_t)108 * 1024;
+    const bool use_small = fused && nframes > num_sms && small_smem <= (size_t)108 * 1024;
     const int key_bits = 31 + ws.idx_bits;
     // the fused kernel leaves the per-frame counters reset behind it
     if (!(fused && ws.counters_ready && nframes == 1)) {
@@ -567,16 +567,12 @@ void launch_gftt(const uint8_t* gray, size_t gray_frame_stride, int w, int h, in
     {
         // rows per warp: long segments amortise the 4 halo rows; a few frames alone (streaming) want more, shorter
         // warps instead (latency)
-        static int seg_env = -1;
-        if (seg_env < 0) { const char* e = getenv("VSTAB_EIG_SEGH"); seg_env = e ? atoi(e) : 0; }
-        const int seg_h = seg_env > 0 ? seg_env : (nframes >= 8 ? kSegH : 15);
+        const int seg_h = nframes >= 8 ? kSegH : 15;
         const int nstrips = (w + kStripW - 1) / kStripW, nsegs = (h + seg_h - 1) / seg_h;
         dim3 grid((nstrips * nsegs + kEigWarps - 1) / kEigWarps, nframes);
         count_launch(1);
-        static int pf = -1;
-        if (pf < 0) { const char* e = getenv("VSTAB_EIG_PF"); pf = e ? atoi(e) : 4; }
         eig_kernel<<<grid, 32 * kEigWarps, 0, st>>>(gray, gray_frame_stride, w, h, nstrips, nsegs, seg_h, ws.idx_bits, eig_out, ws.maxbits,
-                                                    ws.keys, ws.seg_end, ws.cap, quality, pf);
+                                                    ws.keys, ws.seg_end, ws.cap, quality, kEigPrefetchRows);
     }
     if (fused) {
         count_launch(1);

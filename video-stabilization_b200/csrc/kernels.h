@@ -165,17 +165,15 @@ void launch_featprep(const uint8_t* frame, size_t pitch, const int* xofs, const 
 // The ORB and SIFT front ends are long sequences of small dependent launches (44 / 118 per frame) whose arguments
 // do not change from call to call in streaming.  The second call with the same arguments captures the sequence on
 // its stream (thread-local capture) and every later one replays the graph: one launch, no per-kernel host cost,
-// back-to-back scheduling on the device.  VSTAB_GRAPHS=0 disables it.
+// back-to-back scheduling on the device.
 struct GraphCache {
     struct Entry { unsigned long long key[5]; cudaGraphExec_t exec; cudaGraph_t graph; int launches; int seen; };
     std::vector<Entry> entries;
     ~GraphCache();
 };
-bool graphs_enabled();
 // body(): enqueues the sequence on `st` (must be capturable: no allocation, no synchronisation)
 template <class F>
 void run_graphed(GraphCache& gc, const unsigned long long (&key)[5], cudaStream_t st, F&& body) {
-    if (!graphs_enabled()) { body(); return; }
     GraphCache::Entry* e = nullptr;
     for (auto& x : gc.entries) {
         bool same = true;
@@ -266,12 +264,14 @@ void launch_sift(SiftPlan* P, const uint8_t* gray, OrbKeypoint* kps_out, uint8_t
 // ---------------------------------------------------------------- K12 exact L2 matcher (tcgen05)
 // descriptors: u8 [n][128] (SIFT descriptors are integers 0..255).  best_d2 = exact squared distances.
 // scratch: l2_match_scratch_bytes(max_kp, 1) device bytes.  The current rows beyond *ncur up to the next multiple of 128 are zeroed.
+// Both return false, having launched nothing, when the driver's tensor-map encoder (cuTensorMapEncodeTiled) is missing or
+// rejects the descriptor arrays.
 size_t l2_match_scratch_bytes(int max_kp, int nframes);
-void launch_l2_match(const uint8_t* ref_desc, const int* nref, const OrbKeypoint* ref_kps, uint8_t* cur_desc,
+bool launch_l2_match(const uint8_t* ref_desc, const int* nref, const OrbKeypoint* ref_kps, uint8_t* cur_desc,
                      const int* ncur, const OrbKeypoint* cur_kps, int max_kp, void* scratch, int* best_idx, int* best_d2, uint8_t* good,
                      float2* ref_pts, float2* cur_pts, uint8_t* status, int* nmatch, cudaStream_t st);
 // the nearest-neighbour search alone, `nframes` current sets (cur_desc + f * max_kp * 128, ncur[f]) against one reference set
-void launch_l2_nn_batch(const uint8_t* ref_desc, const int* nref, uint8_t* cur_desc, const int* ncur, int max_kp, int nframes,
+bool launch_l2_nn_batch(const uint8_t* ref_desc, const int* nref, uint8_t* cur_desc, const int* ncur, int max_kp, int nframes,
                         void* scratch, int* best_idx, int* best_d2, cudaStream_t st);
 
 // ---------------------------------------------------------------- K13 simulator render

@@ -6,26 +6,18 @@
 //   ||a_i - b_j||^2 = ||a_i||^2 + ||b_j||^2 - 2 a_i . b_j
 // SIFT descriptors are integers 0..255 (SURVEY A.12): the dot products are exact integers <= 128 * 255^2 = 8.3e6.
 //
-// Default path, l2_nn_i8_kernel (further down): tcgen05 kind::i8 on the raw descriptor bytes (u8 x u8 -> s32), operand
-// tiles by TMA (SWIZZLE_128B: a descriptor row is one 128-byte swizzle row), a 4-stage ring of B tiles with full / empty
-// mbarriers, two 128-column TMEM accumulators, warp-specialised CTAs (producer lane, MMA lane, four epilogue warps), a
-// whole batch of frames along grid.z.  The epilogue folds each 128 x 128 tile into a row-wise arg-min on the packed key
-// (|b|^2 - 2 a.b) * 128 + column; the distance matrix never leaves the SM.
-//
-// VSTAB_L2_VARIANT=0 keeps round 1's kernel below for comparison (l2_nn_kernel): descriptors converted to fp16 by the
-// CTA itself (exact: 0..255; fp32 accumulation of 128 products <= 8.4e6 < 2^24 is exact), one shared-memory stage, one
-// 128-column accumulator, 8 x tcgen05.mma (M128 N128 K16, kind::f16) per tile, MMA -> commit -> wait -> epilogue in series.
-#include <cstdlib>
+// l2_nn_i8_kernel: tcgen05 kind::i8 on the raw descriptor bytes (u8 x u8 -> s32), operand tiles by TMA (SWIZZLE_128B: a
+// descriptor row is one 128-byte swizzle row), a 4-stage ring of B tiles with full / empty mbarriers, two 128-column TMEM
+// accumulators, warp-specialised CTAs (producer lane, MMA lane, four epilogue warps), a whole batch of frames along
+// grid.z.  The epilogue folds each 128 x 128 tile into a row-wise arg-min on the packed key (|b|^2 - 2 a.b) * 128 +
+// column; the distance matrix never leaves the SM.
 #include <cuda.h>
-#include <cuda_fp16.h>
 #include "kernels.h"
 
 namespace vstabk {
 namespace {
 
 constexpr int TM = 128, TN = 128, TK = 128;          // tile: reference rows, current rows, descriptor length
-constexpr int KB = 64;                                // fp16 elements per 128-byte swizzle row
-constexpr int kTileBytes = TM * KB * 2;               // one K-block of one operand tile: 16 KB
 
 VSTAB_D unsigned smem_addr(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 
@@ -41,142 +33,8 @@ VSTAB_D unsigned long long umma_desc(unsigned saddr) {
     return d;
 }
 
-// byte offset of element (row, k) inside one K-block tile [rows][64 fp16] with the 128-B swizzle:
-// 16-byte chunk c of row r lives at chunk position c ^ (r & 7)
-VSTAB_D int swz_off(int row, int k) {
-    const int chunk = k >> 3;
-    return (row >> 3) * 1024 + (row & 7) * 128 + ((chunk ^ (row & 7)) << 4) + (k & 7) * 2;
-}
-
-// Stage 128 descriptors (u8, 128 bytes each; rows >= n are zero) as fp16 into two swizzled K-block
-// tiles and return the squared norm of row `tid`.
-VSTAB_D int stage_tile(const uint8_t* __restrict__ desc, int row0, int n, unsigned char* smem_tile, int tid) {
-    // thread t converts row t: 128 bytes = 8 x uint4
-    const int row = row0 + tid;
-    int norm = 0;
-#pragma unroll
-    for (int c = 0; c < 8; ++c) {                      // 16 descriptor bytes -> 2 chunks of 8 fp16
-        uint4 v = make_uint4(0, 0, 0, 0);
-        if (row < n) v = __ldg(reinterpret_cast<const uint4*>(desc + (size_t)row * TK) + c);
-        const unsigned w[4] = {v.x, v.y, v.z, v.w};
-        __half2 h[8];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const int b0 = w[i] & 0xff, b1 = (w[i] >> 8) & 0xff, b2 = (w[i] >> 16) & 0xff, b3 = w[i] >> 24;
-            norm += b0 * b0 + b1 * b1 + b2 * b2 + b3 * b3;
-            h[2 * i] = __halves2half2(__int2half_rn(b0), __int2half_rn(b1));
-            h[2 * i + 1] = __halves2half2(__int2half_rn(b2), __int2half_rn(b3));
-        }
-        const int k = c * 16;                          // first of the 16 elements
-        unsigned char* blk = smem_tile + (k / KB) * kTileBytes;
-        *reinterpret_cast<uint4*>(blk + swz_off(tid, k % KB)) = *reinterpret_cast<uint4*>(&h[0]);
-        *reinterpret_cast<uint4*>(blk + swz_off(tid, (k % KB) + 8)) = *reinterpret_cast<uint4*>(&h[4]);
-    }
-    return norm;
-}
-
-__global__ void __launch_bounds__(128, 1)
-l2_nn_kernel(const uint8_t* __restrict__ ref, const int* __restrict__ nref_p, int nref_max,
-             const uint8_t* __restrict__ cur, const int* __restrict__ ncur_p, int ncur_max,
-             int* __restrict__ best_idx, int* __restrict__ best_d2) {
-    extern __shared__ unsigned char smem_raw[];
-    // SWIZZLE_128B operand tiles need 1024-byte alignment (the launch reserves 1 KB of slack)
-    unsigned char* smem = smem_raw + ((1024u - (smem_addr(smem_raw) & 1023u)) & 1023u);
-    unsigned char* sA = smem;                         // 2 K-blocks x 16 KB
-    unsigned char* sB = smem + 2 * kTileBytes;        // 2 K-blocks x 16 KB
-    __shared__ int nb[TN];
-    __shared__ unsigned long long mbar;
-    __shared__ unsigned tmem_base_smem;
-    const int nref = min(*nref_p, nref_max), ncur = min(*ncur_p, ncur_max);
-    const int tid = threadIdx.x, warp = tid >> 5;
-    const int row0 = blockIdx.x * TM;
-    if (row0 >= nref) return;
-
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_addr(&tmem_base_smem)), "r"(TN) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_addr(&mbar)), "r"(1) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    const int na = stage_tile(ref, row0, nref, sA, tid);
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const unsigned tmem = tmem_base_smem;
-
-    // instruction descriptor (cute::UMMA::InstrDescriptor): D = F32, A = B = F16, both K-major, N, M
-    const unsigned idesc = (1u << 4) | ((unsigned)(TN >> 3) << 17) | ((unsigned)(TM >> 4) << 24);
-    int bd = 0x7fffffff, bi = -1;
-    unsigned phase = 0;
-    for (int j0 = 0; j0 < ncur; j0 += TN) {
-        nb[tid] = stage_tile(cur, j0, ncur, sB, tid);
-        // generic-proxy writes to shared memory must be visible to the tensor core (async proxy)
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-            for (int k = 0; k < TK / 16; ++k) {                     // UMMA_K = 16 fp16 = 32 bytes
-                const unsigned koff = (unsigned)((k / 4) * kTileBytes + (k % 4) * 32);
-                const unsigned long long da = umma_desc(smem_addr(sA) + koff), db = umma_desc(smem_addr(sB) + koff);
-                const unsigned acc = k > 0 ? 1u : 0u;
-                asm volatile(
-                    "{\n\t"
-                    ".reg .pred p;\n\t"
-                    "setp.ne.b32 p, %4, 0;\n\t"
-                    "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t"
-                    "}\n" ::"r"(tmem), "l"(da), "l"(db), "r"(idesc), "r"(acc) : "memory");
-            }
-            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_addr(&mbar)) : "memory");
-        }
-        // wait for the accumulator
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "WAIT_%=:\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-            "@p bra DONE_%=;\n"
-            "bra WAIT_%=;\n"
-            "DONE_%=:\n"
-            "}\n" ::"r"(smem_addr(&mbar)), "r"(phase) : "memory");
-        phase ^= 1u;
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        // epilogue: thread `tid` owns TMEM lane (= reference row) tid; warp w may touch lanes 32w..32w+31
-        const unsigned taddr = tmem + ((unsigned)(warp * 32) << 16);
-#pragma unroll 1
-        for (int c0 = 0; c0 < TN; c0 += 32) {
-            unsigned r[32];
-            asm volatile(
-                "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-                "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-                : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-                  "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-                  "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-                  "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-                : "r"(taddr + (unsigned)c0)
-                : "memory");
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-            for (int c = 0; c < 32; ++c) {
-                const int j = j0 + c0 + c;
-                const int dot = __float2int_rn(__uint_as_float(r[c]));          // exact integer
-                const int d2 = na + nb[c0 + c] - 2 * dot;
-                if (j < ncur && d2 < bd) { bd = d2; bi = j; }                   // ascending j, strict <: lowest index wins ties
-            }
-        }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();                                  // TMEM and sB are free for the next tile
-    }
-    if (row0 + tid < nref) { best_idx[row0 + tid] = bi; best_d2[row0 + tid] = bd; }
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TN) : "memory");
-}
-
 // ---------------------------------------------------------------------------------------------------------------------
-// Pipelined version (default): kind::i8 on the raw descriptor bytes (u8 x u8 -> s32, exact; no conversion pass), operand
+// Pipelined: kind::i8 on the raw descriptor bytes (u8 x u8 -> s32, exact; no conversion pass), operand
 // tiles brought in by the TMA engine (cp.async.bulk.tensor.2d, SWIZZLE_128B: a descriptor row IS the 128-byte swizzle
 // row), a 4-stage ring of B tiles, two 128-column TMEM accumulators, warp-specialised CTAs of 6 warps:
 //   warp 0 (one lane)  TMA producer: A tile once, then B tiles into the ring (full / empty mbarriers)
@@ -497,26 +355,15 @@ size_t l2_match_scratch_bytes(int max_kp, int nframes) {
 }
 
 // `nframes` current sets (cur_desc + f * max_kp * 128, ncur[f]) against ONE reference set: one launch.  Per frame f the
-// results land in best_idx / best_d2 + f * max_kp.
-void launch_l2_nn_batch(const uint8_t* ref_desc, const int* nref, uint8_t* cur_desc, const int* ncur, int max_kp, int nframes,
+// results land in best_idx / best_d2 + f * max_kp.  false: no tensor map could be made for the descriptor arrays (the
+// driver's cuTensorMapEncodeTiled is missing or refused them), nothing was launched.
+bool launch_l2_nn_batch(const uint8_t* ref_desc, const int* nref, uint8_t* cur_desc, const int* ncur, int max_kp, int nframes,
                         void* scratch, int* best_idx, int* best_d2, cudaStream_t st) {
     unsigned long long* packed = reinterpret_cast<unsigned long long*>(scratch);
     int* na = reinterpret_cast<int*>(packed + (size_t)max_kp * nframes);
     int* nb = na + max_kp;
     CUtensorMap mapA, mapB;
-    const bool maps = make_desc_map(&mapA, ref_desc, (size_t)max_kp) && make_desc_map(&mapB, cur_desc, (size_t)max_kp * nframes);
-    static const int variant = getenv("VSTAB_L2_VARIANT") ? atoi(getenv("VSTAB_L2_VARIANT")) : 1;
-    if (!maps || variant == 0) {
-        // unpipelined fp16 kernel (one frame per launch): kept as the fall-back when the driver has no tensor-map encoder
-        const int smem = 4 * kTileBytes + 1024;
-        static PerDeviceOnce once0;
-        once0.run([&] { cudaFuncSetAttribute(l2_nn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); });
-        count_launch(nframes);
-        for (int f = 0; f < nframes; ++f)
-            l2_nn_kernel<<<(max_kp + TM - 1) / TM, 128, smem, st>>>(ref_desc, nref, max_kp, cur_desc + (size_t)f * max_kp * TK, ncur + f, max_kp,
-                                                                    best_idx + (size_t)f * max_kp, best_d2 + (size_t)f * max_kp);
-        return;
-    }
+    if (!make_desc_map(&mapA, ref_desc, (size_t)max_kp) || !make_desc_map(&mapB, cur_desc, (size_t)max_kp * nframes)) return false;
     const int smem = (int)sizeof(L2Smem) + 1024;
     static PerDeviceOnce once;
     once.run([&] { cudaFuncSetAttribute(l2_nn_i8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); });
@@ -528,15 +375,17 @@ void launch_l2_nn_batch(const uint8_t* ref_desc, const int* nref, uint8_t* cur_d
     l2_prep_kernel<<<dim3((max_kp + 7) / 8, nframes), 256, 0, st>>>(ref_desc, nref, cur_desc, ncur, max_kp, (size_t)max_kp * TK, na, nb, packed);
     l2_nn_i8_kernel<<<dim3(mt, splits, nframes), 192, smem, st>>>(mapA, mapB, nref, ncur, max_kp, na, nb, packed);
     l2_unpack_kernel<<<dim3((max_kp + 255) / 256, nframes), 256, 0, st>>>(packed, nref, max_kp, best_idx, best_d2);
+    return true;
 }
 
-void launch_l2_match(const uint8_t* ref_desc, const int* nref, const OrbKeypoint* ref_kps, uint8_t* cur_desc,
+bool launch_l2_match(const uint8_t* ref_desc, const int* nref, const OrbKeypoint* ref_kps, uint8_t* cur_desc,
                      const int* ncur, const OrbKeypoint* cur_kps, int max_kp, void* scratch, int* best_idx, int* best_d2, uint8_t* good,
                      float2* ref_pts, float2* cur_pts, uint8_t* status, int* nmatch, cudaStream_t st) {
-    launch_l2_nn_batch(ref_desc, nref, cur_desc, ncur, max_kp, 1, scratch, best_idx, best_d2, st);
+    if (!launch_l2_nn_batch(ref_desc, nref, cur_desc, ncur, max_kp, 1, scratch, best_idx, best_d2, st)) return false;
     count_launch(1);
     l2_filter_kernel<<<1, 256, 0, st>>>(best_idx, best_d2, nref, max_kp, ncur, ref_kps, cur_kps, good, ref_pts, cur_pts, status,
                                         nmatch);
+    return true;
 }
 
 }  // namespace vstabk

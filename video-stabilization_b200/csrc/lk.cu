@@ -29,7 +29,6 @@
 // argument the 7 taps of a strip are ONE pointer + immediate offsets.  Intensities come from the padded
 // u8 level (reflect-101 border) and derivatives from the padded Scharr level (zero border) that K2
 // prepares, so no tap ever needs border logic; both are tiny and L1/L2-resident.
-#include <cstdlib>
 #include "kernels.h"
 
 namespace vstabk {
@@ -457,15 +456,11 @@ void launch_lk(const uint8_t* prev_pyr, const uint8_t* next_pyr, size_t prev_str
     count_launch(1);
     // One warp per CTA: a CTA's registers and shared memory are held until its slowest feature converges, so one-warp
     // CTAs refill soonest (round 1: 4 / 2 / 1 warps per CTA 1.73 / 1.71 / 1.66 ms per 256 frames).
-    // VSTAB_LK_REGS: 128 (16 CTAs per SM), 96 (20) or 80 (24) registers per thread.
-    static const int regs = [] { const char* r = getenv("VSTAB_LK_REGS"); return r ? atoi(r) : 128; }();
     bool uniform = true;
     for (int l = 1; l < d.nlev; ++l) uniform = uniform && d.pitch[l] == d.pitch[0];
     const int P = uniform ? d.pitch[0] : 0;
-#define VSTAB_LK_ARGS P, nframes, st, prev_pyr, next_pyr, prev_stride, next_stride, d, pts, counts, out_pts, status
-    // min blocks per SM = 65536 / (registers * threads per CTA)
-    if (regs == 80) launch_chain<1, 24>(VSTAB_LK_ARGS); else if (regs == 96) launch_chain<1, 20>(VSTAB_LK_ARGS); else launch_chain<1, 16>(VSTAB_LK_ARGS);
-#undef VSTAB_LK_ARGS
+    // 16 CTAs per SM: 128 registers per thread (min blocks per SM = 65536 / (registers * threads per CTA))
+    launch_chain<1, 16>(P, nframes, st, prev_pyr, next_pyr, prev_stride, next_stride, d, pts, counts, out_pts, status);
 }
 
 }  // namespace vstabk

@@ -824,8 +824,7 @@ static void launch_sift_body(SiftPlan* P, const uint8_t* gray, OrbKeypoint* kps_
     // extrema pass of octave o: octaves >= 1 alternate between two auxiliary streams (fork / join by events; inside a
     // graph capture these become parallel branches).  The small octaves are ~40 launches of a few CTAs each, about
     // 0.5 ms of pure latency per 4K frame when they run behind octave 0 instead of beside it.
-    static const bool fork = !(getenv("VSTAB_SIFT_FORK") && atoi(getenv("VSTAB_SIFT_FORK")) == 0);
-    if (fork && !P->aux[0]) {
+    if (!P->aux[0]) {
         // highest priority: their few CTAs are dispatched ahead of the thousands queued by the octave-0 kernels
         int prio_lo = 0, prio_hi = 0;
         cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
@@ -839,9 +838,10 @@ static void launch_sift_body(SiftPlan* P, const uint8_t* gray, OrbKeypoint* kps_
         const size_t plane = (size_t)w * h;
         float* g = P->pyr + O.off[o];
         const int lane = (o - 1) & 1;
-        cudaStream_t q = (fork && o > 0) ? P->aux[lane] : st;
+        cudaStream_t q = o > 0 ? P->aux[lane] : st;
         if (o > 0) {
-            if (fork) { cudaStreamWaitEvent(q, P->ev_g3[o - 1], 0); used[lane] = true; }
+            cudaStreamWaitEvent(q, P->ev_g3[o - 1], 0);
+            used[lane] = true;
             const float* src = P->pyr + O.off[o - 1] + (size_t)kLayers * O.w[o - 1] * O.h[o - 1];
             sift_decimate_kernel<<<dim3((w + 255) / 256, h), 256, 0, q>>>(src, O.w[o - 1], g, w, h);
             ++launches;
@@ -849,7 +849,7 @@ static void launch_sift_body(SiftPlan* P, const uint8_t* gray, OrbKeypoint* kps_
         for (int i = 1; i < kGauss; ++i) {
             blur(g + (size_t)(i - 1) * plane, g + (size_t)i * plane, w, h, i, q);
             ++launches;
-            if (fork && i == kLayers && o + 1 < O.n) cudaEventRecord(P->ev_g3[o], q);
+            if (i == kLayers && o + 1 < O.n) cudaEventRecord(P->ev_g3[o], q);
         }
         if (w > 2 * kBorder && h > 2 * kBorder) {
             sift_extrema_tile_kernel<<<dim3((w - 2 * kBorder + EXW - 1) / EXW, (h - 2 * kBorder + EXH - 1) / EXH), 256, 0, q>>>(

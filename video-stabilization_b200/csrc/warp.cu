@@ -16,14 +16,8 @@
 //   * interior tiles (the unclamped footprint lies inside the image): branch-free path, no per-tap tests;
 //   * tiles touching the image border, non-affine H, footprints larger than a stage: per-pixel path with
 //     border substitution (generic_pixel).
-// Two schedules of the same tile code:
-//   variant 0  one CTA per tile, the box is filled with 16-byte cp.async copies by the CTA itself;
-//   variant 1  persistent CTAs (one wave), a producer thread has the TMA engine copy the box of the NEXT tile
-//              (cp.async.bulk.tensor.3d over a {pitch/4, rows, frames} u32 tensor map, zero fill outside)
-//              into the free stage while the 8 consumer warps blend the current one; mbarrier full/empty pairs.
-#include <cstdlib>
+// One CTA per tile; the box is filled with 16-byte cp.async copies by the CTA itself.
 #include <cstring>
-#include <cuda.h>
 #include "kernels.h"
 
 namespace vstabk {
@@ -133,12 +127,10 @@ VSTAB_D unsigned staged_pixel(const uint8_t* __restrict__ sm, int o, unsigned ax
 // staged box: x in [fx0, fx0+fxn], y in [fy0, fy0+fyn]; rows of `nb` bytes (from byte b0 of the source row) at a
 // stride of SP = kSP = 512 bytes (0: nothing staged): a multiple of 128, so that a lane whose taps sit one source
 // row lower hits the same banks (lanes are 3 words apart along a row: conflict-free).  `inside`: the unclamped footprint lies inside the
-// image, i.e. every tap of every pixel of the tile is in the box -> the branch-free path.  (fx0, fy0) may be
-// negative only in the TMA schedule, whose boxes are not clamped (the copy engine zero-fills; such tiles are not
-// `inside` and never read the zeros).
+// image, i.e. every tap of every pixel of the tile is in the box -> the branch-free path.
 struct TileBox { int fx0, fxn, fy0, fyn, b0, SP, nb, inside; };
 
-// Everything the consumer warps need to know about one destination tile.
+// Everything the CTA needs to know about its destination tile.
 struct TileInfo {
     double M[9];
     const uint8_t* src;
@@ -148,8 +140,7 @@ struct TileInfo {
 };
 
 // Source bounding box of the destination tile at (tx0, ty0) under the inverse map M, when M is affine and the box
-// fits a stage; otherwise the empty box.  kClamp: clip the box to the image (the ld.global fill must not leave it).
-template <bool kClamp>
+// fits a stage; otherwise the empty box.  The box is clipped to the image (the ld.global fill must not leave it).
 VSTAB_D TileBox tile_box(const double* M, const uint8_t* src, size_t pitch, int w, int h, int tx0, int ty0) {
     TileBox bx{0, 0, 0, 0, 0, 0, 0, 0};                                      // empty: nothing staged, no pixel is "inside"
     const bool al_ok = ((pitch & 15) == 0) && ((reinterpret_cast<uintptr_t>(src) & 15) == 0);
@@ -168,10 +159,10 @@ VSTAB_D TileBox tile_box(const double* M, const uint8_t* src, size_t pitch, int 
             const int ux0 = (int)floor(xmn) - 1, ux1 = (int)floor(xmx) + 2;
             const int uy0 = (int)floor(ymn) - 1, uy1 = (int)floor(ymx) + 2;
             const int inside = (ux0 >= 0 && ux1 <= w - 1 && uy0 >= 0 && uy1 <= h - 1) ? 1 : 0;
-            const int fx0 = kClamp ? max(0, ux0) : ux0, fx1 = kClamp ? min(w - 1, ux1) : ux1;
-            const int fy0 = kClamp ? max(0, uy0) : uy0, fy1 = kClamp ? min(h - 1, uy1) : uy1;
-            const int b0 = (3 * fx0) & ~15;                                  // (two's complement: rounds down for negatives)
-            const int b1 = kClamp ? min((int)pitch, (3 * (fx1 + 1) + 15) & ~15) : ((3 * (fx1 + 1) + 15) & ~15);
+            const int fx0 = max(0, ux0), fx1 = min(w - 1, ux1);
+            const int fy0 = max(0, uy0), fy1 = min(h - 1, uy1);
+            const int b0 = (3 * fx0) & ~15;
+            const int b1 = min((int)pitch, (3 * (fx1 + 1) + 15) & ~15);
             const int nb = b1 - b0;
             if (fx1 > fx0 && fy1 > fy0 && nb <= kSP && kSP * (fy1 - fy0 + 1) <= kStageBytes)
                 bx = TileBox{fx0, fx1 - fx0, fy0, fy1 - fy0, b0, kSP, nb, inside};
@@ -264,7 +255,7 @@ VSTAB_D void compute_tile_border(const uint8_t* __restrict__ sm, const TileBox b
     const double wdiv = kAffine ? __ddiv_rn(32.0, M8) : 0.0;
     const bool vec = x0 + 4 <= w && (out_pitch & 3) == 0 && ((reinterpret_cast<uintptr_t>(dst) & 3) == 0);
     const int obase = -box.fy0 * kSP - box.b0;
-    // only the part of the box inside the image may be read (unclamped TMA boxes hold zeros outside the image)
+    // a pixel reads the stage when its taps sx, sx + 1 and sy, sy + 1 all lie in the box
     const int cx0 = max(box.fx0, 0), cxn = box.SP > 0 ? max(min(box.fx0 + box.fxn, w - 1) - cx0, 0) : 0;
     const int cy0 = max(box.fy0, 0), cyn = box.SP > 0 ? max(min(box.fy0 + box.fyn, h - 1) - cy0, 0) : 0;
     const double XB = __dmul_rn(M0, bx), YB = __dmul_rn(M3, bx), WB = __dmul_rn(M6, bx);
@@ -328,7 +319,6 @@ VSTAB_D void fill_tile_info(TileInfo& I, const WarpParams& P, const uint8_t* fra
     I.src = frames + (size_t)I.slot * frame_stride;
 }
 
-// ---- variant 0: one CTA per tile ----------------------------------------------------------------------------
 template <bool kCheck>
 __global__ void __launch_bounds__(NTX * NTY, 4)
 warp_tile_kernel(const uint8_t* __restrict__ frames, size_t pitch, size_t frame_stride, long slot_mod,
@@ -341,7 +331,7 @@ warp_tile_kernel(const uint8_t* __restrict__ frames, size_t pitch, size_t frame_
     const int tx0 = blockIdx.x * TW, ty0 = blockIdx.y * TH;
     if (tid == 0) {
         fill_tile_info(I, wps[oi], frames, frame_stride, slot_mod);
-        I.box = tile_box<true>(I.M, I.src, pitch, w, h, tx0, ty0);
+        I.box = tile_box(I.M, I.src, pitch, w, h, tx0, ty0);
     }
     __syncthreads();
     const TileBox box = I.box;
@@ -364,185 +354,13 @@ warp_tile_kernel(const uint8_t* __restrict__ frames, size_t pitch, size_t frame_
                          threadIdx.x, threadIdx.y, kCheck ? check + oi : nullptr);
 }
 
-// ---- variant 1: persistent, TMA-fed ------------------------------------------------------------------------
-constexpr int kStages = 2;
-constexpr int kConsumerWarps = NTY;                        // 8 warps x 32 lanes = the 32 x 8 thread tile
-constexpr int kThreads = 32 * (1 + kConsumerWarps);        // + 1 producer warp
-constexpr int kTmaBoxW = 128;                              // u32 elements per box row  = 512 bytes = the row stride SP
-constexpr int kTmaRowBytes = kTmaBoxW * 4;
-static_assert(kTmaRowBytes == kSP, "the TMA box row is the stage row");
-constexpr int kTmaRowsA = 40, kTmaRowsB = 48;              // box rows: typical footprint / up to ~5 degrees of rotation
-constexpr int kTmaStageStride = kTmaRowsB * kTmaRowBytes + 128;
-
-struct __align__(128) WarpSmem {
-    unsigned char stage[kStages][kTmaStageStride];
-    TileInfo info[kStages];
-    unsigned long long full[kStages], empty[kStages];
-};
-
-VSTAB_D unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-VSTAB_D void mbar_init(unsigned long long* bar, unsigned count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-VSTAB_D void mbar_arrive(unsigned long long* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-VSTAB_D void mbar_arrive_expect_tx(unsigned long long* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-VSTAB_D void mbar_wait(unsigned long long* bar, unsigned parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-// same, for the lone producer thread: back off between polls instead of competing for issue slots
-VSTAB_D void mbar_wait_sleep(unsigned long long* bar, unsigned parity) {
-    const unsigned addr = smem_u32(bar);
-    for (;;) {
-        unsigned done;
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-            "selp.u32 %0, 1, 0, p;\n"
-            "}\n" : "=r"(done) : "r"(addr), "r"(parity) : "memory");
-        if (done) break;
-        __nanosleep(200);
-    }
-}
-// TMA: 3-D tiled tensor copy global -> shared, completion counted on an mbarrier (UTMALDG in SASS)
-VSTAB_D void tma_load_3d(void* dst, const CUtensorMap* map, int c0, int c1, int c2, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-                 ::"r"(smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-
-// mapA: box {128 u32, 40 rows, 1 frame}; mapB: box {128 u32, 48 rows, 1 frame} over the same {pitch/4, h, frames} tensor.
-// Footprints that need more rows (rotations beyond ~5 degrees) take the per-pixel path here; variant 0 stages up to 40 KB.
-__global__ void __launch_bounds__(kThreads, 4)
-warp_tma_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
-                const uint8_t* __restrict__ frames, size_t pitch, size_t frame_stride, long slot_mod,
-                const WarpParams* __restrict__ wps, int nout, int w, int h,
-                uint8_t* __restrict__ out, size_t out_pitch, size_t out_frame_stride) {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    WarpSmem& S = *reinterpret_cast<WarpSmem*>(smem_raw);
-    const int ntx = (w + TW - 1) / TW, nty = (h + TH - 1) / TH;
-    const int tiles_per_frame = ntx * nty;
-    const long ntiles = (long)tiles_per_frame * nout;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) {
-#pragma unroll
-        for (int s = 0; s < kStages; ++s) { mbar_init(&S.full[s], 1); mbar_init(&S.empty[s], kConsumerWarps); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    if (warp == 0) {
-        // ================================ producer (one thread) ==================================
-        if (lane != 0) return;
-        int it = 0;
-        for (long t = blockIdx.x; t < ntiles; t += gridDim.x, ++it) {
-            const int s = it % kStages;
-            if (it >= kStages) mbar_wait_sleep(&S.empty[s], ((it / kStages) - 1) & 1);
-            const int oi = (int)(t / tiles_per_frame);
-            const int tt = (int)(t - (long)oi * tiles_per_frame);
-            const int tyi = tt / ntx, txi = tt - tyi * ntx;
-            TileInfo& I = S.info[s];
-            fill_tile_info(I, wps[oi], frames, frame_stride, slot_mod);
-            I.oi = oi; I.tx0 = txi * TW; I.ty0 = tyi * TH;
-            TileBox bx = tile_box<false>(I.M, I.src, pitch, w, h, I.tx0, I.ty0);
-            if (bx.fyn + 1 > kTmaRowsB) { bx.SP = 0; bx.inside = 0; }       // footprint taller than a box: per-pixel path
-            if (bx.SP > 0) {
-                const bool small = bx.fyn + 1 <= kTmaRowsA;
-                I.box = bx;
-                mbar_arrive_expect_tx(&S.full[s], (unsigned)(kTmaRowBytes * (small ? kTmaRowsA : kTmaRowsB)));
-                tma_load_3d(&S.stage[s][0], small ? &mapA : &mapB, bx.b0 >> 2, bx.fy0, I.slot, &S.full[s]);
-            } else {
-                I.box = bx;
-                mbar_arrive(&S.full[s]);
-            }
-        }
-        return;
-    }
-
-    // ==================================== consumers ==============================================
-    const int tx = lane, ty = warp - 1;                       // 32 x 8 thread tile
-    int it = 0;
-    for (long t = blockIdx.x; t < ntiles; t += gridDim.x, ++it) {
-        const int s = it % kStages;
-        mbar_wait(&S.full[s], (it / kStages) & 1);
-        const TileInfo& I = S.info[s];
-        uint8_t* dst = out + (size_t)I.oi * out_frame_stride;
-        compute_tile<false>(S.stage[s], I.box, I.M, I.border, I.src, pitch, w, h, dst, out_pitch, I.tx0, I.ty0, tx, ty, nullptr);
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&S.empty[s]);            // this warp is done reading stage s
-    }
-}
-
-// ---- host: tensor maps for the TMA schedule --------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-struct TmaMaps {
-    const void* base = nullptr;
-    size_t pitch = 0, frame_stride = 0;
-    int h = 0;
-    bool ok = false;
-    CUtensorMap a, b;
-};
-
-bool make_maps(TmaMaps& m, const uint8_t* frames, size_t pitch, size_t frame_stride, int h) {
-    if (m.base == frames && m.pitch == pitch && m.frame_stride == frame_stride && m.h == h) return m.ok;
-    m.base = frames; m.pitch = pitch; m.frame_stride = frame_stride; m.h = h; m.ok = false;
-    static EncodeTiledFn encode = nullptr;
-    if (!encode) {
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn) return false;
-        encode = (EncodeTiledFn)fn;
-    }
-    if ((pitch & 15) || (reinterpret_cast<uintptr_t>(frames) & 15) || (frame_stride & 15)) return false;
-    const size_t fs = frame_stride ? frame_stride : ((pitch * (size_t)h + 15) & ~(size_t)15);
-    const cuuint64_t dims[3] = {pitch / 4, (cuuint64_t)h, frame_stride ? (cuuint64_t)1 << 22 : 1};
-    const cuuint64_t strides[2] = {pitch, fs};
-    const cuuint32_t estr[3] = {1, 1, 1};
-    const cuuint32_t boxA[3] = {kTmaBoxW, kTmaRowsA, 1}, boxB[3] = {kTmaBoxW, kTmaRowsB, 1};
-    if (encode(&m.a, CU_TENSOR_MAP_DATA_TYPE_UINT32, 3, (void*)frames, dims, strides, boxA, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return false;
-    if (encode(&m.b, CU_TENSOR_MAP_DATA_TYPE_UINT32, 3, (void*)frames, dims, strides, boxB, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return false;
-    m.ok = true;
-    return true;
-}
-
 }  // namespace
 
 void launch_warp(const uint8_t* frames, size_t pitch, size_t frame_stride, long slot_mod,
                  const WarpParams* wp, int nout, int w, int h,
                  uint8_t* out, size_t out_pitch, size_t out_frame_stride, cudaStream_t st, unsigned long long* check) {
     if (nout <= 0) return;
-    static const int variant = getenv("VSTAB_WARP_VARIANT") ? atoi(getenv("VSTAB_WARP_VARIANT")) : 0;
-    static const int ctas_per_sm = getenv("VSTAB_WARP_CTAS") && atoi(getenv("VSTAB_WARP_CTAS")) > 0 ? atoi(getenv("VSTAB_WARP_CTAS")) : 4;
-    static thread_local TmaMaps maps;
-    static PerDeviceOnce once;
-    once.run([] { cudaFuncSetAttribute(warp_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(WarpSmem)); });
-    const int num_sms = device_sm_count();
     count_launch(1);
-    const long ntiles = (long)((w + TW - 1) / TW) * ((h + TH - 1) / TH) * nout;
-    if (variant == 1 && !check && make_maps(maps, frames, pitch, frame_stride, h)) {
-        const int grid = (int)(ntiles < (long)num_sms * ctas_per_sm ? ntiles : (long)num_sms * ctas_per_sm);
-        warp_tma_kernel<<<grid, kThreads, sizeof(WarpSmem), st>>>(maps.a, maps.b, frames, pitch, frame_stride, slot_mod, wp, nout,
-                                                                  w, h, out, out_pitch, out_frame_stride);
-        return;
-    }
     dim3 grid((w + TW - 1) / TW, (h + TH - 1) / TH, nout);
     if (check)
         warp_tile_kernel<true><<<grid, dim3(NTX, NTY), 0, st>>>(frames, pitch, frame_stride, slot_mod, wp, w, h, out, out_pitch,

@@ -11,6 +11,7 @@
 // enqueues kernels and copies without ever reading a result back except the output frame.
 #include <atomic>
 #include <dlfcn.h>
+#include <memory>
 #include <mutex>
 #include <utility>
 #include <chrono>
@@ -163,6 +164,8 @@ struct Geometry {
     PyrDesc pd{};
     IngestPlan plan{};
     DevBuf xtab, ytab;
+    DevBuf nn_x, nn_y;           // cv::resize INTER_NEAREST offsets of the ORB / SIFT conditioning (nn_tables)
+    bool nn_ready = false;
     int min_distance = 0;
 
     vstab_status init(int r, int c, int working_height, std::string& err) {
@@ -194,6 +197,21 @@ struct Geometry {
         plan.ytab = ytab.as<int4>();
         min_distance = (int)(10 * ((double)wh / 720.0));                // stabilizer.cpp:938-940
         return VSTAB_OK;
+    }
+
+    // nn_x / nn_y, built on first use: only the ORB / SIFT paths condition frames
+    cudaError_t nn_tables() {
+        if (nn_ready) return cudaSuccess;
+        auto table = [](DevBuf& t, int src, int dst) {
+            std::vector<int> h(dst);
+            build_nn_table(src, dst, h.data());
+            const cudaError_t e = t.alloc(sizeof(int) * dst);
+            return e != cudaSuccess ? e : cudaMemcpy(t.p, h.data(), sizeof(int) * dst, cudaMemcpyHostToDevice);
+        };
+        cudaError_t e = table(nn_x, cols, ww);
+        if (e == cudaSuccess) e = table(nn_y, rows, wh);
+        nn_ready = e == cudaSuccess;
+        return e;
     }
 };
 
@@ -311,6 +329,94 @@ cudaError_t yuv_copy(uint8_t* dst, const vstab_yuv_layout& dl, size_t dst_fs, co
     return cudaSuccess;
 }
 
+// ---- ORB / SIFT registration (stabilizer.cpp:440-787), shared by the streaming instance and the offline runner ---------
+// The reference set is one packed device buffer: {int count, pad to 16 B} {OrbKeypoint[kOrbMaxKp]} {u8 desc[kOrbMaxKp][128]},
+// so the offline ranks can broadcast it as it is.
+constexpr size_t kRefPackKps = 16;
+constexpr size_t kRefPackDesc = kRefPackKps + sizeof(OrbKeypoint) * kOrbMaxKp;
+constexpr size_t kRefPackBytes = kRefPackDesc + (size_t)128 * kOrbMaxKp;
+struct RefSet {
+    int* count;
+    OrbKeypoint* kps;
+    uint8_t* desc;
+    explicit RefSet(void* pack)
+        : count((int*)pack), kps((OrbKeypoint*)((char*)pack + kRefPackKps)), desc((uint8_t*)pack + kRefPackDesc) {}
+};
+
+// Everything one registration in flight needs.  The front ends are replayed as CUDA graphs keyed on their buffers and
+// stream (run_graphed), so a lane passes the same buffers from call to call.
+struct RegLane {
+    OrbPlan* orb = nullptr;              // plan of the mode, created on its first use
+    SiftPlan* sift = nullptr;
+    DevBuf feat_ws, feat_gray, kps, desc, counts, m_idx, m_d0, m_d1, m_good, m_ref, m_cur, m_status, fit;
+    cudaStream_t q = nullptr;            // own stream (offline lanes beyond the first), or null: the caller's
+    cudaEvent_t done = nullptr;
+    ~RegLane() {
+        if (q) { cudaStreamSynchronize(q); cudaStreamDestroy(q); }
+        if (done) cudaEventDestroy(done);
+        if (orb) orb_plan_destroy(orb);
+        if (sift) sift_plan_destroy(sift);
+    }
+    int* ncur() { return counts.as<int>(); }
+    int* nmatch() { return counts.as<int>() + 1; }
+    double* Tfit() { return fit.as<double>(); }
+    int* fitc() { return reinterpret_cast<int*>(fit.as<double>() + 16); }
+    uint8_t* gray(const Geometry& g, int slot) { return feat_gray.as<uint8_t>() + (size_t)slot * g.ww * g.wh; }
+
+    // buffers (on first use: `gray_slots` conditioned images, counts zeroed on `stream`) and the plan of `mode`
+    vstab_status setup(Geometry& g, int mode, int gray_slots, cudaStream_t stream, std::string& err) {
+        auto set_err = [&](const std::string& e) { err = e; };
+        if (!feat_ws.p) {
+            CK(g.nn_tables());
+            CK(feat_ws.alloc(featprep_workspace_bytes(g.ww, g.wh)));
+            CK(feat_gray.alloc((size_t)g.ww * g.wh * gray_slots));
+            CK(kps.alloc(sizeof(OrbKeypoint) * kOrbMaxKp));
+            CK(desc.alloc(128 * kOrbMaxKp));                                    // 32 B (ORB) or 128 B (SIFT) per row
+            CK(counts.alloc(sizeof(int) * 2));                                  // {ncur, nmatch}
+            CK(m_idx.alloc(4 * kOrbMaxKp)); CK(m_d0.alloc(4 * kOrbMaxKp)); CK(m_d1.alloc(l2_match_scratch_bytes(kOrbMaxKp, 1)));   // m_d1: second distances (Hamming) / matcher scratch (L2)
+            CK(m_good.alloc(kOrbMaxKp)); CK(m_status.alloc(kOrbMaxKp));
+            CK(m_ref.alloc(sizeof(float2) * kOrbMaxKp)); CK(m_cur.alloc(sizeof(float2) * kOrbMaxKp));
+            CK(fit.alloc(sizeof(double) * 16 + sizeof(int) * 4));              // T[9], M[6], counts[2]
+            CK(cudaMemsetAsync(counts.p, 0, sizeof(int) * 2, stream));
+        }
+        if (mode == VSTAB_ORB_FULL_LOCK && !orb && !(orb = orb_plan_create(g.ww, g.wh, 0.10, kOrbMaxKp, &err)))    // MAX_KEYPOINT_RELATIVE_SIZE_ORB, :493
+            return VSTAB_ERR_CUDA;
+        if (mode == VSTAB_SIFT_FULL_LOCK && !sift && !(sift = sift_plan_create(g.ww, g.wh, 0.05, kOrbMaxKp, &err)))  // MAX_KEYPOINT_RELATIVE_SIZE_SIFT, :507
+            return VSTAB_ERR_CUDA;
+        return VSTAB_OK;
+    }
+
+    // condition `frame` (:448-477) into gray slot `slot` and detect + describe it into kps / desc / *count
+    void detect(Geometry& g, const uint8_t* frame, size_t step, int slot, bool is_orb, OrbKeypoint* k, uint8_t* d, int* count,
+                bool reference_order, cudaStream_t st) {
+        launch_featprep(frame, step, g.nn_x.as<int>(), g.nn_y.as<int>(), g.ww, g.wh, feat_ws.p, gray(g, slot), st);
+        if (is_orb) launch_orb(orb, gray(g, slot), k, d, count, reference_order, st);               // :557-559 / :604-612
+        else launch_sift(sift, gray(g, slot), k, d, count, st);                                      // :572-574 / :614-621
+    }
+
+    // reference capture (:520-589): the ORB set in cv::ORB's order
+    void capture(Geometry& g, const uint8_t* frame, size_t step, int slot, bool is_orb, const RefSet& ref, cudaStream_t st) {
+        detect(g, frame, step, slot, is_orb, ref.kps, ref.desc, ref.count, true, st);
+    }
+
+    // detect + describe, match against `ref` (:647-716) and fit (:734-758) into Tfit / fitc.  False, having launched no
+    // matcher, when the SIFT matcher could not be launched (kL2MapErr).
+    bool match(Geometry& g, const uint8_t* frame, size_t step, int slot, bool is_orb, const RefSet& ref, cudaStream_t st) {
+        detect(g, frame, step, slot, is_orb, kps.as<OrbKeypoint>(), desc.as<uint8_t>(), ncur(), false, st);
+        if (is_orb)
+            launch_hamming_match(ref.desc, ref.count, ref.kps, desc.as<uint8_t>(), ncur(), kps.as<OrbKeypoint>(), kOrbMaxKp, 0.6f,
+                                 m_idx.as<int>(), m_d0.as<int>(), m_d1.as<int>(), m_good.as<uint8_t>(), m_ref.as<float2>(),
+                                 m_cur.as<float2>(), m_status.as<uint8_t>(), nmatch(), st);
+        else if (!launch_l2_match(ref.desc, ref.count, ref.kps, desc.as<uint8_t>(), ncur(), kps.as<OrbKeypoint>(), kOrbMaxKp, m_d1.p,
+                                  m_idx.as<int>(), m_d0.as<int>(), m_good.as<uint8_t>(), m_ref.as<float2>(), m_cur.as<float2>(),
+                                  m_status.as<uint8_t>(), nmatch(), st))
+            return false;
+        launch_fit_large(m_ref.as<float2>(), m_cur.as<float2>(), m_status.as<uint8_t>(), nmatch(), 5.0, g.ww / 2.0, g.wh / 2.0,
+                         Tfit(), Tfit() + 9, fitc(), st);
+        return true;
+    }
+};
+
 }  // namespace
 
 // =====================================================================================
@@ -367,10 +473,12 @@ struct vstab {
     uint8_t* dout_at(int slot) { return (slot & 1) ? dout1.as<uint8_t>() : dout.as<uint8_t>(); }
     long t_mod = 0;
     GfttWorkspace gws[2] = {};   // [n & 1]: the corner detections of two consecutive frames overlap
-    // ORB registration state (reference: referenceGray_/Keypoints_/Descriptors_, hpp:447-456, and the
-    // function-static previouslyReturnedH, cpp:446 -- per instance here)
-    OrbPlan* orb = nullptr;
-    SiftPlan* sift = nullptr;
+    // ORB / SIFT registration state (reference: referenceGray_/Keypoints_/Descriptors_, hpp:447-456, and the
+    // function-static previouslyReturnedH, cpp:446 -- per instance here).  One lane serves the in-call (out_stream) and the
+    // look-ahead (feat_stream) registration, ordered by ev_reg / ev_feat; its conditioned image is double-buffered by
+    // lock_slot like lock_h / lock_tap.
+    RegLane reg;
+    DevBuf ref, lock_h, lock_tap;        // ref: packed reference set (RefSet)
     bool has_reference = false;
     bool trail = false;                     // copyFeathered branch of stabilizeFrame (:1303-1307)
     bool partial_fix = false;               // TRANSLATION_/ROTATION_LOCK fed with the accumulated lock (hpp:23 @todo)
@@ -378,8 +486,6 @@ struct vstab {
     // YUV calls with host buffers: the input planes are uploaded here (copy_stream) and converted into the ring, the
     // presented BGR frame is converted here (out_stream) and downloaded.  One frame each: every use is ordered by its stream.
     DevBuf yuv_in, yuv_out;
-    DevBuf feat_ws, feat_gray, nn_x, nn_y, ref_kps, ref_desc, cur_kps, cur_desc, orb_counts, m_idx, m_d0, m_d1, m_good,
-        m_ref, m_cur, m_status, lock_fit, lock_h, lock_tap;
     std::string err;
     // VSTAB_TRACE=1: host wall-clock split of the streaming call (printed by vstab_destroy)
     double trace_us[4] = {0, 0, 0, 0};   // enqueue output chain | enqueue upload + estimation | wait upload | wait output
@@ -505,70 +611,29 @@ static vstab_status stream_estimate(vstab* s) {
 static vstab_status stream_feature_lock(vstab* s, long p, cudaStream_t q, int slot) {
     auto set_err = [&](const std::string& e) { s->err = e; };
     Geometry& g = s->g;
+    RegLane& L = s->reg;
     const bool is_orb = s->mode == VSTAB_ORB_FULL_LOCK;
-    if (!s->feat_ws.p) {
-        std::vector<int> xo(g.ww), yo(g.wh);
-        build_nn_table(g.cols, g.ww, xo.data());
-        build_nn_table(g.rows, g.wh, yo.data());
-        CK(s->feat_ws.alloc(featprep_workspace_bytes(g.ww, g.wh)));
-        CK(s->feat_gray.alloc((size_t)g.ww * g.wh * 2));                     // one conditioned image per lock slot
-        CK(s->nn_x.alloc(sizeof(int) * g.ww)); CK(s->nn_y.alloc(sizeof(int) * g.wh));
-        CK(cudaMemcpy(s->nn_x.p, xo.data(), sizeof(int) * g.ww, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(s->nn_y.p, yo.data(), sizeof(int) * g.wh, cudaMemcpyHostToDevice));
-        CK(s->ref_kps.alloc(sizeof(OrbKeypoint) * kOrbMaxKp)); CK(s->cur_kps.alloc(sizeof(OrbKeypoint) * kOrbMaxKp));
-        CK(s->ref_desc.alloc(128 * kOrbMaxKp)); CK(s->cur_desc.alloc(128 * kOrbMaxKp));   // 32 B (ORB) or 128 B (SIFT) per row
-        CK(s->orb_counts.alloc(sizeof(int) * 4));                            // {nref, ncur, nmatch}
-        CK(s->m_idx.alloc(4 * kOrbMaxKp)); CK(s->m_d0.alloc(4 * kOrbMaxKp)); CK(s->m_d1.alloc(l2_match_scratch_bytes(kOrbMaxKp, 1)));   // m_d1: second distances (Hamming) / matcher scratch (L2)
-        CK(s->m_good.alloc(kOrbMaxKp)); CK(s->m_status.alloc(kOrbMaxKp));
-        CK(s->m_ref.alloc(sizeof(float2) * kOrbMaxKp)); CK(s->m_cur.alloc(sizeof(float2) * kOrbMaxKp));
-        CK(s->lock_fit.alloc(sizeof(double) * 16 + sizeof(int) * 4));        // T[9], M[6], counts[2]
+    if (!s->ref.p) {
+        CK(s->ref.alloc(kRefPackBytes));
         CK(s->lock_h.alloc(sizeof(double) * 9 * 2));
         CK(s->lock_tap.alloc(sizeof(int) * 8 * 2));
-        CK(cudaMemsetAsync(s->orb_counts.p, 0, sizeof(int) * 4, q));
+        CK(cudaMemsetAsync(s->ref.p, 0, kRefPackBytes, q));
     }
-    if (is_orb && !s->orb) {
-        s->orb = orb_plan_create(g.ww, g.wh, 0.10, kOrbMaxKp, &s->err);      // MAX_KEYPOINT_RELATIVE_SIZE_ORB, :493
-        if (!s->orb) return VSTAB_ERR_CUDA;
-    }
-    if (!is_orb && !s->sift) {
-        s->sift = sift_plan_create(g.ww, g.wh, 0.05, kOrbMaxKp, &s->err);    // MAX_KEYPOINT_RELATIVE_SIZE_SIFT, :507
-        if (!s->sift) return VSTAB_ERR_CUDA;
-    }
+    vstab_status st = L.setup(g, s->mode, 2, q, s->err);
+    if (st != VSTAB_OK) return st;
     const uint8_t* frame = s->ring.as<uint8_t>() + (size_t)(p % s->W) * g.frame_bytes;           // :444
-    uint8_t* feat_gray = s->feat_gray.as<uint8_t>() + (size_t)slot * g.ww * g.wh;
-    launch_featprep(frame, g.pitch, s->nn_x.as<int>(), s->nn_y.as<int>(), g.ww, g.wh, s->feat_ws.p, feat_gray, q);  // :448-477
-    int* counts = s->orb_counts.as<int>();
-    double* Tfit = s->lock_fit.as<double>();
-    int* fitc = reinterpret_cast<int*>(Tfit + 16);
-    const bool capture = !s->has_reference;                                                      // :520-589
+    const RefSet ref(s->ref.p);
     double* lock_h = s->lock_h.as<double>() + 9 * slot;
     int* lock_tap = s->lock_tap.as<int>() + 8 * slot;
-    // "previously returned H" (:446) carries over from the other half
-    if (!capture) CK(cudaMemcpyAsync(lock_h, s->lock_h.as<double>() + 9 * (slot ^ 1), sizeof(double) * 9, cudaMemcpyDeviceToDevice, q));
-    OrbKeypoint* kps = capture ? s->ref_kps.as<OrbKeypoint>() : s->cur_kps.as<OrbKeypoint>();
-    uint8_t* desc = capture ? s->ref_desc.as<uint8_t>() : s->cur_desc.as<uint8_t>();
-    int* cnt = counts + (capture ? 0 : 1);
-    if (is_orb) launch_orb(s->orb, feat_gray, kps, desc, cnt, capture, q);                       // :557-559 / :604-612
-    else launch_sift(s->sift, feat_gray, kps, desc, cnt, q);                                     // :572-574 / :614-621
-    if (capture) {
-        launch_lock_update(Tfit, fitc, counts + 0, counts + 0, counts + 0, 1, lock_h, lock_tap, q);
+    if (!s->has_reference) {                                                                     // :520-589
+        L.capture(g, frame, g.pitch, slot, is_orb, ref, q);
+        launch_lock_update(L.Tfit(), L.fitc(), ref.count, ref.count, ref.count, 1, lock_h, lock_tap, q);
         s->has_reference = true;
     } else {
-        if (is_orb)
-            launch_hamming_match(s->ref_desc.as<uint8_t>(), counts + 0, s->ref_kps.as<OrbKeypoint>(), s->cur_desc.as<uint8_t>(),
-                                 counts + 1, s->cur_kps.as<OrbKeypoint>(), kOrbMaxKp, 0.6f, s->m_idx.as<int>(), s->m_d0.as<int>(),
-                                 s->m_d1.as<int>(), s->m_good.as<uint8_t>(), s->m_ref.as<float2>(), s->m_cur.as<float2>(),
-                                 s->m_status.as<uint8_t>(), counts + 2, q);                        // :647-673, :711-716
-        else if (!launch_l2_match(s->ref_desc.as<uint8_t>(), counts + 0, s->ref_kps.as<OrbKeypoint>(), s->cur_desc.as<uint8_t>(),
-                                  counts + 1, s->cur_kps.as<OrbKeypoint>(), kOrbMaxKp, s->m_d1.p, s->m_idx.as<int>(), s->m_d0.as<int>(),
-                                  s->m_good.as<uint8_t>(), s->m_ref.as<float2>(), s->m_cur.as<float2>(), s->m_status.as<uint8_t>(),
-                                  counts + 2, q)) {                                               // :675-708, :711-716
-            s->err = kL2MapErr;
-            return VSTAB_ERR_CUDA;
-        }
-        launch_fit_large(s->m_ref.as<float2>(), s->m_cur.as<float2>(), s->m_status.as<uint8_t>(), counts + 2, 5.0,
-                         g.ww / 2.0, g.wh / 2.0, Tfit, Tfit + 9, fitc, q);                         // :734-758
-        launch_lock_update(Tfit, fitc, counts + 0, counts + 1, counts + 2, 0, lock_h, lock_tap, q);  // :784-787
+        // "previously returned H" (:446) carries over from the other half
+        CK(cudaMemcpyAsync(lock_h, s->lock_h.as<double>() + 9 * (slot ^ 1), sizeof(double) * 9, cudaMemcpyDeviceToDevice, q));
+        if (!L.match(g, frame, g.pitch, slot, is_orb, ref, q)) { s->err = kL2MapErr; return VSTAB_ERR_CUDA; }
+        launch_lock_update(L.Tfit(), L.fitc(), ref.count, L.ncur(), L.nmatch(), 0, lock_h, lock_tap, q);  // :784-787
     }
     CK(cudaGetLastError());
     return VSTAB_OK;
@@ -963,8 +1028,6 @@ void vstab_destroy(vstab_t* s) {
     if (s->pre_stream) { cudaStreamSynchronize(s->pre_stream); cudaStreamDestroy(s->pre_stream); }
     if (s->ev_pre) cudaEventDestroy(s->ev_pre);
     if (s->ev_chain) cudaEventDestroy(s->ev_chain);
-    if (s->orb) orb_plan_destroy(s->orb);
-    if (s->sift) sift_plan_destroy(s->sift);
     for (auto& set : s->tev) for (auto& e : set) if (e) cudaEventDestroy(e);     // VSTAB_TRACE marks
     delete s;
 }
@@ -1124,7 +1187,7 @@ long vstab_read_tap(vstab_t* s, int tap, void* dst, size_t dst_bytes) {
         case VSTAB_TAP_INLIERS: if (last == 0) return 0; return copy(s->fitc.p, sizeof(int) * 2, 2);
         case VSTAB_TAP_LOCK_H: if (!s->lock_h.p) return 0; return copy(s->lock_h.as<double>() + 9 * s->lock_slot, sizeof(double) * 9, 9);
         case VSTAB_TAP_ORB_COUNTS: if (!s->lock_tap.p) return 0; return copy(s->lock_tap.as<int>() + 8 * s->lock_slot, sizeof(int) * 5, 5);
-        case VSTAB_TAP_FEAT_GRAY: if (!s->feat_gray.p) return 0; return copy(s->feat_gray.as<uint8_t>() + (size_t)s->lock_slot * g.ww * g.wh, (size_t)g.ww * g.wh, (long)g.ww * g.wh);
+        case VSTAB_TAP_FEAT_GRAY: if (!s->reg.feat_gray.p) return 0; return copy(s->reg.gray(g, s->lock_slot), (size_t)g.ww * g.wh, (long)g.ww * g.wh);
         case VSTAB_TAP_CHANNEL_SUMS:
             return copy(s->sums.as<unsigned long long>() + (s->last_presented % s->W) * 3, sizeof(unsigned long long) * 3, 3);
     }
@@ -1153,24 +1216,14 @@ struct vstab_offline {
     DevBuf clip, outbuf, clipT, clipSums;
     size_t clip_frames = 0;
     cudaStream_t copy_in = nullptr, copy_out = nullptr;
-    // ORB / SIFT registration (offline): reference set, per-launch scratch, gathered registrations
-    OrbPlan* orb = nullptr;
-    SiftPlan* sift = nullptr;
+    // ORB / SIFT registration (offline): packed reference set (RefSet) and its mode, gathered registrations
     int ref_mode = -1;
-    DevBuf feat_ws, feat_gray, nn_x, nn_y, ref_pack, cur_kps, cur_desc, f_counts, m_idx, m_d0, m_d1, m_good, m_ref, m_cur,
-        m_status, lock_fit;
+    DevBuf ref_pack;
     const double* reg_all = nullptr;
     long reg_n = 0;
-    // extra registration lanes: frames of a shard are independent units, so vstab_offline_register deals them round-robin
-    // to lanes with their own stream, plan and scratch (lane 0 = the members above on `stream`)
-    struct RegLane {
-        cudaStream_t q = nullptr;
-        cudaEvent_t done = nullptr;
-        OrbPlan* orb = nullptr;
-        SiftPlan* sift = nullptr;
-        DevBuf feat_ws, feat_gray, cur_kps, cur_desc, f_counts, m_idx, m_d0, m_d1, m_good, m_ref, m_cur, m_status, lock_fit;
-    };
-    std::vector<RegLane*> lanes;
+    // registration lanes: frames of a shard are independent units, so vstab_offline_register deals them round-robin to
+    // lanes; lane 0 runs on `stream` (it also captures the reference set), every other one on a stream of its own
+    std::vector<std::unique_ptr<RegLane>> lanes;
     cudaEvent_t ev_reg_fork = nullptr;
     // sharded job (vstab_offline_run): NCCL communicator of this rank, chunk buffers kept between runs
     void* comm = nullptr;
@@ -1187,36 +1240,35 @@ struct vstab_offline {
     void set_err(const std::string& e) { err = e; }
 };
 
-// packed reference set: {int count, pad to 16 B} {OrbKeypoint[kOrbMaxKp]} {u8 desc[kOrbMaxKp][128]}
-static constexpr size_t kRefPackKps = 16;
-static constexpr size_t kRefPackDesc = kRefPackKps + sizeof(OrbKeypoint) * kOrbMaxKp;
-static constexpr size_t kRefPackBytes = kRefPackDesc + (size_t)128 * kOrbMaxKp;
+// the first K registration lanes, set up for `mode`
+static vstab_status offline_lanes(vstab_offline* o, int mode, int K) {
+    auto set_err = [&](const std::string& e) { o->err = e; };
+    while ((int)o->lanes.size() < K) {
+        std::unique_ptr<RegLane> L(new (std::nothrow) RegLane());
+        if (!L) { o->err = "out of memory"; return VSTAB_ERR_CUDA; }
+        if (!o->lanes.empty()) {
+            CK(cudaStreamCreateWithFlags(&L->q, cudaStreamNonBlocking));
+            CK(cudaEventCreateWithFlags(&L->done, cudaEventDisableTiming));
+        }
+        o->lanes.push_back(std::move(L));
+    }
+    for (int k = 0; k < K; ++k) {
+        RegLane& L = *o->lanes[k];
+        vstab_status st = L.setup(o->g, mode, 1, L.q ? L.q : o->stream, o->err);
+        if (st != VSTAB_OK) return st;
+    }
+    return VSTAB_OK;
+}
 
+// the reference set and lane 0 (which captures it) for `mode`
 static vstab_status offline_feature_setup(vstab_offline* o, int mode) {
     auto set_err = [&](const std::string& e) { o->err = e; };
-    Geometry& g = o->g;
     if (mode != VSTAB_ORB_FULL_LOCK && mode != VSTAB_SIFT_FULL_LOCK) { o->err = "mode must be ORB_FULL_LOCK or SIFT_FULL_LOCK"; return VSTAB_ERR_INVALID_ARGUMENT; }
-    if (!o->feat_ws.p) {
-        std::vector<int> xo(g.ww), yo(g.wh);
-        build_nn_table(g.cols, g.ww, xo.data());
-        build_nn_table(g.rows, g.wh, yo.data());
-        CK(o->feat_ws.alloc(featprep_workspace_bytes(g.ww, g.wh)));
-        CK(o->feat_gray.alloc((size_t)g.ww * g.wh));
-        CK(o->nn_x.alloc(sizeof(int) * g.ww)); CK(o->nn_y.alloc(sizeof(int) * g.wh));
-        CK(cudaMemcpy(o->nn_x.p, xo.data(), sizeof(int) * g.ww, cudaMemcpyHostToDevice));
-        CK(cudaMemcpy(o->nn_y.p, yo.data(), sizeof(int) * g.wh, cudaMemcpyHostToDevice));
+    if (!o->ref_pack.p) {
         CK(o->ref_pack.alloc(kRefPackBytes));
-        CK(o->cur_kps.alloc(sizeof(OrbKeypoint) * kOrbMaxKp)); CK(o->cur_desc.alloc(128 * kOrbMaxKp));
-        CK(o->f_counts.alloc(sizeof(int) * 4));
-        CK(o->m_idx.alloc(4 * kOrbMaxKp)); CK(o->m_d0.alloc(4 * kOrbMaxKp)); CK(o->m_d1.alloc(l2_match_scratch_bytes(kOrbMaxKp, 1)));
-        CK(o->m_good.alloc(kOrbMaxKp)); CK(o->m_status.alloc(kOrbMaxKp));
-        CK(o->m_ref.alloc(sizeof(float2) * kOrbMaxKp)); CK(o->m_cur.alloc(sizeof(float2) * kOrbMaxKp));
-        CK(o->lock_fit.alloc(sizeof(double) * 16 + sizeof(int) * 4));
-        CK(cudaMemset(o->ref_pack.p, 0, kRefPackBytes));
+        CK(cudaMemsetAsync(o->ref_pack.p, 0, kRefPackBytes, o->stream));
     }
-    if (mode == VSTAB_ORB_FULL_LOCK && !o->orb) { o->orb = orb_plan_create(g.ww, g.wh, 0.10, kOrbMaxKp, &o->err); if (!o->orb) return VSTAB_ERR_CUDA; }
-    if (mode == VSTAB_SIFT_FULL_LOCK && !o->sift) { o->sift = sift_plan_create(g.ww, g.wh, 0.05, kOrbMaxKp, &o->err); if (!o->sift) return VSTAB_ERR_CUDA; }
-    return VSTAB_OK;
+    return offline_lanes(o, mode, 1);
 }
 
 extern "C" {
@@ -1232,14 +1284,7 @@ vstab_status vstab_offline_reference_capture(vstab_offline_t* o, const uint8_t* 
     CK(cudaSetDevice(o->device));
     vstab_status st = offline_feature_setup(o, mode);
     if (st != VSTAB_OK) return st;
-    Geometry& g = o->g;
-    cudaStream_t q = o->stream;
-    char* pack = o->ref_pack.as<char>();
-    launch_featprep(d_frame, step, o->nn_x.as<int>(), o->nn_y.as<int>(), g.ww, g.wh, o->feat_ws.p, o->feat_gray.as<uint8_t>(), q);
-    if (mode == VSTAB_ORB_FULL_LOCK)
-        launch_orb(o->orb, o->feat_gray.as<uint8_t>(), (OrbKeypoint*)(pack + kRefPackKps), (uint8_t*)(pack + kRefPackDesc), (int*)pack, true, q);
-    else
-        launch_sift(o->sift, o->feat_gray.as<uint8_t>(), (OrbKeypoint*)(pack + kRefPackKps), (uint8_t*)(pack + kRefPackDesc), (int*)pack, q);
+    o->lanes[0]->capture(o->g, d_frame, step, 0, mode == VSTAB_ORB_FULL_LOCK, RefSet(o->ref_pack.p), o->stream);
     CK(cudaGetLastError());
     o->ref_mode = mode;
     return VSTAB_OK;
@@ -1273,78 +1318,30 @@ vstab_status vstab_offline_register(vstab_offline_t* o, const uint8_t* d_frames,
     auto set_err = [&](const std::string& e) { o->err = e; };
     if (o->ref_mode != VSTAB_ORB_FULL_LOCK && o->ref_mode != VSTAB_SIFT_FULL_LOCK) { o->err = "no reference set: call vstab_offline_reference_capture / _import first"; return VSTAB_ERR_STATE; }
     CK(cudaSetDevice(o->device));
-    Geometry& g = o->g;
     cudaStream_t q = o->stream;
-    char* pack = o->ref_pack.as<char>();
-    const int* nref = (const int*)pack;
-    const OrbKeypoint* ref_kps = (const OrbKeypoint*)(pack + kRefPackKps);
-    const uint8_t* ref_desc = (const uint8_t*)(pack + kRefPackDesc);
+    const RefSet ref(o->ref_pack.p);
     const bool is_orb = o->ref_mode == VSTAB_ORB_FULL_LOCK;
     // lanes: the ORB front end is ~44 small dependent launches per frame, SIFT at 4K mostly large ones (and 1.1 GB of pyramid per
     // lane).  Measured on B200, complete offline pass, frames/s with 1 / 2 / 3 / 4 / 8 lanes: ORB 1080p 1950 / - / 2834 / 2981 / 3117,
     // SIFT 4K 442 / 511 / 531 / - / 563.
     int K = is_orb ? 8 : 4;
     if (K > n) K = n;
-    while ((int)o->lanes.size() < K - 1) {
-        auto* L = new (std::nothrow) vstab_offline::RegLane();
-        if (!L) { o->err = "out of memory"; return VSTAB_ERR_CUDA; }
-        o->lanes.push_back(L);
-        CK(cudaStreamCreateWithFlags(&L->q, cudaStreamNonBlocking));
-        CK(cudaEventCreateWithFlags(&L->done, cudaEventDisableTiming));
-        CK(L->feat_ws.alloc(featprep_workspace_bytes(g.ww, g.wh)));
-        CK(L->feat_gray.alloc((size_t)g.ww * g.wh));
-        CK(L->cur_kps.alloc(sizeof(OrbKeypoint) * kOrbMaxKp)); CK(L->cur_desc.alloc(128 * kOrbMaxKp));
-        CK(L->f_counts.alloc(sizeof(int) * 4));
-        CK(L->m_idx.alloc(4 * kOrbMaxKp)); CK(L->m_d0.alloc(4 * kOrbMaxKp)); CK(L->m_d1.alloc(l2_match_scratch_bytes(kOrbMaxKp, 1)));
-        CK(L->m_good.alloc(kOrbMaxKp)); CK(L->m_status.alloc(kOrbMaxKp));
-        CK(L->m_ref.alloc(sizeof(float2) * kOrbMaxKp)); CK(L->m_cur.alloc(sizeof(float2) * kOrbMaxKp));
-        CK(L->lock_fit.alloc(sizeof(double) * 16 + sizeof(int) * 4));
-    }
-    for (int k = 1; k < K; ++k) {
-        auto* L = o->lanes[k - 1];
-        if (is_orb && !L->orb) { L->orb = orb_plan_create(g.ww, g.wh, 0.10, kOrbMaxKp, &o->err); if (!L->orb) return VSTAB_ERR_CUDA; }
-        if (!is_orb && !L->sift) { L->sift = sift_plan_create(g.ww, g.wh, 0.05, kOrbMaxKp, &o->err); if (!L->sift) return VSTAB_ERR_CUDA; }
-    }
+    vstab_status st = offline_lanes(o, o->ref_mode, K);
+    if (st != VSTAB_OK) return st;
     if (K > 1) {
         if (!o->ev_reg_fork) CK(cudaEventCreateWithFlags(&o->ev_reg_fork, cudaEventDisableTiming));
         CK(cudaEventRecord(o->ev_reg_fork, q));                       // reference set, frames: ordered before every lane
-        for (int k = 1; k < K; ++k) CK(cudaStreamWaitEvent(o->lanes[k - 1]->q, o->ev_reg_fork, 0));
+        for (int k = 1; k < K; ++k) CK(cudaStreamWaitEvent(o->lanes[k]->q, o->ev_reg_fork, 0));
     }
     for (int i = 0; i < n; ++i) {
-        const int k = i % K;
-        vstab_offline::RegLane* L = k ? o->lanes[k - 1] : nullptr;
-        cudaStream_t ql = L ? L->q : q;
-        void* feat_ws = L ? L->feat_ws.p : o->feat_ws.p;
-        uint8_t* feat_gray = (L ? L->feat_gray : o->feat_gray).as<uint8_t>();
-        OrbKeypoint* cur_kps = (L ? L->cur_kps : o->cur_kps).as<OrbKeypoint>();
-        uint8_t* cur_desc = (L ? L->cur_desc : o->cur_desc).as<uint8_t>();
-        int* counts = (L ? L->f_counts : o->f_counts).as<int>();
-        int* m_idx = (L ? L->m_idx : o->m_idx).as<int>();
-        int* m_d0 = (L ? L->m_d0 : o->m_d0).as<int>();
-        int* m_d1 = (L ? L->m_d1 : o->m_d1).as<int>();
-        uint8_t* m_good = (L ? L->m_good : o->m_good).as<uint8_t>();
-        float2* m_ref = (L ? L->m_ref : o->m_ref).as<float2>();
-        float2* m_cur = (L ? L->m_cur : o->m_cur).as<float2>();
-        uint8_t* m_status = (L ? L->m_status : o->m_status).as<uint8_t>();
-        double* Tfit = (L ? L->lock_fit : o->lock_fit).as<double>();
-        int* fitc = reinterpret_cast<int*>(Tfit + 16);
-        const uint8_t* frame = d_frames + (size_t)i * frame_stride;
-        launch_featprep(frame, step, o->nn_x.as<int>(), o->nn_y.as<int>(), g.ww, g.wh, feat_ws, feat_gray, ql);
-        if (is_orb) {
-            launch_orb(L ? L->orb : o->orb, feat_gray, cur_kps, cur_desc, counts + 1, false, ql);
-            launch_hamming_match(ref_desc, nref, ref_kps, cur_desc, counts + 1, cur_kps, kOrbMaxKp, 0.6f, m_idx, m_d0, m_d1, m_good,
-                                 m_ref, m_cur, m_status, counts + 2, ql);
-        } else {
-            launch_sift(L ? L->sift : o->sift, feat_gray, cur_kps, cur_desc, counts + 1, ql);
-            if (!launch_l2_match(ref_desc, nref, ref_kps, cur_desc, counts + 1, cur_kps, kOrbMaxKp, m_d1, m_idx, m_d0, m_good, m_ref,
-                                 m_cur, m_status, counts + 2, ql)) { o->err = kL2MapErr; return VSTAB_ERR_CUDA; }
-        }
-        launch_fit_large(m_ref, m_cur, m_status, counts + 2, 5.0, g.ww / 2.0, g.wh / 2.0, Tfit, Tfit + 9, fitc, ql);
-        launch_reg_store(Tfit, fitc, nref, counts + 1, counts + 2, d_reg + (size_t)i * 10, ql);
+        RegLane& L = *o->lanes[i % K];
+        cudaStream_t ql = L.q ? L.q : q;
+        if (!L.match(o->g, d_frames + (size_t)i * frame_stride, step, 0, is_orb, ref, ql)) { o->err = kL2MapErr; return VSTAB_ERR_CUDA; }
+        launch_reg_store(L.Tfit(), L.fitc(), ref.count, L.ncur(), L.nmatch(), d_reg + (size_t)i * 10, ql);
     }
     for (int k = 1; k < K; ++k) {
-        CK(cudaEventRecord(o->lanes[k - 1]->done, o->lanes[k - 1]->q));
-        CK(cudaStreamWaitEvent(q, o->lanes[k - 1]->done, 0));
+        CK(cudaEventRecord(o->lanes[k]->done, o->lanes[k]->q));
+        CK(cudaStreamWaitEvent(q, o->lanes[k]->done, 0));
     }
     CK(cudaGetLastError());
     return VSTAB_OK;
@@ -1398,15 +1395,6 @@ void vstab_offline_destroy(vstab_offline_t* o) {
     if (o->stream) { cudaStreamSynchronize(o->stream); cudaStreamDestroy(o->stream); }
     if (o->copy_in) { cudaStreamSynchronize(o->copy_in); cudaStreamDestroy(o->copy_in); }
     if (o->copy_out) { cudaStreamSynchronize(o->copy_out); cudaStreamDestroy(o->copy_out); }
-    if (o->orb) orb_plan_destroy(o->orb);
-    if (o->sift) sift_plan_destroy(o->sift);
-    for (auto* L : o->lanes) {
-        if (L->q) { cudaStreamSynchronize(L->q); cudaStreamDestroy(L->q); }
-        if (L->done) cudaEventDestroy(L->done);
-        if (L->orb) orb_plan_destroy(L->orb);
-        if (L->sift) sift_plan_destroy(L->sift);
-        delete L;
-    }
     if (o->ev_reg_fork) cudaEventDestroy(o->ev_reg_fork);
     if (o->comm) nccl_comm_destroy(o->comm);
     for (auto e : o->host_events) if (e) cudaEventDestroy(e);
@@ -2507,38 +2495,36 @@ extern "C" vstab_status vstab_k_featprep(int device, const uint8_t* bgr, int row
     Geometry g;
     vstab_status st = g.init(rows, cols, working_height, g_err);
     if (st != VSTAB_OK) return st;
-    std::vector<int> xo(g.ww), yo(g.wh);
-    build_nn_table(cols, g.ww, xo.data());
-    build_nn_table(rows, g.wh, yo.data());
-    DevBuf frame, ws, out, dx, dy;
+    DevBuf frame, ws, out;
     CK(frame.alloc(g.frame_bytes + 64));
     CK(ws.alloc(featprep_workspace_bytes(g.ww, g.wh)));
     CK(out.alloc((size_t)g.ww * g.wh));
-    CK(dx.alloc(sizeof(int) * g.ww)); CK(dy.alloc(sizeof(int) * g.wh));
+    CK(g.nn_tables());
     CK(cudaMemcpy2D(frame.p, g.pitch, bgr, step, (size_t)cols * 3, rows, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(dx.p, xo.data(), sizeof(int) * g.ww, cudaMemcpyHostToDevice));
-    CK(cudaMemcpy(dy.p, yo.data(), sizeof(int) * g.wh, cudaMemcpyHostToDevice));
-    launch_featprep(frame.as<uint8_t>(), g.pitch, dx.as<int>(), dy.as<int>(), g.ww, g.wh, ws.p, out.as<uint8_t>(), 0);
+    launch_featprep(frame.as<uint8_t>(), g.pitch, g.nn_x.as<int>(), g.nn_y.as<int>(), g.ww, g.wh, ws.p, out.as<uint8_t>(), 0);
     CK(cudaGetLastError());
     CK(cudaMemcpy(gray_out, out.p, (size_t)g.ww * g.wh, cudaMemcpyDeviceToHost));
     return VSTAB_OK;
 }
 
-extern "C" vstab_status vstab_k_orb(int device, const uint8_t* gray, int rows, int cols, double size_ratio,
-                                    int reference_order, float* kps_out, uint8_t* desc_out, int* n_out, int max_out) {
-    auto set_err = [&](const std::string& e) { g_err = e; };
+// vstab_k_orb / vstab_k_sift: one detector run on a host gray image.  `launch(plan, img, kps, desc, count)` enqueues it on
+// the default stream; keypoints come out as {x, y, size, angle, response, octave} floats, descriptors `width` bytes each.
+template <class Plan, class Launch>
+static vstab_status k_detect(int device, Plan* (*create)(int, int, double, int, std::string*), void (*destroy)(Plan*),
+                             const char* name, int width, const uint8_t* gray, int rows, int cols, double size_ratio,
+                             float* kps_out, uint8_t* desc_out, int* n_out, int max_out, Launch&& launch) {
     if (!gray || !kps_out || !desc_out || !n_out || max_out < 1) return VSTAB_ERR_INVALID_ARGUMENT;
     if (!device_ok(device, g_err)) return VSTAB_ERR_CUDA;
-    OrbPlan* P = orb_plan_create(cols, rows, size_ratio, kOrbMaxKp, &g_err);
+    Plan* P = create(cols, rows, size_ratio, kOrbMaxKp, &g_err);
     if (!P) return VSTAB_ERR_CUDA;
     DevBuf img, kps, desc, cnt;
     vstab_status st = VSTAB_OK;
-    auto fail = [&](const char* m) { g_err = m; st = VSTAB_ERR_CUDA; };
+    auto fail = [&](const std::string& m) { g_err = m; st = VSTAB_ERR_CUDA; };
     if (img.alloc((size_t)rows * cols) != cudaSuccess || kps.alloc(sizeof(OrbKeypoint) * kOrbMaxKp) != cudaSuccess ||
-        desc.alloc(32 * kOrbMaxKp) != cudaSuccess || cnt.alloc(sizeof(int)) != cudaSuccess) fail("cudaMalloc failed");
+        desc.alloc((size_t)width * kOrbMaxKp) != cudaSuccess || cnt.alloc(sizeof(int)) != cudaSuccess) fail("cudaMalloc failed");
     if (st == VSTAB_OK) {
         cudaMemcpy(img.p, gray, (size_t)rows * cols, cudaMemcpyHostToDevice);
-        launch_orb(P, img.as<uint8_t>(), kps.as<OrbKeypoint>(), desc.as<uint8_t>(), cnt.as<int>(), reference_order != 0, 0);
+        launch(P, img.as<uint8_t>(), kps.as<OrbKeypoint>(), desc.as<uint8_t>(), cnt.as<int>());
         int n = 0;
         if (cudaMemcpy(&n, cnt.p, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess) fail(cudaGetErrorString(cudaGetLastError()));
         if (st == VSTAB_OK) {
@@ -2547,16 +2533,24 @@ extern "C" vstab_status vstab_k_orb(int device, const uint8_t* gray, int rows, i
             *n_out = n;
             std::vector<OrbKeypoint> h(n);
             cudaMemcpy(h.data(), kps.p, sizeof(OrbKeypoint) * n, cudaMemcpyDeviceToHost);
-            cudaMemcpy(desc_out, desc.p, (size_t)32 * n, cudaMemcpyDeviceToHost);
+            cudaMemcpy(desc_out, desc.p, (size_t)width * n, cudaMemcpyDeviceToHost);
             for (int i = 0; i < n; ++i) {
                 float* o = kps_out + (size_t)i * 6;
                 o[0] = h[i].x; o[1] = h[i].y; o[2] = h[i].size; o[3] = h[i].angle; o[4] = h[i].response; o[5] = (float)h[i].octave;
             }
-            if (cudaGetLastError() != cudaSuccess) fail("CUDA failure in vstab_k_orb");
+            if (cudaGetLastError() != cudaSuccess) fail(std::string("CUDA failure in ") + name);
         }
     }
-    orb_plan_destroy(P);
+    destroy(P);
     return st;
+}
+
+extern "C" vstab_status vstab_k_orb(int device, const uint8_t* gray, int rows, int cols, double size_ratio,
+                                    int reference_order, float* kps_out, uint8_t* desc_out, int* n_out, int max_out) {
+    return k_detect(device, orb_plan_create, orb_plan_destroy, "vstab_k_orb", 32, gray, rows, cols, size_ratio, kps_out, desc_out,
+                    n_out, max_out, [&](OrbPlan* P, const uint8_t* img, OrbKeypoint* k, uint8_t* d, int* c) {
+                        launch_orb(P, img, k, d, c, reference_order != 0, 0);
+                    });
 }
 
 extern "C" vstab_status vstab_k_hamming(int device, const uint8_t* ref, int nref, const uint8_t* cur, int ncur, float ratio,
@@ -2657,35 +2651,8 @@ extern "C" vstab_status vstab_k_l2match_batch(int device, const uint8_t* ref, in
 
 extern "C" vstab_status vstab_k_sift(int device, const uint8_t* gray, int rows, int cols, double size_ratio,
                                      float* kps_out, uint8_t* desc_out, int* n_out, int max_out) {
-    auto set_err = [&](const std::string& e) { g_err = e; };
-    if (!gray || !kps_out || !desc_out || !n_out || max_out < 1) return VSTAB_ERR_INVALID_ARGUMENT;
-    if (!device_ok(device, g_err)) return VSTAB_ERR_CUDA;
-    SiftPlan* P = sift_plan_create(cols, rows, size_ratio, kOrbMaxKp, &g_err);
-    if (!P) return VSTAB_ERR_CUDA;
-    DevBuf img, kps, desc, cnt;
-    vstab_status st = VSTAB_OK;
-    auto fail = [&](const char* m) { g_err = m; st = VSTAB_ERR_CUDA; };
-    if (img.alloc((size_t)rows * cols) != cudaSuccess || kps.alloc(sizeof(OrbKeypoint) * kOrbMaxKp) != cudaSuccess ||
-        desc.alloc(128 * kOrbMaxKp) != cudaSuccess || cnt.alloc(sizeof(int)) != cudaSuccess) fail("cudaMalloc failed");
-    if (st == VSTAB_OK) {
-        cudaMemcpy(img.p, gray, (size_t)rows * cols, cudaMemcpyHostToDevice);
-        launch_sift(P, img.as<uint8_t>(), kps.as<OrbKeypoint>(), desc.as<uint8_t>(), cnt.as<int>(), 0);
-        int n = 0;
-        if (cudaMemcpy(&n, cnt.p, sizeof(int), cudaMemcpyDeviceToHost) != cudaSuccess) fail(cudaGetErrorString(cudaGetLastError()));
-        if (st == VSTAB_OK) {
-            if (n > kOrbMaxKp) n = kOrbMaxKp;
-            if (n > max_out) n = max_out;
-            *n_out = n;
-            std::vector<OrbKeypoint> h(n);
-            cudaMemcpy(h.data(), kps.p, sizeof(OrbKeypoint) * n, cudaMemcpyDeviceToHost);
-            cudaMemcpy(desc_out, desc.p, (size_t)128 * n, cudaMemcpyDeviceToHost);
-            for (int i = 0; i < n; ++i) {
-                float* o = kps_out + (size_t)i * 6;
-                o[0] = h[i].x; o[1] = h[i].y; o[2] = h[i].size; o[3] = h[i].angle; o[4] = h[i].response; o[5] = (float)h[i].octave;
-            }
-            if (cudaGetLastError() != cudaSuccess) fail("CUDA failure in vstab_k_sift");
-        }
-    }
-    sift_plan_destroy(P);
-    return st;
+    return k_detect(device, sift_plan_create, sift_plan_destroy, "vstab_k_sift", 128, gray, rows, cols, size_ratio, kps_out, desc_out,
+                    n_out, max_out, [](SiftPlan* P, const uint8_t* img, OrbKeypoint* k, uint8_t* d, int* c) {
+                        launch_sift(P, img, k, d, c, 0);
+                    });
 }

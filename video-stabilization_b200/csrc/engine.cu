@@ -19,6 +19,7 @@
 #include <cstdio>
 #include <cstring>
 #include <new>
+#include <optional>
 #include <string>
 #include <vector>
 
@@ -329,6 +330,114 @@ cudaError_t yuv_copy(uint8_t* dst, const vstab_yuv_layout& dl, size_t dst_fs, co
     return cudaSuccess;
 }
 
+// n BGR frames between two pitched layouts, one cudaMemcpy2DAsync per frame -- or ONE copy when neither side has a byte
+// between rows or frames (the rule of yuv_copy)
+cudaError_t bgr_copy(uint8_t* dst, size_t dst_step, size_t dst_fs, const uint8_t* src, size_t src_step, size_t src_fs, long n,
+                     int rows, int cols, cudaMemcpyKind kind, cudaStream_t q) {
+    const size_t rb = (size_t)cols * 3, packed = rb * (size_t)rows;
+    if (dst_step == rb && src_step == rb && (n == 1 || (dst_fs == packed && src_fs == packed)))
+        return cudaMemcpyAsync(dst, src, packed * (size_t)n, kind, q);
+    for (long i = 0; i < n; ++i) {
+        const cudaError_t e = cudaMemcpy2DAsync(dst + (size_t)i * dst_fs, dst_step, src + (size_t)i * src_fs, src_step, rb, rows, kind, q);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
+// ---- caller frames <-> the library's BGR frames (g.pitch bytes per row, g.frame_bytes per frame) ------------------------
+// Every entry point moves its caller's frames in and out through the functions below.  Each direction has two phases, so
+// that the copy and the conversion can run on different streams: input = transfer (BGR straight into the library's frames,
+// host YUV into a staging buffer in the library's plane layout) then convert (YUV -> BGR); output = convert (BGR -> YUV, into
+// staging for host memory, into the caller's frames for device memory) then transfer.  Device YUV frames are converted
+// where they are.  Copies never touch the caller's bytes between rows, planes or frames.
+struct FrameFmt {
+    bool host = true;                          // host memory, else device memory
+    const vstab_yuv_layout* yuv = nullptr;     // YUV 4:2:0 planes; null: BGR rows `step` bytes apart
+    size_t step = 0;
+    size_t stride = 0;                         // bytes from one frame of a run to the next
+
+    // device BGR: the library reads and writes these frames where they are
+    bool direct() const { return !host && !yuv; }
+    // device bytes per frame of the staging buffer the transfer goes through (host YUV only), enough for either YUV format
+    size_t staging_bytes(const Geometry& g) const { return host && yuv ? yuv_staging_bytes(g.rows, g.cols) : 0; }
+    // `runs`: frames of a run sit `stride` bytes apart and must not overlap
+    vstab_status check(int rows, int cols, bool runs, std::string& err, const char* step_err = "row step smaller than 3*cols") const {
+        if (!yuv) {
+            if (step >= (size_t)cols * 3) return VSTAB_OK;
+            err = step_err;
+            return VSTAB_ERR_INVALID_ARGUMENT;
+        }
+        const size_t extent = yuv_extent(yuv, rows, cols, err);
+        if (!extent) return VSTAB_ERR_INVALID_ARGUMENT;
+        if (runs && stride < extent) { err = "frame stride smaller than the extent of the YUV layout's planes"; return VSTAB_ERR_INVALID_ARGUMENT; }
+        return VSTAB_OK;
+    }
+    // the staging frames of a host YUV format: the library's plane layout, `*fs` bytes apart
+    vstab_yuv_layout staging(const Geometry& g, size_t* fs) const { return yuv_staging_layout(yuv->format, g.rows, g.cols, fs); }
+};
+
+// input, transfer: n caller frames at `src` -> BGR frames at `dst` (BGR), or -> `stage` (host YUV)
+cudaError_t frames_in_transfer(const Geometry& g, const FrameFmt& f, const uint8_t* src, long n, uint8_t* dst, uint8_t* stage,
+                               cudaStream_t q) {
+    if (!f.yuv)
+        return bgr_copy(dst, g.pitch, g.frame_bytes, src, f.step, f.stride, n, g.rows, g.cols,
+                        f.host ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, q);
+    if (!f.host) return cudaSuccess;
+    size_t sfs = 0;
+    const vstab_yuv_layout S = f.staging(g, &sfs);
+    return yuv_copy(stage, S, sfs, src, *f.yuv, f.stride, n, g.rows, g.cols, cudaMemcpyHostToDevice, q);
+}
+
+// input, convert: YUV -> BGR frames at `dst`, from `stage` (host) or from the caller's frames at `src` (device)
+cudaError_t frames_in_convert(const Geometry& g, const FrameFmt& f, const uint8_t* src, long n, uint8_t* dst, const uint8_t* stage,
+                              cudaStream_t q) {
+    if (!f.yuv) return cudaSuccess;
+    if (f.host) {
+        size_t sfs = 0;
+        const vstab_yuv_layout S = f.staging(g, &sfs);
+        launch_yuv420_to_bgr(stage, yuv_planes_of(S), sfs, (int)n, g.rows, g.cols, dst, g.pitch, g.frame_bytes, q);
+    } else {
+        launch_yuv420_to_bgr(src, yuv_planes_of(*f.yuv), f.stride, (int)n, g.rows, g.cols, dst, g.pitch, g.frame_bytes, q);
+    }
+    return cudaGetLastError();
+}
+
+cudaError_t frames_in(const Geometry& g, const FrameFmt& f, const uint8_t* src, long n, uint8_t* dst, uint8_t* stage, cudaStream_t q) {
+    const cudaError_t e = frames_in_transfer(g, f, src, n, dst, stage, q);
+    return e != cudaSuccess ? e : frames_in_convert(g, f, src, n, dst, stage, q);
+}
+
+// output, convert: BGR frames at `src` -> YUV, into `stage` (host) or into the caller's frames at `dst` (device)
+cudaError_t frames_out_convert(const Geometry& g, const FrameFmt& f, const uint8_t* src, long n, uint8_t* dst, uint8_t* stage,
+                               cudaStream_t q) {
+    if (!f.yuv) return cudaSuccess;
+    if (f.host) {
+        size_t sfs = 0;
+        const vstab_yuv_layout S = f.staging(g, &sfs);
+        launch_bgr_to_yuv420(src, g.pitch, g.frame_bytes, (int)n, g.rows, g.cols, stage, yuv_planes_of(S), sfs, q);
+    } else {
+        launch_bgr_to_yuv420(src, g.pitch, g.frame_bytes, (int)n, g.rows, g.cols, dst, yuv_planes_of(*f.yuv), f.stride, q);
+    }
+    return cudaGetLastError();
+}
+
+// output, transfer: -> the caller's frames at `dst`, from the BGR frames at `src` (BGR) or from `stage` (host YUV)
+cudaError_t frames_out_transfer(const Geometry& g, const FrameFmt& f, const uint8_t* src, long n, uint8_t* dst, const uint8_t* stage,
+                                cudaStream_t q) {
+    if (!f.yuv)
+        return bgr_copy(dst, f.step, f.stride, src, g.pitch, g.frame_bytes, n, g.rows, g.cols,
+                        f.host ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, q);
+    if (!f.host) return cudaSuccess;
+    size_t sfs = 0;
+    const vstab_yuv_layout S = f.staging(g, &sfs);
+    return yuv_copy(dst, *f.yuv, f.stride, stage, S, sfs, n, g.rows, g.cols, cudaMemcpyDeviceToHost, q);
+}
+
+cudaError_t frames_out(const Geometry& g, const FrameFmt& f, const uint8_t* src, long n, uint8_t* dst, uint8_t* stage, cudaStream_t q) {
+    const cudaError_t e = frames_out_convert(g, f, src, n, dst, stage, q);
+    return e != cudaSuccess ? e : frames_out_transfer(g, f, src, n, dst, stage, q);
+}
+
 // ---- ORB / SIFT registration (stabilizer.cpp:440-787), shared by the streaming instance and the offline runner ---------
 // The reference set is one packed device buffer: {int count, pad to 16 B} {OrbKeypoint[kOrbMaxKp]} {u8 desc[kOrbMaxKp][128]},
 // so the offline ranks can broadcast it as it is.
@@ -483,7 +592,7 @@ struct vstab {
     bool trail = false;                     // copyFeathered branch of stabilizeFrame (:1303-1307)
     bool partial_fix = false;               // TRANSLATION_/ROTATION_LOCK fed with the accumulated lock (hpp:23 @todo)
     DevBuf trail_bg, trail_ws;              // trail_background_ (:129) and K14 scratch
-    // YUV calls with host buffers: the input planes are uploaded here (copy_stream) and converted into the ring, the
+    // staging of host YUV frames (FrameFmt): the input frame is uploaded here (copy_stream) and converted into the ring, the
     // presented BGR frame is converted here (out_stream) and downloaded.  One frame each: every use is ordered by its stream.
     DevBuf yuv_in, yuv_out;
     std::string err;
@@ -719,53 +828,17 @@ static vstab_status stream_output(vstab* s, long n, uint8_t* d_out, size_t out_p
     return VSTAB_OK;
 }
 
-// YUV input frame -> BGR ring slot on q: device frames are converted where they are, host frames uploaded first
-static vstab_status stream_yuv_in(vstab* s, const uint8_t* in, const vstab_yuv_layout& L, bool host, uint8_t* slot, cudaStream_t q) {
-    auto set_err = [&](const std::string& e) { s->err = e; };
-    Geometry& g = s->g;
-    if (!host) {
-        launch_yuv420_to_bgr(in, yuv_planes_of(L), 0, 1, g.rows, g.cols, slot, g.pitch, 0, q);
-    } else {
-        size_t fb = 0;
-        const vstab_yuv_layout S = yuv_staging_layout(L.format, g.rows, g.cols, &fb);
-        if (!s->yuv_in.p) CK(s->yuv_in.alloc(yuv_staging_bytes(g.rows, g.cols)));
-        CK(yuv_copy(s->yuv_in.as<uint8_t>(), S, fb, in, L, 0, 1, g.rows, g.cols, cudaMemcpyHostToDevice, q));
-        launch_yuv420_to_bgr(s->yuv_in.as<uint8_t>(), yuv_planes_of(S), fb, 1, g.rows, g.cols, slot, g.pitch, 0, q);
-    }
-    CK(cudaGetLastError());
-    return VSTAB_OK;
-}
-
-// presented BGR frame -> YUV output frame on out_stream: into device memory directly, or through staging to host memory
-static vstab_status stream_yuv_out(vstab* s, const uint8_t* bgr, size_t pitch, uint8_t* out, const vstab_yuv_layout& L, bool host) {
-    auto set_err = [&](const std::string& e) { s->err = e; };
-    Geometry& g = s->g;
-    cudaStream_t q = s->out_stream;
-    if (!host) {
-        launch_bgr_to_yuv420(bgr, pitch, 0, 1, g.rows, g.cols, out, yuv_planes_of(L), 0, q);
-    } else {
-        size_t fb = 0;
-        const vstab_yuv_layout S = yuv_staging_layout(L.format, g.rows, g.cols, &fb);
-        if (!s->yuv_out.p) CK(s->yuv_out.alloc(yuv_staging_bytes(g.rows, g.cols)));
-        launch_bgr_to_yuv420(bgr, pitch, 0, 1, g.rows, g.cols, s->yuv_out.as<uint8_t>(), yuv_planes_of(S), fb, q);
-        CK(yuv_copy(out, L, 0, s->yuv_out.as<uint8_t>(), S, fb, 1, g.rows, g.cols, cudaMemcpyDeviceToHost, q));
-    }
-    CK(cudaGetLastError());
-    return VSTAB_OK;
-}
-
-// One stabilizeFrame call; `kind` selects how frame pixels move (host<->device or device<->device).  in_yuv / out_yuv:
-// layouts of YUV frames (null: BGR with `step` / `out_step`).
-static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols, size_t step, uint8_t* out,
-                                size_t out_step, cudaMemcpyKind in_kind, cudaMemcpyKind out_kind, bool host_wait,
-                                const vstab_yuv_layout* in_yuv = nullptr, const vstab_yuv_layout* out_yuv = nullptr) {
+// One stabilizeFrame call: frame `in` in the caller's format `in_fmt`, its output into `out` in `out_fmt`.  A call on host
+// frames returns when `out` is complete.
+static vstab_status stream_call(vstab* s, const uint8_t* in, const FrameFmt& in_fmt, uint8_t* out, const FrameFmt& out_fmt) {
     auto set_err = [&](const std::string& e) { s->err = e; };
     Geometry& g = s->g;
     uint8_t* slot = s->ring.as<uint8_t>() + (size_t)(s->n % s->W) * g.frame_bytes;
-    const size_t row_bytes = (size_t)cols * 3;
-    const bool device_out = out_kind == cudaMemcpyDeviceToDevice;
-    const bool direct_out = device_out && !out_yuv;     // the warp writes the caller's BGR buffer itself
+    const bool host_wait = in_fmt.host;
+    const bool direct_out = out_fmt.direct();          // the warp writes the caller's BGR buffer itself
     const bool out_first = s->n > 0 && s->F >= 1;      // output chain does not need this call's transform
+    if (!s->yuv_in.p && in_fmt.staging_bytes(g)) CK(s->yuv_in.alloc(in_fmt.staging_bytes(g)));
+    if (!s->yuv_out.p && out_fmt.staging_bytes(g)) CK(s->yuv_out.alloc(out_fmt.staging_bytes(g)));
     static const bool trace = getenv("VSTAB_TRACE") != nullptr;
     auto now_us = [] { return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
     const double tr0 = trace ? now_us() : 0.0;
@@ -787,13 +860,12 @@ static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols,
     };
     auto output_into = [&](long c, int slot, cudaStream_t q, bool ahead) -> vstab_status {
         uint8_t* dst = direct_out ? out : s->dout_at(slot);
-        return stream_output(s, c, dst, direct_out ? out_step : g.pitch, s->wp_at(slot), q, ahead);
+        return stream_output(s, c, dst, direct_out ? out_fmt.step : g.pitch, s->wp_at(slot), q, ahead);
     };
-    // YUV outputs are converted from whichever BGR half is presented (an output prepared one call ahead did not know the layout)
+    // the presented BGR half -> `out` on out_stream, unless the warp wrote it there (an output prepared one call ahead
+    // did not know the caller's format)
     auto copy_out = [&](int slot) -> vstab_status {
-        if (out_yuv) return stream_yuv_out(s, s->dout_at(slot), g.pitch, out, *out_yuv, !device_out);
-        if (!device_out)
-            CK(cudaMemcpy2DAsync(out, out_step, s->dout_at(slot), g.pitch, row_bytes, rows, out_kind, s->out_stream));
+        if (!direct_out) CK(frames_out(g, out_fmt, s->dout_at(slot), 1, out, s->yuv_out.as<uint8_t>(), s->out_stream));
         return VSTAB_OK;
     };
 
@@ -828,12 +900,7 @@ static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols,
     cudaStream_t up = s->copy_stream;
     if (s->n > 0) CK(cudaStreamWaitEvent(up, s->ev_out, 0));
     s->mark(0, up);
-    if (in_yuv) {
-        vstab_status sy = stream_yuv_in(s, in, *in_yuv, in_kind == cudaMemcpyHostToDevice, slot, up);
-        if (sy != VSTAB_OK) return sy;
-    } else {
-        CK(cudaMemcpy2DAsync(slot, g.pitch, in, step, row_bytes, rows, in_kind, up));
-    }
+    CK(frames_in(g, in_fmt, in, 1, slot, s->yuv_in.as<uint8_t>(), up));
     s->mark(1, up);
     CK(cudaEventRecord(s->ev_in, up));
     vstab_status st = stream_estimate(s);
@@ -842,12 +909,7 @@ static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols,
         if (s->n == 0) {
             // call 0 returns the input frame itself (:1181)
             CK(cudaStreamWaitEvent(s->out_stream, s->ev_in, 0));
-            if (out_yuv) {
-                st = stream_yuv_out(s, slot, g.pitch, out, *out_yuv, !device_out);
-                if (st != VSTAB_OK) return st;
-            } else {
-                CK(cudaMemcpy2DAsync(out, out_step, slot, g.pitch, row_bytes, rows, out_kind, s->out_stream));
-            }
+            CK(frames_out(g, out_fmt, slot, 1, out, s->yuv_out.as<uint8_t>(), s->out_stream));
             s->last_presented = 0;
         } else {
             CK(cudaStreamWaitEvent(s->out_stream, s->ev_fit[s->n & 7], 0));   // future == 0: needs T[n] of this call
@@ -862,7 +924,7 @@ static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols,
     }
     // the next call's output, beside this call's download (see pre_stream)
     const bool lk_mode = s->mode != VSTAB_ORB_FULL_LOCK && s->mode != VSTAB_SIFT_FULL_LOCK;
-    if (host_wait && !device_out && s->F >= 1 && lk_mode && !s->trail) {
+    if (host_wait && out_fmt.host && s->F >= 1 && lk_mode && !s->trail) {
         const long c = s->n + 1;
         if (in_call_chain) CK(cudaStreamWaitEvent(s->pre_stream, s->ev_chain, 0));
         CK(cudaStreamWaitEvent(s->pre_stream, fit_event(c), 0));
@@ -902,15 +964,18 @@ static vstab_status stream_call(vstab* s, const uint8_t* in, int rows, int cols,
     return VSTAB_OK;
 }
 
-static vstab_status stream_check_args(vstab* s, const void* in, int rows, int cols, size_t step, const void* out,
-                                      size_t out_step) {
+// The vstab_stabilize_frame* entry points: argument checks, device, set-up on the first call, then the call
+static vstab_status stream_entry(vstab* s, const uint8_t* in, const FrameFmt& in_fmt, int rows, int cols, uint8_t* out,
+                                 const FrameFmt& out_fmt) {
     if (!s) return VSTAB_ERR_INVALID_ARGUMENT;
     if (!in || !out) { s->err = "null image pointer"; return VSTAB_ERR_INVALID_ARGUMENT; }
     if (rows <= 10 || cols <= 10) {                                                                    // :99-103
         s->err = "Stabilizer: Frame has invalid size. Rows: " + std::to_string(rows) + ", Cols: " + std::to_string(cols);
         return VSTAB_ERR_INVALID_ARGUMENT;
     }
-    if (step < (size_t)cols * 3 || out_step < (size_t)cols * 3) { s->err = "row step smaller than 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
+    vstab_status st = in_fmt.check(rows, cols, false, s->err);
+    if (st == VSTAB_OK) st = out_fmt.check(rows, cols, false, s->err);
+    if (st != VSTAB_OK) return st;
     if (s->inited && (s->g.rows != rows || s->g.cols != cols)) {                                        // :110-112
         s->err = "Stabilizer: Frame size has changed. This is not supported.";
         return VSTAB_ERR_SIZE_CHANGED;
@@ -926,7 +991,10 @@ static vstab_status stream_check_args(vstab* s, const void* in, int rows, int co
             return VSTAB_ERR_STATE;
         }
     }
-    return VSTAB_OK;
+    auto set_err = [&](const std::string& e) { s->err = e; };
+    CK(cudaSetDevice(s->device));
+    if (!s->inited && (st = stream_init(s, rows, cols)) != VSTAB_OK) return st;
+    return stream_call(s, in, in_fmt, out, out_fmt);
 }
 
 extern "C" {
@@ -1068,23 +1136,12 @@ vstab_status vstab_synchronize(vstab_t* s) {
 
 vstab_status vstab_stabilize_frame(vstab_t* s, const uint8_t* bgr, int rows, int cols, size_t step,
                                    uint8_t* out_bgr, size_t out_step) {
-    vstab_status st = stream_check_args(s, bgr, rows, cols, step, out_bgr, out_step);
-    if (st != VSTAB_OK) return st;
-    auto set_err = [&](const std::string& e) { s->err = e; };
-    CK(cudaSetDevice(s->device));
-    if (!s->inited) { st = stream_init(s, rows, cols); if (st != VSTAB_OK) return st; }
-    return stream_call(s, bgr, rows, cols, step, out_bgr, out_step, cudaMemcpyHostToDevice, cudaMemcpyDeviceToHost, true);
+    return stream_entry(s, bgr, {true, nullptr, step}, rows, cols, out_bgr, {true, nullptr, out_step});
 }
 
 vstab_status vstab_stabilize_frame_device(vstab_t* s, const uint8_t* d_bgr, int rows, int cols, size_t step,
                                           uint8_t* d_out_bgr, size_t out_step) {
-    vstab_status st = stream_check_args(s, d_bgr, rows, cols, step, d_out_bgr, out_step);
-    if (st != VSTAB_OK) return st;
-    auto set_err = [&](const std::string& e) { s->err = e; };
-    CK(cudaSetDevice(s->device));
-    if (!s->inited) { st = stream_init(s, rows, cols); if (st != VSTAB_OK) return st; }
-    return stream_call(s, d_bgr, rows, cols, step, d_out_bgr, out_step, cudaMemcpyDeviceToDevice,
-                       cudaMemcpyDeviceToDevice, false);
+    return stream_entry(s, d_bgr, {false, nullptr, step}, rows, cols, d_out_bgr, {false, nullptr, out_step});
 }
 
 size_t vstab_yuv_layout_packed(int format, int rows, int cols, vstab_yuv_layout* out) {
@@ -1097,28 +1154,16 @@ size_t vstab_yuv_layout_packed(int format, int rows, int cols, vstab_yuv_layout*
     return bytes;
 }
 
-static vstab_status stream_yuv_call(vstab_t* s, const uint8_t* in, const vstab_yuv_layout* in_layout, int rows, int cols,
-                                    uint8_t* out, const vstab_yuv_layout* out_layout, bool device) {
-    if (!s) return VSTAB_ERR_INVALID_ARGUMENT;
-    vstab_status st = stream_check_args(s, in, rows, cols, (size_t)cols * 3, out, (size_t)cols * 3);
-    if (st != VSTAB_OK) return st;
-    if (!yuv_extent(in_layout, rows, cols, s->err) || !yuv_extent(out_layout, rows, cols, s->err)) return VSTAB_ERR_INVALID_ARGUMENT;
-    auto set_err = [&](const std::string& e) { s->err = e; };
-    CK(cudaSetDevice(s->device));
-    if (!s->inited) { st = stream_init(s, rows, cols); if (st != VSTAB_OK) return st; }
-    const cudaMemcpyKind in_kind = device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-    const cudaMemcpyKind out_kind = device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-    return stream_call(s, in, rows, cols, 0, out, 0, in_kind, out_kind, !device, in_layout, out_layout);
-}
-
 vstab_status vstab_stabilize_frame_yuv(vstab_t* s, const uint8_t* in, const vstab_yuv_layout* in_layout, int rows, int cols,
                                        uint8_t* out, const vstab_yuv_layout* out_layout) {
-    return stream_yuv_call(s, in, in_layout, rows, cols, out, out_layout, false);
+    if (s && (!in_layout || !out_layout)) { s->err = "null YUV layout"; return VSTAB_ERR_INVALID_ARGUMENT; }   // FrameFmt: BGR
+    return stream_entry(s, in, {true, in_layout}, rows, cols, out, {true, out_layout});
 }
 
 vstab_status vstab_stabilize_frame_yuv_device(vstab_t* s, const uint8_t* d_in, const vstab_yuv_layout* in_layout, int rows,
                                               int cols, uint8_t* d_out, const vstab_yuv_layout* out_layout) {
-    return stream_yuv_call(s, d_in, in_layout, rows, cols, d_out, out_layout, true);
+    if (s && (!in_layout || !out_layout)) { s->err = "null YUV layout"; return VSTAB_ERR_INVALID_ARGUMENT; }
+    return stream_entry(s, d_in, {false, in_layout}, rows, cols, d_out, {false, out_layout});
 }
 
 int vstab_decompose_homography(const double H[9], double cx, double cy, vstab_hparams* out) {
@@ -1231,11 +1276,10 @@ struct vstab_offline {
     DevBuf job_chunk, job_out;
     size_t job_chunk_frames = 0;
     std::vector<cudaEvent_t> host_events;         // vstab_offline_run_host: upload / render / download / conversion marks per chunk
-    // YUV frames of run_host / run (vstab_offline_set_yuv), and run_host's double-buffered staging (2 x max_batch frames each)
-    bool yuv_in = false, yuv_out = false;
-    vstab_yuv_layout yin{}, yout{};
+    // YUV layouts of the frames of run_host / run (vstab_offline_set_yuv; none: BGR), and run_host's double-buffered
+    // staging of host YUV frames (2 x max_batch frames each)
+    std::optional<vstab_yuv_layout> yin, yout;
     DevBuf ystage_in, ystage_out;
-    size_t ystage_frames = 0;
     std::string err;
     void set_err(const std::string& e) { err = e; }
 };
@@ -1573,13 +1617,11 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
     if (!o || !frames || !out || n_total < 1) return VSTAB_ERR_INVALID_ARGUMENT;
     auto set_err = [&](const std::string& e) { o->err = e; };
     Geometry& g = o->g;
-    const size_t row_bytes = (size_t)g.cols * 3;
-    const bool yin = o->yuv_in, yout = o->yuv_out;
-    if ((!yin && step < row_bytes) || (!yout && out_step < row_bytes)) { o->err = "row step smaller than 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
-    if ((yin && frame_stride < yuv_extent(&o->yin, g.rows, g.cols, o->err)) ||
-        (yout && out_frame_stride < yuv_extent(&o->yout, g.rows, g.cols, o->err))) {
-        o->err = "frame stride smaller than the extent of the YUV layout's planes"; return VSTAB_ERR_INVALID_ARGUMENT;
-    }
+    const FrameFmt in_fmt{true, o->yin ? &*o->yin : nullptr, step, frame_stride};
+    const FrameFmt out_fmt{true, o->yout ? &*o->yout : nullptr, out_step, out_frame_stride};
+    vstab_status st = in_fmt.check(g.rows, g.cols, true, o->err);
+    if (st == VSTAB_OK) st = out_fmt.check(g.rows, g.cols, true, o->err);
+    if (st != VSTAB_OK) return st;
     CK(cudaSetDevice(o->device));
     if (!o->copy_in) CK(cudaStreamCreateWithFlags(&o->copy_in, cudaStreamNonBlocking));
     if (!o->copy_out) CK(cudaStreamCreateWithFlags(&o->copy_out, cudaStreamNonBlocking));
@@ -1594,17 +1636,11 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
     uint8_t* clip = o->clip.as<uint8_t>();
     double* T = o->clipT.as<double>();
     unsigned long long* sums = o->clipSums.as<unsigned long long>();
-    // YUV frames cross the link in staging buffers of two halves of B frames: upload(k) -> convert(k) into the clip, and
-    // render(k) -> convert(k) -> download(k), the halves alternating with k
-    size_t sfb_in = 0, sfb_out = 0;
-    const vstab_yuv_layout S_in = yin ? yuv_staging_layout(o->yin.format, g.rows, g.cols, &sfb_in) : vstab_yuv_layout{};
-    const vstab_yuv_layout S_out = yout ? yuv_staging_layout(o->yout.format, g.rows, g.cols, &sfb_out) : vstab_yuv_layout{};
-    if ((yin || yout) && o->ystage_frames < (size_t)B) {
-        const size_t sb = yuv_staging_bytes(g.rows, g.cols) * 2 * (size_t)B;
-        CK(o->ystage_in.alloc(sb));
-        CK(o->ystage_out.alloc(sb));
-        o->ystage_frames = (size_t)B;
-    }
+    // host YUV frames cross the link in staging buffers of two halves of B frames: upload(k) -> convert(k) into the clip,
+    // and render(k) -> convert(k) -> download(k), the halves alternating with k
+    const size_t half_in = in_fmt.staging_bytes(g) * (size_t)B, half_out = out_fmt.staging_bytes(g) * (size_t)B;
+    if (half_in && !o->ystage_in.p) CK(o->ystage_in.alloc(2 * half_in));
+    if (half_out && !o->ystage_out.p) CK(o->ystage_out.alloc(2 * half_out));
     const long nchunks = (n_total + B - 1) / B;
     // per-chunk events live in the instance (created once, reused by every call, destroyed with it)
     std::vector<cudaEvent_t>& ev = o->host_events;
@@ -1613,14 +1649,10 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
         if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) { o->err = "cudaEventCreate failed"; return VSTAB_ERR_CUDA; }
         ev.push_back(e);
     }
-    auto cleanup = [] {};
     cudaEvent_t* ev_up = ev.data();                 // chunk k uploaded
     cudaEvent_t* ev_rd = ev.data() + nchunks;       // chunk k rendered
     cudaEvent_t* ev_dn = ev.data() + 2 * nchunks;   // chunk k downloaded
-    cudaEvent_t* ev_cv = ev.data() + 3 * nchunks;   // YUV input: chunk k converted (its staging half is free again)
-    vstab_status st = VSTAB_OK;
-    const bool in_contig = step == g.pitch && frame_stride == g.frame_bytes;
-    const bool out_contig = out_step == g.pitch && out_frame_stride == g.frame_bytes;
+    cudaEvent_t* ev_cv = ev.data() + 3 * nchunks;   // staged input: chunk k converted (its staging half is free again)
     // the accumulated-lock prefix is re-scanned after every chunk over the frames seen so far (a few
     // thousand 3x3 products): size its buffer once so no reallocation happens while kernels are in flight
     if (mode == VSTAB_ACCUMULATED_FULL_LOCK) {
@@ -1633,29 +1665,18 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
     for (long k = 0; k < nchunks && st == VSTAB_OK; ++k) {
         const long f0 = k * B, n = (n_total - f0 < B) ? n_total - f0 : B;
         const long seen = f0 + n;                                       // frames uploaded and estimated so far
-        uint8_t* stg_in = o->ystage_in.as<uint8_t>() + (size_t)(k & 1) * B * sfb_in;
-        if (yin) {
-            if (k >= 2) cudaStreamWaitEvent(o->copy_in, ev_cv[k - 2], 0);
-            if (yuv_copy(stg_in, S_in, sfb_in, frames + (size_t)f0 * frame_stride, o->yin, frame_stride, n, g.rows, g.cols,
-                         cudaMemcpyHostToDevice, o->copy_in) != cudaSuccess) { o->err = "upload failed"; st = VSTAB_ERR_CUDA; }
-        } else if (in_contig) {     // tightly packed frames: one large copy per chunk
-            if (cudaMemcpyAsync(clip + (size_t)f0 * g.frame_bytes, frames + (size_t)f0 * frame_stride, (size_t)n * g.frame_bytes,
-                                cudaMemcpyHostToDevice, o->copy_in) != cudaSuccess) { o->err = "upload failed"; st = VSTAB_ERR_CUDA; }
-        } else {
-            for (long i = 0; i < n; ++i)
-                if (cudaMemcpy2DAsync(clip + (size_t)(f0 + i) * g.frame_bytes, g.pitch, frames + (size_t)(f0 + i) * frame_stride,
-                                      step, row_bytes, g.rows, cudaMemcpyHostToDevice, o->copy_in) != cudaSuccess) {
-                    o->err = "upload failed"; st = VSTAB_ERR_CUDA; break;
-                }
+        const uint8_t* src = frames + (size_t)f0 * frame_stride;
+        uint8_t* stg_in = o->ystage_in.as<uint8_t>() + (size_t)(k & 1) * half_in;
+        if (half_in && k >= 2) cudaStreamWaitEvent(o->copy_in, ev_cv[k - 2], 0);
+        if (frames_in_transfer(g, in_fmt, src, n, clip + (size_t)f0 * g.frame_bytes, stg_in, o->copy_in) != cudaSuccess) {
+            o->err = "upload failed"; st = VSTAB_ERR_CUDA; break;
         }
-        if (st != VSTAB_OK) break;
         cudaEventRecord(ev_up[k], o->copy_in);
         cudaStreamWaitEvent(o->stream, ev_up[k], 0);
-        if (yin) {
-            launch_yuv420_to_bgr(stg_in, yuv_planes_of(S_in), sfb_in, (int)n, g.rows, g.cols, clip + (size_t)f0 * g.frame_bytes,
-                                 g.pitch, g.frame_bytes, o->stream);
-            cudaEventRecord(ev_cv[k], o->stream);
+        if (frames_in_convert(g, in_fmt, src, n, clip + (size_t)f0 * g.frame_bytes, stg_in, o->stream) != cudaSuccess) {
+            o->err = "CUDA failure in vstab_offline_run_host"; st = VSTAB_ERR_CUDA; break;
         }
+        if (half_in) cudaEventRecord(ev_cv[k], o->stream);
         st = vstab_offline_estimate(o, clip + (size_t)f0 * g.frame_bytes, g.frame_bytes, g.pitch, (int)n, f0,
                                     f0 > 0 ? clip + (size_t)(f0 - 1) * g.frame_bytes : nullptr, T + (size_t)f0 * 9,
                                     sums + (size_t)f0 * 3);
@@ -1669,41 +1690,29 @@ extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t
         st = vstab_offline_render(o, clip, g.frame_bytes, g.pitch, 0, (int)n, f0, T, seen, rmode, lock_call, sums, ob,
                                   g.frame_bytes, g.pitch);
         if (st != VSTAB_OK) break;
-        uint8_t* stg_out = o->ystage_out.as<uint8_t>() + (size_t)(k & 1) * B * sfb_out;      // free: ev_dn[k - 2] above
-        if (yout)
-            launch_bgr_to_yuv420(ob, g.pitch, g.frame_bytes, (int)n, g.rows, g.cols, stg_out, yuv_planes_of(S_out), sfb_out, o->stream);
+        uint8_t* dst = out + (size_t)f0 * out_frame_stride;
+        uint8_t* stg_out = o->ystage_out.as<uint8_t>() + (size_t)(k & 1) * half_out;      // free: ev_dn[k - 2] above
+        if (frames_out_convert(g, out_fmt, ob, n, dst, stg_out, o->stream) != cudaSuccess) {
+            o->err = "CUDA failure in vstab_offline_run_host"; st = VSTAB_ERR_CUDA; break;
+        }
         cudaEventRecord(ev_rd[k], o->stream);
         cudaStreamWaitEvent(o->copy_out, ev_rd[k], 0);
-        if (yout) {
-            if (yuv_copy(out + (size_t)f0 * out_frame_stride, o->yout, out_frame_stride, stg_out, S_out, sfb_out, n, g.rows, g.cols,
-                         cudaMemcpyDeviceToHost, o->copy_out) != cudaSuccess) { o->err = "download failed"; st = VSTAB_ERR_CUDA; }
-        } else if (out_contig) {
-            if (cudaMemcpyAsync(out + (size_t)f0 * out_frame_stride, ob, (size_t)n * g.frame_bytes, cudaMemcpyDeviceToHost,
-                                o->copy_out) != cudaSuccess) { o->err = "download failed"; st = VSTAB_ERR_CUDA; }
-        } else {
-            for (long i = 0; i < n; ++i)
-                if (cudaMemcpy2DAsync(out + (size_t)(f0 + i) * out_frame_stride, out_step, ob + (size_t)i * g.frame_bytes, g.pitch,
-                                      row_bytes, g.rows, cudaMemcpyDeviceToHost, o->copy_out) != cudaSuccess) {
-                    o->err = "download failed"; st = VSTAB_ERR_CUDA; break;
-                }
-        }
+        if (frames_out_transfer(g, out_fmt, ob, n, dst, stg_out, o->copy_out) != cudaSuccess) { o->err = "download failed"; st = VSTAB_ERR_CUDA; }
         cudaEventRecord(ev_dn[k], o->copy_out);
     }
     cudaStreamSynchronize(o->copy_in);
     cudaStreamSynchronize(o->stream);
     cudaStreamSynchronize(o->copy_out);
-    cleanup();
     if (st == VSTAB_OK && cudaGetLastError() != cudaSuccess) { o->err = "CUDA failure in vstab_offline_run_host"; st = VSTAB_ERR_CUDA; }
     return st;
 }
 
 extern "C" vstab_status vstab_offline_set_yuv(vstab_offline_t* o, const vstab_yuv_layout* in, const vstab_yuv_layout* out) {
     if (!o) return VSTAB_ERR_INVALID_ARGUMENT;
-    if ((in && !yuv_extent(in, o->g.rows, o->g.cols, o->err)) || (out && !yuv_extent(out, o->g.rows, o->g.cols, o->err)))
-        return VSTAB_ERR_INVALID_ARGUMENT;
-    o->yuv_in = in != nullptr; o->yuv_out = out != nullptr;
-    o->yin = in ? *in : vstab_yuv_layout{};
-    o->yout = out ? *out : vstab_yuv_layout{};
+    for (const vstab_yuv_layout* L : {in, out})
+        if (L && FrameFmt{true, L}.check(o->g.rows, o->g.cols, false, o->err) != VSTAB_OK) return VSTAB_ERR_INVALID_ARGUMENT;
+    o->yin = in ? std::make_optional(*in) : std::nullopt;
+    o->yout = out ? std::make_optional(*out) : std::nullopt;
     return VSTAB_OK;
 }
 
@@ -1909,20 +1918,22 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     const long N = cfg->n_total;
     const int mode = cfg->mode;
     const bool sim = cfg->source == VSTAB_SRC_SIMULATOR;
-    const bool dev_src = cfg->source == VSTAB_SRC_DEVICE;
-    const bool yin = o->yuv_in && !sim, yout = o->yuv_out;
-    // a YUV device shard is staged through the chunk ring like a host one (converted instead of copied)
-    const bool resident = dev_src && !yin;
+    // caller frames (the simulator's frames are the library's own) and the sink of the outputs, if any
+    const FrameFmt in{cfg->source != VSTAB_SRC_DEVICE, o->yin && !sim ? &*o->yin : nullptr, cfg->step, cfg->frame_stride};
+    const FrameFmt out{cfg->host_out != nullptr, o->yout ? &*o->yout : nullptr, cfg->out_step, cfg->out_frame_stride};
+    uint8_t* const sink = cfg->d_out ? cfg->d_out : cfg->host_out;
+    // a device BGR shard is read where it is; a YUV device shard is staged through the chunk ring like a host one
+    // (converted instead of copied)
+    const bool resident = in.direct();
+    const bool direct = sink && out.direct();                      // the warp writes the caller's BGR buffer itself
     const bool feature_lock = mode == VSTAB_ORB_FULL_LOCK || mode == VSTAB_SIFT_FULL_LOCK;
     if (mode < 0 || mode > 5) { o->err = "Stabilizer: Invalid stabilization mode"; return VSTAB_ERR_INVALID_ARGUMENT; }
     if (sim && (!cfg->d_texture || !cfg->poses || cfg->tex_rows < 1 || cfg->tex_cols < 1)) { o->err = "simulator source needs d_texture and poses"; return VSTAB_ERR_INVALID_ARGUMENT; }
-    const size_t row_bytes = (size_t)g.cols * 3;
-    if (!sim && (!cfg->host_frames || (!yin && cfg->step < row_bytes))) { o->err = "host / device source needs frames with step >= 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
-    if ((cfg->host_out || cfg->d_out) && !yout && cfg->out_step < row_bytes) { o->err = "out_step smaller than 3*cols"; return VSTAB_ERR_INVALID_ARGUMENT; }
-    if ((yin && cfg->frame_stride < yuv_extent(&o->yin, g.rows, g.cols, o->err)) ||
-        (yout && (cfg->host_out || cfg->d_out) && cfg->out_frame_stride < yuv_extent(&o->yout, g.rows, g.cols, o->err))) {
-        o->err = "frame stride smaller than the extent of the YUV layout's planes"; return VSTAB_ERR_INVALID_ARGUMENT;
-    }
+    const char* src_err = "host / device source needs frames with step >= 3*cols";
+    if (!sim && !cfg->host_frames) { o->err = src_err; return VSTAB_ERR_INVALID_ARGUMENT; }
+    vstab_status st = sim ? VSTAB_OK : in.check(g.rows, g.cols, true, o->err, src_err);
+    if (st == VSTAB_OK && sink) st = out.check(g.rows, g.cols, true, o->err, "out_step smaller than 3*cols");
+    if (st != VSTAB_OK) return st;
     if (cfg->host_out && cfg->d_out) { o->err = "give host_out or d_out, not both"; return VSTAB_ERR_INVALID_ARGUMENT; }
     if ((mode == VSTAB_ACCUMULATED_FULL_LOCK || feature_lock) && cfg->lock_call < (long)o->F) {
         o->err = "lock modes must be set at a call index >= future (SURVEY B.6)"; return VSTAB_ERR_STATE;
@@ -1951,7 +1962,7 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     const long ring_chunks = fused ? fp.ring_chunks : 1;
     const long ring_frames = ring_chunks * B;                       // + one slot for the halo frame of the first chunk
     DevBuf& chunk = o->job_chunk; DevBuf& outc = o->job_out;
-    if (!(resident && cfg->d_out && !yout) && o->job_chunk_frames < (size_t)ring_frames + 1) {
+    if (!(resident && direct) && o->job_chunk_frames < (size_t)ring_frames + 1) {
         CK(chunk.alloc(g.frame_bytes * ((size_t)ring_frames + 1) + 64));
         CK(outc.alloc(g.frame_bytes * (size_t)B + 64));
         o->job_chunk_frames = (size_t)ring_frames + 1;
@@ -1966,14 +1977,11 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     CK(cudaMemsetAsync(checks.p, 0, sizeof(unsigned long long) * (size_t)(n_calls > 0 ? n_calls : 1), q));
     uint8_t* cb = chunk.as<uint8_t>();
     const size_t fb = g.frame_bytes;
-    // YUV: host frames are uploaded into a staging buffer of the stream that fetches them (q, and qs in the fused pass) and
-    // converted into the chunk slots; YUV outputs are converted from the BGR output chunk, into d_out or a download staging
-    size_t sfb_in = 0, sfb_out = 0;
-    const vstab_yuv_layout S_in = yin ? yuv_staging_layout(o->yin.format, g.rows, g.cols, &sfb_in) : vstab_yuv_layout{};
-    const vstab_yuv_layout S_out = yout ? yuv_staging_layout(o->yout.format, g.rows, g.cols, &sfb_out) : vstab_yuv_layout{};
+    // staging of host YUV frames: one upload staging per stream that fetches frames (q, and qs in the fused pass), one
+    // download staging
     DevBuf ystage_q, ystage_qs, ystage_o;
-    if (yin && !dev_src) { CK(ystage_q.alloc(sfb_in * (size_t)B)); CK(ystage_qs.alloc(sfb_in * (size_t)B)); }
-    if (yout && cfg->host_out) CK(ystage_o.alloc(sfb_out * (size_t)B));
+    if (in.staging_bytes(g)) { CK(ystage_q.alloc(in.staging_bytes(g) * (size_t)B)); CK(ystage_qs.alloc(in.staging_bytes(g) * (size_t)B)); }
+    if (out.staging_bytes(g)) CK(ystage_o.alloc(out.staging_bytes(g) * (size_t)B));
     // resident shard: frame f of the clip lives at dframe(f); no staging
     auto dframe = [&](long f) -> const uint8_t* { return f == pl.first - 1 ? cfg->host_halo : cfg->host_frames + (size_t)(f - pl.first) * cfg->frame_stride; };
     const size_t src_fs = resident ? cfg->frame_stride : fb, src_step = resident ? cfg->step : g.pitch;
@@ -1997,29 +2005,16 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
         if (sim) {
             launch_render(cfg->d_texture, cfg->tex_rows, cfg->tex_cols, poses_d.as<RenderPose>() + f0, (int)n, g.cols, g.rows, cfg->focal,
                           cb + (size_t)slot * fb, g.pitch, fb, q, rays_d.as<double>(), tex4_d.as<unsigned>());
-        } else if (yin) {
+        } else {
             if (f0 < pl.first - 1 || f0 + n > pl.last) { o->err = "internal: frame outside the rank's shard"; return VSTAB_ERR_STATE; }
+            uint8_t* stg = (q == o->stream ? ystage_q : ystage_qs).as<uint8_t>();
             for (long i = 0; i < n;) {
                 const long f = f0 + i;
                 const bool halo = f == pl.first - 1;
                 const long m = halo ? 1 : n - i;                    // the halo frame alone, then one contiguous run
                 const uint8_t* src = halo ? cfg->host_halo : cfg->host_frames + (size_t)(f - pl.first) * cfg->frame_stride;
-                uint8_t* dst = cb + (size_t)(slot + i) * fb;
-                if (dev_src) {
-                    launch_yuv420_to_bgr(src, yuv_planes_of(o->yin), cfg->frame_stride, (int)m, g.rows, g.cols, dst, g.pitch, fb, q);
-                } else {
-                    uint8_t* stg = (q == o->stream ? ystage_q : ystage_qs).as<uint8_t>();
-                    CK(yuv_copy(stg, S_in, sfb_in, src, o->yin, cfg->frame_stride, m, g.rows, g.cols, cudaMemcpyHostToDevice, q));
-                    launch_yuv420_to_bgr(stg, yuv_planes_of(S_in), sfb_in, (int)m, g.rows, g.cols, dst, g.pitch, fb, q);
-                }
+                CK(frames_in(g, in, src, m, cb + (size_t)(slot + i) * fb, stg, q));
                 i += m;
-            }
-        } else {
-            for (long i = 0; i < n; ++i) {
-                const long f = f0 + i;
-                if (f < pl.first - 1 || f >= pl.last) { o->err = "internal: frame outside the rank's shard"; return VSTAB_ERR_STATE; }
-                const uint8_t* src = f == pl.first - 1 ? cfg->host_halo : cfg->host_frames + (size_t)(f - pl.first) * cfg->frame_stride;
-                CK(cudaMemcpy2DAsync(cb + (size_t)(slot + i) * fb, g.pitch, src, cfg->step, row_bytes, g.rows, cudaMemcpyHostToDevice, q));
             }
         }
         clock.end(q);
@@ -2028,7 +2023,6 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     };
     cudaEvent_t ev_t0 = clock.get(), ev_t1 = clock.get();
     CK(cudaEventRecord(ev_t0, q));
-    vstab_status st = VSTAB_OK;
 
     // ---- ORB / SIFT lock: reference set from the anchor frame, broadcast from its owner --------------------------
     if (feature_lock) {
@@ -2066,7 +2060,6 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
             vstab_status s2;
             if (ring == 0 && (s2 = fetch(p_lo, p_hi - p_lo + 1, 0, qw)) != VSTAB_OK) return s2;
             clock.begin(PH_RENDER, qw);
-            const bool direct = cfg->d_out && !yout;                // warp straight into the caller's BGR buffer
             uint8_t* dst = direct ? cfg->d_out + (size_t)(c - pl.call_first) * cfg->out_frame_stride : outc.as<uint8_t>();
             const long base = ring > 0 ? pl.first : p_lo;          // frame held by slot 0 (ring: modulo `ring`)
             s2 = offline_render_impl(o, resident ? dframe(p_lo) : cb, src_fs, src_step, base, (int)n, c, T_all.as<double>(), N, mode,
@@ -2075,24 +2068,9 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
                                      cfg->checksums ? checks.as<unsigned long long>() + (c - pl.call_first) : nullptr, ring, qw);
             clock.end(qw);
             if (s2 != VSTAB_OK) return s2;
-            uint8_t* yuv_dst = cfg->d_out ? cfg->d_out : cfg->host_out;
-            if (yout && yuv_dst) {
-                uint8_t* d = yuv_dst + (size_t)(c - pl.call_first) * cfg->out_frame_stride;
-                if (cfg->d_out) {
-                    launch_bgr_to_yuv420(outc.as<uint8_t>(), g.pitch, fb, (int)n, g.rows, g.cols, d, yuv_planes_of(o->yout),
-                                         cfg->out_frame_stride, qw);
-                } else {
-                    launch_bgr_to_yuv420(outc.as<uint8_t>(), g.pitch, fb, (int)n, g.rows, g.cols, ystage_o.as<uint8_t>(),
-                                         yuv_planes_of(S_out), sfb_out, qw);
-                    CK(yuv_copy(d, o->yout, cfg->out_frame_stride, ystage_o.as<uint8_t>(), S_out, sfb_out, n, g.rows, g.cols,
-                                cudaMemcpyDeviceToHost, qw));
-                }
-                CK(cudaGetLastError());
-            } else if (cfg->host_out) {
-                for (long i = 0; i < n; ++i)
-                    CK(cudaMemcpy2DAsync(cfg->host_out + (size_t)(c - pl.call_first + i) * cfg->out_frame_stride, cfg->out_step,
-                                         outc.as<uint8_t>() + (size_t)i * fb, g.pitch, row_bytes, g.rows, cudaMemcpyDeviceToHost, qw));
-            }
+            if (sink && !direct)
+                CK(frames_out(g, out, outc.as<uint8_t>(), n, sink + (size_t)(c - pl.call_first) * cfg->out_frame_stride,
+                              ystage_o.as<uint8_t>(), qw));
         }
         return VSTAB_OK;
     };

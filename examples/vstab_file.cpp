@@ -19,6 +19,7 @@
 // "-" means stdin / stdout.  Exit status: 0 ok, 1 bad usage, 2 I/O, 3 stabilizer error.
 #include <chrono>
 #include <cstdio>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <deque>
@@ -38,6 +39,7 @@ struct Options {
     bool side_by_side = false, have_mode = false;
     StabilizationMode mode = StabilizationMode::GLOBAL_SMOOTHING;
     int pix_fmt = 0, out_pix_fmt = -1;   // 0 = bgr24, else vstab_pixel_format; -1: as the input
+    double crop = 1.0, crop_release = 0.002;   // auto-crop (1: off)
 };
 
 // ffmpeg's pixel format names
@@ -60,11 +62,26 @@ bool parse_mode(const std::string& s, StabilizationMode& m) {
     return true;
 }
 
+// --crop MAX_ZOOM[,RELEASE]: 1 < MAX_ZOOM <= 4, RELEASE > 0 (default 0.002 per call), ceil((MAX_ZOOM - 1) / RELEASE) <= 4096
+bool parse_crop(const std::string& s, double& max_zoom, double& release) {
+    const size_t comma = s.find(',');
+    const std::string a = s.substr(0, comma), b = comma == std::string::npos ? "" : s.substr(comma + 1);
+    if (a.empty() || (comma != std::string::npos && b.empty())) return false;
+    char* end = nullptr;
+    max_zoom = std::strtod(a.c_str(), &end);
+    if (*end) return false;
+    release = 0.002;
+    if (!b.empty()) { release = std::strtod(b.c_str(), &end); if (*end) return false; }
+    return max_zoom > 1.0 && max_zoom <= 4.0 && release > 0.0 && std::isfinite(release) &&
+           std::ceil((max_zoom - 1.0) / release) <= 4096.0;
+}
+
 int usage(const char* argv0) {
     std::fprintf(stderr,
                  "usage: %s --file <in.bgr|-> --width W --height H [--out <out.bgr|->] [--past-window N] [--future-window N]\n"
                  "          [--working-height N] [--mode global|lock|orb|sift|translation|rotation] [--mode-at CALL]\n"
-                 "          [--side-by-side] [--frames N] [--pix-fmt bgr24|nv12|yuv420p] [--out-pix-fmt bgr24|nv12|yuv420p]\n", argv0);
+                 "          [--side-by-side] [--frames N] [--pix-fmt bgr24|nv12|yuv420p] [--out-pix-fmt bgr24|nv12|yuv420p]\n"
+                 "          [--crop MAX_ZOOM[,RELEASE]]\n", argv0);
     return 1;
 }
 
@@ -99,6 +116,7 @@ int main(int argc, char** argv) {
         else if (a == "--mode") { if (!parse_mode(next("--mode"), o.mode)) return usage(argv[0]); o.have_mode = true; }
         else if (a == "--mode-at") o.mode_at = std::atol(next("--mode-at"));
         else if (a == "--side-by-side") o.side_by_side = true;
+        else if (a == "--crop") { if (!parse_crop(next("--crop"), o.crop, o.crop_release)) return usage(argv[0]); }
         else if (a == "--pix-fmt") { if (!parse_pix_fmt(next("--pix-fmt"), o.pix_fmt)) return usage(argv[0]); }
         else if (a == "--out-pix-fmt") { if (!parse_pix_fmt(next("--out-pix-fmt"), o.out_pix_fmt)) return usage(argv[0]); }
         else { std::fprintf(stderr, "Error: unknown argument %s\n", a.c_str()); return usage(argv[0]); }
@@ -134,6 +152,7 @@ int main(int argc, char** argv) {
     int rc = 0;
     try {
         Stabilizer stabilizer((size_t)o.past, (size_t)o.future, o.working_height);   // argument errors throw before any device work
+        if (o.crop > 1.0) stabilizer.setAutoCrop(o.crop, o.crop_release);
         // pinned staging buffers: the per-frame call copies straight from / into them
         hin = static_cast<uint8_t*>(vstab_host_alloc(in_bytes));
         hout = static_cast<uint8_t*>(vstab_host_alloc(out_bytes));

@@ -17,6 +17,7 @@
 // Exit status: 0 ok, 1 bad usage, 2 I/O, 3 stabilizer error.
 #include <chrono>
 #include <cstdio>
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <string>
@@ -36,6 +37,7 @@ struct Options {
     int width = 0, height = 0, working_height = 360, batch = 128, rank = 0, world = 1, device = -1;
     long frames = -1, mode_at = 0, past = 60, future = 45;        // 2.0 s / 1.5 s at 30 fps (src/main.cpp:205-206)
     int mode = VSTAB_GLOBAL_SMOOTHING;
+    double crop = 1.0, crop_release = 0.002;                      // auto-crop (1: off)
 };
 
 bool parse_mode(const std::string& s, int& m) {
@@ -47,11 +49,25 @@ bool parse_mode(const std::string& s, int& m) {
     return true;
 }
 
+// --crop MAX_ZOOM[,RELEASE]: 1 < MAX_ZOOM <= 4, RELEASE > 0 (default 0.002 per call), ceil((MAX_ZOOM - 1) / RELEASE) <= 4096
+bool parse_crop(const std::string& s, double& max_zoom, double& release) {
+    const size_t comma = s.find(',');
+    const std::string a = s.substr(0, comma), b = comma == std::string::npos ? "" : s.substr(comma + 1);
+    if (a.empty() || (comma != std::string::npos && b.empty())) return false;
+    char* end = nullptr;
+    max_zoom = std::strtod(a.c_str(), &end);
+    if (*end) return false;
+    release = 0.002;
+    if (!b.empty()) { release = std::strtod(b.c_str(), &end); if (*end) return false; }
+    return max_zoom > 1.0 && max_zoom <= 4.0 && release > 0.0 && std::isfinite(release) &&
+           std::ceil((max_zoom - 1.0) / release) <= 4096.0;
+}
+
 int usage(const char* argv0) {
     std::fprintf(stderr,
                  "usage: %s --file <in.bgr> --width W --height H --out <out.bgr> [--past-window N] [--future-window N]\n"
                  "          [--working-height N] [--batch N] [--mode global|lock|orb|sift] [--mode-at CALL] [--frames N]\n"
-                 "          [--rank R --world S --id-file PATH] [--device D] [--checksums FILE]\n", argv0);
+                 "          [--rank R --world S --id-file PATH] [--device D] [--checksums FILE] [--crop MAX_ZOOM[,RELEASE]]\n", argv0);
     return 1;
 }
 
@@ -122,6 +138,7 @@ int main(int argc, char** argv) {
         else if (a == "--id-file") o.id_file = next("--id-file");
         else if (a == "--device") o.device = std::atoi(next("--device"));
         else if (a == "--checksums") o.checksums = next("--checksums");
+        else if (a == "--crop") { if (!parse_crop(next("--crop"), o.crop, o.crop_release)) return usage(argv[0]); }
         else return usage(argv[0]);
     }
     if (o.in.empty() || o.out.empty() || o.width <= 0 || o.height <= 0 || o.batch < 1 || o.past < 0 || o.future < 0 ||
@@ -150,6 +167,7 @@ int main(int argc, char** argv) {
         vstab_offline_destroy(job);
         return code;
     };
+    if (o.crop > 1.0 && vstab_offline_set_crop(job, o.crop, o.crop_release) != VSTAB_OK) return fail(1, "vstab_offline_set_crop");
     if (o.world > 1) {
         vstab_nccl_id id;
         if (!exchange_id(o, &id)) return fail(2, "NCCL id exchange through --id-file failed");

@@ -116,6 +116,9 @@ public:
     // The reference selects its feathered-trail output (copyFeathered, src/stabilizer.cpp:1303-1307) at compile time with
     // `#if 0`; here it is a run-time switch, off by default.
     void setTrailCompositing(bool enable) { check(vstab_set_trail(h_, enable ? 1 : 0)); }
+    // Auto-crop (vstab_set_crop, include/vstab.h): zoom each output just enough to hide its border, up to maxZoom
+    // (1 < maxZoom <= 4; 1 turns it off), the zoom falling back by at most `release` per call.  Beyond the reference.
+    void setAutoCrop(double maxZoom, double release = 0.002) { check(vstab_set_crop(h_, maxZoom, release)); }
 
     // TRANSLATION_LOCK / ROTATION_LOCK evaluate to the identity in the reference (include/stabilizer.hpp:23 "@todo fix
     // partial locking modes"); with this switch its formulas (src/stabilizer.cpp:1246-1260) are fed with the accumulated

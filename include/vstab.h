@@ -140,6 +140,31 @@ vstab_status vstab_set_trail(vstab_t* s, int enable);
  * setStabilizationMode): translation lock keeps the accumulated rotation and cancels the drift of the image centre,
  * rotation lock cancels only the accumulated rotation about the image centre.  Per-frame API only. */
 vstab_status vstab_set_partial_lock_fix(vstab_t* s, int enable);
+
+/* ---- auto-crop: zoom each output just enough to hide the border of its warp ---------------------------------------------
+ * Beyond the reference (like vstab_set_trail): without it, wherever the warp reads outside the presentation frame the output
+ * shows the border colour (half the frame's mean, src/stabilizer.cpp:1309).  Off by default (max_zoom == 1).
+ * Notation: rows x cols the frame, c0 = ((cols-1)/2, (rows-1)/2), S = [0, cols-1] x [0, rows-1] the pixel centres, H_c the
+ * H_stabilize_scaled of call c, Z(z) = [[z, 0, (1-z) c0x], [0, z, (1-z) c0y], [0, 0, 1]] the zoom by z about c0.
+ *  1. need(H) (vstab_crop_zoom, f64, closed form): max_zoom if H is not finite or w = h20 x + h21 y + h22 <= 0 at a corner
+ *     of S.  Else Q = H(S) is a convex quadrilateral; edge k runs Q[k] -> Q[k+1] (corners of S in the order (0,0),
+ *     (cols-1,0), (cols-1,rows-1), (0,rows-1)), g = sign of Q's signed area (+1 when > 0, else -1).  Per edge (a, b):
+ *     s0 = g cross(b-a, c0-a); s0 <= 0 (centre outside Q) -> max_zoom; per corner q of S, s1 = g cross(b-a, q-c0), and
+ *     s1 < 0 bounds t <= s0 / -s1.  t* = min(1, every bound); need = clamp(1 / t*, 1, max_zoom).  need(I) == 1 exactly;
+ *     a shift by dx needs ((cols-1)/2) / ((cols-1)/2 - |dx|).  No margin: the warp's 1/32-px source coordinates put a
+ *     point within 1/64 px outside S on S, with zero weight on the taps outside it.
+ *  2. zoom of call c (causal, so streaming and every offline split agree bit for bit):
+ *     z_c = clamp(max over j in [max(0, c-R), c] of (n_j - (double)(c-j) * release), 1, max_zoom), n_j = need(H_j),
+ *     R = ceil((max_zoom - 1) / release).  The zoom rises at once to what the current call needs and falls by at most
+ *     `release` per call.  Streaming: calls before the call that enabled the crop count as n_j = 1.
+ *  3. call c warps (or trails) with Hc = Z(z_c) * H_c, its inverse computed like H_c's.  Call 0 (H = I) stays the copy of
+ *     its input.  Where z_c is capped at max_zoom a border can still show, in the usual colour.
+ *  4. VSTAB_TAP_H_SCALED and vstab_offline_read_h report Hc; VSTAB_TAP_H_STABILIZE stays the working-resolution H.
+ * Crop on: 1 < max_zoom <= 4, 0 < release (finite), R <= 4096; anything else (NaN included) is VSTAB_ERR_INVALID_ARGUMENT.
+ * A switch drops an output prepared ahead, like vstab_set_trail; mode switches keep the history. */
+vstab_status vstab_set_crop(vstab_t* s, double max_zoom, double release);
+/* need(H) of rule 1 on the host: -1 for a NULL H, rows or cols < 2, or max_zoom outside [1, 4]. */
+double vstab_crop_zoom(const double H[9], int rows, int cols, double max_zoom);
 const char* vstab_last_error(const vstab_t* s);      /* message of the last non-OK status */
 const char* vstab_status_string(vstab_status st);
 int vstab_abi_version(void);
@@ -328,6 +353,12 @@ vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offline_cfg* cfg,
  * building blocks (estimate, render, register, reference_capture) take BGR only.  VSTAB_ERR_INVALID_ARGUMENT for a
  * layout that does not fit the instance's frame size. */
 vstab_status vstab_offline_set_yuv(vstab_offline_t* o, const vstab_yuv_layout* in, const vstab_yuv_layout* out);
+/* Auto-crop (vstab_set_crop above, same parameters and semantics) for vstab_offline_render, _run_host and _run.  Every
+ * render recomputes the matrices of the R calls before its first one, so the outputs equal the streaming calls' whatever
+ * the batches or shards.  So with the crop on, the d_T_all of vstab_offline_render must hold T[max(1, call_first-R-P-F+1) ..],
+ * and in vstab_offline_run's fused GLOBAL_SMOOTHING pass a call's matrices read like a window of past P + R (the fused plan
+ * of past_frames + R: on ranks > 0 the first P + R - 1 calls wait for the exchange). */
+vstab_status vstab_offline_set_crop(vstab_offline_t* o, double max_zoom, double release);
 /* the checksum the warp kernel accumulates, of a host frame (tests) */
 uint64_t vstab_frame_checksum(const uint8_t* bgr, int rows, int cols, size_t step);
 

@@ -2,10 +2,11 @@
 library) produces, call by call, the same output checksums and the same transforms as a world of one.
 
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port 29511 \
-      tools/verify_sharded.py [--frames 384] [--modes smooth,lock,orb,sift]
+      tools/verify_sharded.py [--frames 384] [--modes smooth,lock,orb,sift] [--crop MAX_ZOOM[,RELEASE]]
 
 Every rank runs its shard of the clip (device simulator source); rank 0 additionally runs the whole clip alone on its
-GPU and compares.  Prints one JSON line per mode on rank 0; exit code 1 on any mismatch."""
+GPU and compares.  --crop runs both with auto-crop (vstab_offline_set_crop).  Prints one JSON line per mode on rank 0;
+exit code 1 on any mismatch."""
 import argparse
 import json
 import os
@@ -29,7 +30,9 @@ def main():
     ap.add_argument("--frames", type=int, default=384)
     ap.add_argument("--modes", default="smooth,lock,orb")
     ap.add_argument("--batch", type=int, default=32)
+    ap.add_argument("--crop", help="MAX_ZOOM[,RELEASE]: auto-crop on every instance (release default: vs.CROP_RELEASE)")
     a = ap.parse_args()
+    crop = [float(x) for x in a.crop.split(",")] if a.crop else None
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
     torch.cuda.set_device(local)
@@ -43,6 +46,8 @@ def main():
         mode = getattr(vs, mname)
         poses = synth.camera_path(n, drift=0.0 if lock_at else 0.0015)
         off = offline.OfflineStabilizer(60, 45, wh, H, W, a.batch, device=local)
+        if crop:
+            off.set_crop(*crop)
         off.comm_init(rank, world)
         r = off.run(n, mode, lock_at or 0, texture=tex, poses=poses, focal=synth.focal_for_width(W), want_T=True)
         off.close()
@@ -54,6 +59,8 @@ def main():
             parts = [mine]
         if rank == 0:
             solo = offline.OfflineStabilizer(60, 45, wh, H, W, a.batch, device=local)
+            if crop:
+                solo.set_crop(*crop)
             solo.comm_init(0, 1)
             s = solo.run(n, mode, lock_at or 0, texture=tex, poses=poses, focal=synth.focal_for_width(W), want_T=True)
             solo.close()
@@ -65,7 +72,7 @@ def main():
             ok_cs = bool(seen.all() and np.array_equal(got, s["checksums"]))
             ok_T = bool(np.array_equal(r["T"], s["T"]))
             bad += int(not (ok_cs and ok_T))
-            print(json.dumps({"mode": mname, "world": world, "frames": n, "size": [W, H], "working_height": wh,
+            print(json.dumps({"mode": mname, "world": world, "frames": n, "size": [W, H], "working_height": wh, "crop": crop,
                               "checksums_equal_world1": ok_cs, "transforms_bit_equal_world1": ok_T,
                               "calls_mismatching": int((got != s["checksums"]).sum()),
                               "ms_max_over_ranks": max(p[3] for p in parts), "ms_world1": s["total_ms"]}), flush=True)

@@ -15,6 +15,7 @@
 #include <mutex>
 #include <utility>
 #include <chrono>
+#include <cmath>
 #include <cstdlib>
 #include <cstdio>
 #include <cstring>
@@ -100,6 +101,23 @@ thread_local std::string g_err;   // for entry points without an instance
 // a SIFT matcher launch (launch_l2_match / launch_l2_nn_batch) returned false
 constexpr const char* kL2MapErr = "SIFT matcher: cuTensorMapEncodeTiled (the driver's tensor-map encoder) is missing or rejected the descriptor arrays";
 void nccl_comm_destroy(void* comm);
+
+// auto-crop parameters (vstab_set_crop / vstab_offline_set_crop); max_zoom == 1 turns the crop off
+constexpr int kCropMaxR = 4096;
+bool crop_params(double max_zoom, double release, CropArgs* out, std::string& err) {
+    CropArgs c{1.0, 0.0, 0};
+    if (max_zoom != 1.0) {
+        if (!(max_zoom > 1.0 && max_zoom <= 4.0) || !(release > 0.0) || !std::isfinite(release)) {
+            err = "auto-crop: max_zoom must be 1 (off) or in (1, 4], and release a finite value > 0";
+            return false;
+        }
+        const double R = std::ceil((max_zoom - 1.0) / release);
+        if (!(R <= kCropMaxR)) { err = "auto-crop: (max_zoom - 1) / release exceeds 4096 calls"; return false; }
+        c.max_zoom = max_zoom; c.release = release; c.R = (int)R;
+    }
+    *out = c;
+    return true;
+}
 
 // VSTAB_GUARD=1 (tests): every device buffer of the library is allocated between two 4 KB guard bands filled with a pattern;
 // when the buffer is released the bands are read back and every byte that changed counts as an out-of-bounds WRITE
@@ -592,6 +610,11 @@ struct vstab {
     bool trail = false;                     // copyFeathered branch of stabilizeFrame (:1303-1307)
     bool partial_fix = false;               // TRANSLATION_/ROTATION_LOCK fed with the accumulated lock (hpp:23 @todo)
     DevBuf trail_bg, trail_ws;              // trail_background_ (:129) and K14 scratch
+    // auto-crop (vstab_set_crop): on when crop.max_zoom > 1.  crop_need holds n_j of call j in slot j % (R + 1); crop_reset:
+    // the next output chain first sets the whole history to 1 (calls before the enabling call need no zoom)
+    CropArgs crop{1.0, 0.0, 0};
+    bool crop_reset = false;
+    DevBuf crop_need;
     // staging of host YUV frames (FrameFmt): the input frame is uploaded here (copy_stream) and converted into the ring, the
     // presented BGR frame is converted here (out_stream) and downloaded.  One frame each: every use is ordered by its stream.
     DevBuf yuv_in, yuv_out;
@@ -794,6 +817,17 @@ static vstab_status stream_output(vstab* s, long n, uint8_t* d_out, size_t out_p
     a.partial_fix = s->partial_fix ? 1 : 0;
     a.cx = (double)(float)(g.ww / 2.0); a.cy = (double)(float)(g.wh / 2.0);                            // Point2f centre
     launch_smooth(a, n, 1, wp, q);                                                                     // :1234-1296
+    if (s->crop.max_zoom > 1.0) {
+        // one history slot per call, written by the chain that builds the call: a prepared output that is dropped and
+        // rebuilt writes the same slot again, and successive chains are ordered by ev_pre / ev_chain
+        if (!s->crop_need.p) CK(s->crop_need.alloc(sizeof(double) * (kCropMaxR + 1)));
+        CropArgs ca = s->crop;
+        ca.rows = g.rows; ca.cols = g.cols;
+        ca.need = s->crop_need.as<double>(); ca.need_base = 0; ca.need_mod = ca.R + 1;
+        ca.reset = s->crop_reset ? 1 : 0;
+        s->crop_reset = false;
+        launch_crop(ca, nullptr, 0, wp, n, 1, q);
+    }
     if (!prepared_ahead) s->mark(8, q);
     if (feature_lock && s->F >= 2 && s->has_reference) {
         // registration of the next call's presentation frame, beside this call's warp and download.  Only with
@@ -1280,6 +1314,10 @@ struct vstab_offline {
     // staging of host YUV frames (2 x max_batch frames each)
     std::optional<vstab_yuv_layout> yin, yout;
     DevBuf ystage_in, ystage_out;
+    // auto-crop (vstab_offline_set_crop): every render recomputes the warp parameters of the R calls before its first one
+    // (crop_halo) and their needs (crop_need, halo + batch), so no state is carried from one render to the next
+    CropArgs crop{1.0, 0.0, 0};
+    DevBuf crop_halo, crop_need;
     std::string err;
     void set_err(const std::string& e) { err = e; }
 };
@@ -1562,6 +1600,19 @@ static vstab_status offline_render_impl(vstab_offline_t* o, const uint8_t* d_fra
     a.npix = (double)g.rows * (double)g.cols;
     o->timer.begin(ST_SMOOTH, q);
     launch_smooth(a, call_first, n, o->wp.as<WarpParams>(), q);
+    if (o->crop.max_zoom > 1.0) {
+        // the zoom of call c reads the needs of calls [c - R, c]: recompute the matrices of the calls before call_first here
+        // (their presentation frames and channel sums belong to other chunks: no sums, matrices only)
+        const int nhalo = (int)(call_first < o->crop.R ? call_first : o->crop.R);
+        SmoothArgs ah = a;
+        ah.sums = nullptr;
+        launch_smooth(ah, call_first - nhalo, nhalo, o->crop_halo.as<WarpParams>(), q);
+        CropArgs ca = o->crop;
+        ca.rows = g.rows; ca.cols = g.cols;
+        ca.need = o->crop_need.as<double>(); ca.need_base = call_first - nhalo; ca.need_mod = (long)nhalo + n;
+        ca.reset = 0;
+        launch_crop(ca, o->crop_halo.as<WarpParams>(), nhalo, o->wp.as<WarpParams>(), call_first, n, q);
+    }
     o->timer.end(ST_SMOOTH, q);
     o->timer.begin(ST_WARP, q);
     launch_warp(d_frames, step, frame_stride, slot_mod, o->wp.as<WarpParams>(), n, g.cols, g.rows, d_out, out_step,
@@ -1713,6 +1764,21 @@ extern "C" vstab_status vstab_offline_set_yuv(vstab_offline_t* o, const vstab_yu
         if (L && FrameFmt{true, L}.check(o->g.rows, o->g.cols, false, o->err) != VSTAB_OK) return VSTAB_ERR_INVALID_ARGUMENT;
     o->yin = in ? std::make_optional(*in) : std::nullopt;
     o->yout = out ? std::make_optional(*out) : std::nullopt;
+    return VSTAB_OK;
+}
+
+extern "C" vstab_status vstab_offline_set_crop(vstab_offline_t* o, double max_zoom, double release) {
+    if (!o) return VSTAB_ERR_INVALID_ARGUMENT;
+    auto set_err = [&](const std::string& e) { o->err = e; };
+    CropArgs c;
+    if (!crop_params(max_zoom, release, &c, o->err)) return VSTAB_ERR_INVALID_ARGUMENT;
+    if (c.max_zoom > 1.0) {
+        CK(cudaSetDevice(o->device));
+        CK(cudaStreamSynchronize(o->stream));                      // a render in flight may still read the old buffers
+        CK(o->crop_halo.alloc(sizeof(WarpParams) * (size_t)c.R));
+        CK(o->crop_need.alloc(sizeof(double) * ((size_t)c.R + (size_t)o->max_batch + 1)));
+    }
+    o->crop = c;
     return VSTAB_OK;
 }
 
@@ -1958,7 +2024,8 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     // into a neighbour's shard (the first P-1 and the last F-1 of a rank in a world > 1) wait for the all-gather as before.
     const bool fused = !resident && mode == VSTAB_GLOBAL_SMOOTHING;
     vstab_fused_plan fp;
-    vstab_offline_fused_plan(N, world, rank, o->P, o->F, B, &fp);
+    // with auto-crop the matrices of call c come from the windows of calls c - R .. c: a window of past P + R
+    vstab_offline_fused_plan(N, world, rank, o->P + (size_t)o->crop.R, o->F, B, &fp);
     const long ring_chunks = fused ? fp.ring_chunks : 1;
     const long ring_frames = ring_chunks * B;                       // + one slot for the halo frame of the first chunk
     DevBuf& chunk = o->job_chunk; DevBuf& outc = o->job_out;
@@ -2439,6 +2506,19 @@ extern "C" vstab_status vstab_set_trail(vstab_t* s, int enable) {
     s->trail = enable != 0;
     s->epoch += 1;                       // an output prepared ahead without the trail is dropped
     return VSTAB_OK;
+}
+
+extern "C" vstab_status vstab_set_crop(vstab_t* s, double max_zoom, double release) {
+    if (!s) return VSTAB_ERR_INVALID_ARGUMENT;
+    if (!crop_params(max_zoom, release, &s->crop, s->err)) return VSTAB_ERR_INVALID_ARGUMENT;
+    s->crop_reset = true;
+    s->epoch += 1;                       // an output prepared ahead with the old crop is dropped
+    return VSTAB_OK;
+}
+
+extern "C" double vstab_crop_zoom(const double H[9], int rows, int cols, double max_zoom) {
+    if (!H || rows < 2 || cols < 2 || !(max_zoom >= 1.0 && max_zoom <= 4.0)) return -1.0;
+    return crop_need(H, rows, cols, max_zoom);
 }
 
 extern "C" vstab_status vstab_k_copy_feathered(int device, const uint8_t* fg, const uint8_t* bg, int rows, int cols, size_t step,

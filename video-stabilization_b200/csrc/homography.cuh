@@ -135,4 +135,53 @@ VSTAB_HD void compose_h(const HParams* p, double cx, double cy, double* H) {
     H[8] = 1.0;
 }
 
+// ---- auto-crop (K16, vstab_set_crop; semantics in include/vstab.h) ---------------------------------------------------
+// Zoom about the centre c0 of a rows x cols frame that keeps the warp by H from showing any point outside the pixel-centre
+// rectangle S = [0, cols-1] x [0, rows-1]: the least z >= 1 with Z(z)^-1(S) inside Q = H(S), clamped to max_zoom.
+// Q is convex when w > 0 at every corner of S; for each edge (a, b) of Q, oriented so that its inside is on the left, the
+// corner q of S shrunk towards c0 by t stays inside while s0 + t * s1 >= 0.  Operation order is fixed (the restatement in
+// tests/crop_ref.py follows it; crop.cu is built without FMA contraction).
+VSTAB_HD double crop_need(const double* H, int rows, int cols, double max_zoom) {
+    if (!finite9(H)) return max_zoom;
+    const double xs[4] = {0.0, cols - 1.0, cols - 1.0, 0.0};
+    const double ys[4] = {0.0, 0.0, rows - 1.0, rows - 1.0};
+    double qx[4], qy[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const double w = H[6] * xs[k] + H[7] * ys[k] + H[8];
+        if (!(w > 0.0)) return max_zoom;
+        qx[k] = (H[0] * xs[k] + H[1] * ys[k] + H[2]) / w;
+        qy[k] = (H[3] * xs[k] + H[4] * ys[k] + H[5]) / w;
+    }
+    double area2 = 0.0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) area2 = area2 + (qx[k] * qy[(k + 1) & 3] - qx[(k + 1) & 3] * qy[k]);
+    const double sg = area2 > 0.0 ? 1.0 : -1.0;         // edge k runs Q[k] -> Q[k+1]; sg puts its inside on the left
+    const double cx = (cols - 1.0) * 0.5, cy = (rows - 1.0) * 0.5;
+    double t = 1.0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const double ex = qx[(k + 1) & 3] - qx[k], ey = qy[(k + 1) & 3] - qy[k];
+        const double s0 = sg * (ex * (cy - qy[k]) - ey * (cx - qx[k]));
+        if (!(s0 > 0.0)) return max_zoom;               // the centre is not inside Q
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const double s1 = sg * (ex * (ys[j] - cy) - ey * (xs[j] - cx));
+            if (s1 < 0.0) {
+                const double b = s0 / -s1;
+                if (b < t) t = b;
+            }
+        }
+    }
+    const double z = 1.0 / t;
+    return z < 1.0 ? 1.0 : (z > max_zoom ? max_zoom : z);
+}
+
+// Hc = Z(z) * H, Z(z) = [[z, 0, (1-z) c0x], [0, z, (1-z) c0y], [0, 0, 1]]
+VSTAB_HD void crop_apply(double z, const double* H, int rows, int cols, double* Hc) {
+    const double cx = (cols - 1.0) * 0.5, cy = (rows - 1.0) * 0.5;
+    const double Z[9] = {z, 0.0, (1.0 - z) * cx, 0.0, z, (1.0 - z) * cy, 0.0, 0.0, 1.0};
+    matmul3(Z, H, Hc);
+}
+
 }  // namespace vstabk

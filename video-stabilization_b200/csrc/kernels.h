@@ -109,7 +109,7 @@ struct SmoothArgs {
     const double* reg;           // offline ORB / SIFT: per frame {H[9], valid} by absolute frame index, or null
     long reg_lo;                 // first frame a call after lock_call can present (lower end of the carry scan)
     double scale;                // workingHeight / rows
-    const unsigned long long* sums;   // [slot][3] channel sums by frame slot
+    const unsigned long long* sums;   // [slot][3] channel sums by frame slot; null: border left 0 (matrices only)
     long sums_mod;               // slot = abs frame % sums_mod   (ring) or abs - frame_base (offline: see frame_base)
     long frame_base;             // offline: slot = abs - frame_base; streaming: 0 with modulo
     double npix;                 // rows*cols
@@ -127,6 +127,19 @@ void launch_reg_store(const double* Tfit, const int* fit_counts, const int* nref
 void launch_acc_update(const double* T, long t_mod, long p, int reset, double* acc_state, cudaStream_t st);
 // offline: acc[k] for k in [a, a+n): acc[a] = I, acc[k] = T[k] * acc[k-1]
 void launch_acc_scan(const double* T, long n_total, long anchor, double* acc, cudaStream_t st);
+
+// ---------------------------------------------------------------- K16 auto-crop (vstab_set_crop)
+struct CropArgs {
+    double max_zoom, release;    // crop on: 1 < max_zoom <= 4, release > 0
+    int R;                       // ceil((max_zoom - 1) / release): calls a need stays in the zoom of later calls
+    int rows, cols;              // full-resolution frame
+    double* need;                // n_j of call j at need[(j - need_base) % need_mod]
+    long need_base, need_mod;
+    int reset;                   // set need[0 .. need_mod) to 1 first (streaming: the calls before the enabling call)
+};
+// n_j for the nhalo calls before call_first (warp parameters in `halo`, read only) and for calls [call_first, +n) (in wp);
+// then z_c for every call of wp, whose Hs / Minv become Z(z_c) * Hs and its inverse.
+void launch_crop(const CropArgs& a, const WarpParams* halo, int nhalo, WarpParams* wp, long call_first, int n, cudaStream_t st);
 
 // ---------------------------------------------------------------- K7 warpPerspective + border
 void launch_warp(const uint8_t* frames, size_t pitch, size_t frame_stride, long slot_mod,

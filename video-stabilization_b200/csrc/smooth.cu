@@ -149,12 +149,14 @@ smooth_kernel(SmoothArgs a, long call_first, int ncalls, WarpParams* __restrict_
     invert3(H, wp.Minv);
     const long slot = a.sums_mod > 0 ? (p % a.sums_mod) : (p - a.frame_base);
     wp.src_slot = (int)slot;
-    for (int ch = 0; ch < 3; ++ch) {
+    // no sums: the matrices alone are wanted (auto-crop's halo calls, whose presentation frames another chunk holds)
+    for (int ch = 0; ch < 3 && a.sums; ++ch) {
         const double mean = (double)a.sums[(size_t)slot * 3 + ch] / a.npix;   // cv::mean
         int v = __double2int_rn(0.5 * mean);                                  // saturate_cast<uchar>
         v = v < 0 ? 0 : (v > 255 ? 255 : v);
         wp.border[ch] = (unsigned char)v;
     }
+    if (!a.sums) wp.border[0] = wp.border[1] = wp.border[2] = 0;
     wp.border[3] = 0;
     out[ci] = wp;
 }

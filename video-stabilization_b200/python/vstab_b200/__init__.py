@@ -102,6 +102,9 @@ SYMBOLS = {
     "vstab_last_error": (C.c_char_p, [_vp]),
     "vstab_set_trail": (C.c_int, [_vp, C.c_int]),
     "vstab_set_partial_lock_fix": (C.c_int, [_vp, C.c_int]),
+    "vstab_set_crop": (C.c_int, [_vp, C.c_double, C.c_double]),
+    "vstab_crop_zoom": (C.c_double, [_f64p, C.c_int, C.c_int, C.c_double]),
+    "vstab_offline_set_crop": (C.c_int, [_vp, C.c_double, C.c_double]),
     "vstab_k_copy_feathered": (C.c_int, [C.c_int, _vp, _vp, C.c_int, C.c_int, C.c_size_t, _f64p, _vp, C.c_size_t]),
     "vstab_host_alloc": (_vp, [C.c_size_t]),
     "vstab_host_free": (None, [_vp]),
@@ -213,6 +216,19 @@ def frame_checksum(img: np.ndarray) -> int:
         return int(t.sum(dtype=np.uint64))
 
 
+CROP_RELEASE = 0.002      # default zoom release per call of set_crop and the front ends' --crop
+
+
+def crop_zoom(H: np.ndarray, rows: int, cols: int, max_zoom: float) -> float:
+    """The zoom about the centre a rows x cols frame warped by H needs to show no border (vstab_crop_zoom), at most
+    max_zoom.  Host only."""
+    Hc = np.ascontiguousarray(np.asarray(H, np.float64).reshape(9))
+    z = float(load_library().vstab_crop_zoom(Hc.ctypes.data_as(_f64p), int(rows), int(cols), float(max_zoom)))
+    if z < 0:
+        raise ValueError("crop_zoom: rows and cols must be >= 2 and max_zoom in [1, 4]")
+    return z
+
+
 def yuv_layout_packed(fmt: int, rows: int, cols: int):
     """The tight rawvideo layout of a rows x cols NV12 / I420 frame -> (YuvLayout, frame bytes).  Host only."""
     L = YuvLayout()
@@ -270,6 +286,11 @@ class Stabilizer:
         """TRANSLATION_/ROTATION_LOCK from the accumulated lock (src/stabilizer.cpp:1246-1260 fed as intended; the
         reference returns the identity in these modes, which stays the default)."""
         _check(self._lib.vstab_set_partial_lock_fix(self._h, 1 if enable else 0), self._h)
+
+    def set_crop(self, max_zoom: float, release: float = CROP_RELEASE) -> None:
+        """Auto-crop (vstab_set_crop): zoom each output about its centre just enough to hide the border of its warp, at most
+        `max_zoom` (1 < max_zoom <= 4; 1.0 turns it off), falling back by at most `release` per call."""
+        _check(self._lib.vstab_set_crop(self._h, float(max_zoom), float(release)), self._h)
 
     def set_stabilization_mode(self, mode: int) -> None:
         _check(self._lib.vstab_set_mode(self._h, int(mode)), self._h)

@@ -18,7 +18,7 @@ from __future__ import annotations
 
 import ctypes as C
 
-from . import (ACCUMULATED_FULL_LOCK, GLOBAL_SMOOTHING, SRC_DEVICE, SRC_HOST, SRC_SIMULATOR, NcclId, OfflineCfg, OfflineReport,  # noqa: F401
+from . import (ACCUMULATED_FULL_LOCK, CROP_RELEASE, GLOBAL_SMOOTHING, SRC_DEVICE, SRC_HOST, SRC_SIMULATOR, NcclId, OfflineCfg, OfflineReport,  # noqa: F401
                ShardPlan, YuvLayout, _vp, load_library, yuv_layout_packed)
 from . import _check as _check_any
 
@@ -102,6 +102,11 @@ class OfflineStabilizer:
             return None if f is None else f if isinstance(f, YuvLayout) else yuv_layout_packed(f, self.rows, self.cols)[0]
         self._yuv = (lay(in_fmt), lay(out_fmt))
         _check(self._lib.vstab_offline_set_yuv(self._h, *(C.byref(x) if x is not None else None for x in self._yuv)), self._h)
+
+    def set_crop(self, max_zoom: float, release: float = CROP_RELEASE):
+        """Auto-crop for render, run_host and run (vstab_offline_set_crop; see Stabilizer.set_crop).  With it on, render's
+        T_all must also hold the transforms of the R calls before call_first."""
+        _check(self._lib.vstab_offline_set_crop(self._h, float(max_zoom), float(release)), self._h)
 
     def estimate(self, frames, first: int, halo, T_out, sums_out=None):
         """T_out[i] <- transform frame (first+i-1) -> (first+i); sums_out[i] <- channel byte sums."""

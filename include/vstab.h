@@ -383,6 +383,10 @@ vstab_status vstab_k_lk(int device, const uint8_t* prev, const uint8_t* next, in
 vstab_status vstab_k_fit(int device, const float* prev_pts, const float* next_pts,
                          const uint8_t* status, int n, double thresh, int work_w, int work_h,
                          double M_out[6], double T_out[9], int counts_out[2]);
+/* the same estimator for up to 4096 pairs (the ORB / SIFT registration fit, one CTA on one pair set) */
+vstab_status vstab_k_fit_large(int device, const float* ref_pts, const float* cur_pts,
+                               const uint8_t* status, int n, double thresh, int work_w, int work_h,
+                               double M_out[6], double T_out[9], int counts_out[2]);
 vstab_status vstab_k_warp(int device, const uint8_t* bgr, int rows, int cols, size_t step,
                           const double H[9], const uint8_t border[3], uint8_t* out, size_t out_step);
 /* Stabilizer::copyFeathered(foreground, background, H) (src/stabilizer.cpp:1051-1155): warp + feathered alpha blend over a
@@ -412,6 +416,25 @@ vstab_status vstab_k_hamming(int device, const uint8_t* ref, int nref, const uin
  * 128 bytes each (OpenCV stores the same integers as float). */
 vstab_status vstab_k_sift(int device, const uint8_t* gray, int rows, int cols, double size_ratio,
                           float* kps_out, uint8_t* desc_out, int* n_out, int max_out);
+/* vstab_k_sift with its stages read back (tests): `calls` runs on one plan (the second captures the CUDA graph, later
+ * ones replay it), everything returned from the last.  geom[1 + 3 * 12]: octave count n, then w[12], h[12] of the
+ * octaves (base image = 2x the input) and off[12].  pyr (may be NULL, else >= pyr_cap floats): the 6 Gaussians of
+ * every octave, octave o as [6][h][w] float32 from pyr + off[o].  cand (may be NULL): the DoG extrema as
+ * octave << 56 | layer << 48 | row << 24 | col, min(count, cap, cand_max) of them.  kps_pre (may be NULL): the refined,
+ * oriented keypoints before duplicate removal and selection, {x, y, size, angle, response: float, octave: int32},
+ * min(count, cap, kp_max) of them.  counts: {candidates found, candidate capacity, keypoints found, keypoint
+ * capacity, keypoints selected}; a count above its capacity means entries were dropped (the selected keypoints
+ * beyond max_out, 4096 at most, are dropped too: retainBest keeps every tie of its threshold).  kps_out / desc_out /
+ * n_out as vstab_k_sift. */
+vstab_status vstab_k_sift_stages(int device, const uint8_t* gray, int rows, int cols, double size_ratio, int calls,
+                                 int* geom, float* pyr, size_t pyr_cap, uint64_t* cand, int cand_max,
+                                 float* kps_pre, int kp_max, int counts[5], float* kps_out, uint8_t* desc_out,
+                                 int* n_out, int max_out);
+/* The DoG extrema pass of vstab_k_sift alone on a caller-made Gaussian pyramid for a rows x cols input (tests): pyr
+ * holds the octaves of vstab_k_sift_stages' geometry one after the other without padding, each [6][h][w] float32,
+ * pyr_floats in all; cand and counts ({found, capacity}) as vstab_k_sift_stages. */
+vstab_status vstab_k_sift_extrema(int device, const float* pyr, size_t pyr_floats, int rows, int cols, uint64_t* cand,
+                                  int cand_max, int counts[2]);
 /* Exact L2 1-NN of SIFT descriptors (u8 [n][128]) on the tensor cores + the reference's distance filter
  * d <= max(0.5 * mean(d), 0.02) (src/stabilizer.cpp:675-697).  best_d2: exact squared distances. */
 vstab_status vstab_k_l2match(int device, const uint8_t* ref, int nref, const uint8_t* cur, int ncur,

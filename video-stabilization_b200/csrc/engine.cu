@@ -2714,3 +2714,112 @@ extern "C" vstab_status vstab_k_sift(int device, const uint8_t* gray, int rows, 
                         launch_sift(P, img, k, d, c, 0);
                     });
 }
+
+// K11 with its stages read back (stage tests): `calls` runs of launch_sift on ONE plan and one non-blocking stream (the
+// second call captures the CUDA graph, later calls replay it); everything returned is from the last call.
+extern "C" vstab_status vstab_k_sift_stages(int device, const uint8_t* gray, int rows, int cols, double size_ratio, int calls,
+                                            int* geom, float* pyr, size_t pyr_cap, uint64_t* cand, int cand_max,
+                                            float* kps_pre, int kp_max, int counts[5], float* kps_out, uint8_t* desc_out,
+                                            int* n_out, int max_out) {
+    auto set_err = [&](const std::string& e) { g_err = e; };
+    if (!gray || !geom || !counts || !kps_out || !desc_out || !n_out || rows < 1 || cols < 1 || calls < 1 || max_out < 1 ||
+        (cand && cand_max < 0) || (kps_pre && kp_max < 0))
+        return VSTAB_ERR_INVALID_ARGUMENT;
+    if (!device_ok(device, g_err)) return VSTAB_ERR_CUDA;
+    std::unique_ptr<SiftPlan, void (*)(SiftPlan*)> P(sift_plan_create(cols, rows, size_ratio, kOrbMaxKp, &g_err), sift_plan_destroy);
+    if (!P) return VSTAB_ERR_CUDA;
+    int w[kSiftMaxOctaves] = {}, h[kSiftMaxOctaves] = {};
+    size_t off[kSiftMaxOctaves] = {};
+    const int n_oct = sift_plan_geometry(P.get(), w, h, off);
+    geom[0] = n_oct;
+    for (int o = 0; o < kSiftMaxOctaves; ++o) {
+        geom[1 + o] = w[o]; geom[1 + kSiftMaxOctaves + o] = h[o]; geom[1 + 2 * kSiftMaxOctaves + o] = (int)off[o];
+    }
+    if (pyr && pyr_cap < P->pyr_floats) {
+        g_err = "vstab_k_sift_stages: the pyramid needs " + std::to_string(P->pyr_floats) + " floats";
+        return VSTAB_ERR_INVALID_ARGUMENT;
+    }
+    DevBuf img, kps, desc, cnt;
+    CK(img.alloc((size_t)rows * cols)); CK(kps.alloc(sizeof(OrbKeypoint) * kOrbMaxKp)); CK(desc.alloc((size_t)128 * kOrbMaxKp));
+    CK(cnt.alloc(sizeof(int)));
+    cudaStream_t st = nullptr;
+    CK(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
+    // the upload is ordered before the first launch on the same stream (a pageable cudaMemcpy on the legacy stream is not)
+    cudaMemcpyAsync(img.p, gray, (size_t)rows * cols, cudaMemcpyHostToDevice, st);
+    for (int c = 0; c < calls; ++c) launch_sift(P.get(), img.as<uint8_t>(), kps.as<OrbKeypoint>(), desc.as<uint8_t>(), cnt.as<int>(), st);
+    const cudaError_t e = cudaStreamSynchronize(st);
+    cudaStreamDestroy(st);
+    CK(e);
+    CK(cudaGetLastError());
+    int hc[3] = {0, 0, 0}, n = 0;
+    CK(cudaMemcpy(hc, P->counters, sizeof(hc), cudaMemcpyDeviceToHost));
+    counts[0] = hc[0]; counts[1] = P->cand_cap; counts[2] = hc[1]; counts[3] = P->kp_cap; counts[4] = hc[2];
+    if (pyr) CK(cudaMemcpy(pyr, P->pyr, sizeof(float) * P->pyr_floats, cudaMemcpyDeviceToHost));
+    if (cand) CK(cudaMemcpy(cand, P->cand, 8 * (size_t)std::min(std::min(hc[0], P->cand_cap), cand_max), cudaMemcpyDeviceToHost));
+    if (kps_pre) CK(cudaMemcpy(kps_pre, P->kps, sizeof(OrbKeypoint) * (size_t)std::min(std::min(hc[1], P->kp_cap), kp_max),
+                               cudaMemcpyDeviceToHost));      // SiftKp has OrbKeypoint's layout: the octave word is an int
+    CK(cudaMemcpy(&n, cnt.p, sizeof(int), cudaMemcpyDeviceToHost));
+    n = std::min(std::min(n, kOrbMaxKp), max_out);
+    *n_out = n;
+    std::vector<OrbKeypoint> hk(n);
+    CK(cudaMemcpy(hk.data(), kps.p, sizeof(OrbKeypoint) * n, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(desc_out, desc.p, (size_t)128 * n, cudaMemcpyDeviceToHost));
+    for (int i = 0; i < n; ++i) {
+        float* o = kps_out + (size_t)i * 6;
+        o[0] = hk[i].x; o[1] = hk[i].y; o[2] = hk[i].size; o[3] = hk[i].angle; o[4] = hk[i].response; o[5] = (float)hk[i].octave;
+    }
+    return VSTAB_OK;
+}
+
+// K5's estimator instantiated for kOrbMaxKp pairs (the ORB / SIFT registration fit), on one pair set of up to 4096 pairs
+extern "C" vstab_status vstab_k_fit_large(int device, const float* ref_pts, const float* cur_pts, const uint8_t* status, int n,
+                                          double thresh, int work_w, int work_h, double M_out[6], double T_out[9],
+                                          int counts_out[2]) {
+    auto set_err = [&](const std::string& e) { g_err = e; };
+    if (!ref_pts || !cur_pts || !status || !T_out || n < 0 || n > kOrbMaxKp) return VSTAB_ERR_INVALID_ARGUMENT;
+    if (!device_ok(device, g_err)) return VSTAB_ERR_CUDA;
+    DevBuf a, b, s, c, T, M, fc;
+    CK(a.alloc(sizeof(float2) * kOrbMaxKp)); CK(b.alloc(sizeof(float2) * kOrbMaxKp)); CK(s.alloc(kOrbMaxKp));
+    CK(c.alloc(sizeof(int))); CK(T.alloc(sizeof(double) * 9)); CK(M.alloc(sizeof(double) * 6)); CK(fc.alloc(sizeof(int) * 2));
+    CK(cudaMemcpy(a.p, ref_pts, sizeof(float2) * n, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(b.p, cur_pts, sizeof(float2) * n, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(s.p, status, n, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(c.p, &n, sizeof(int), cudaMemcpyHostToDevice));
+    launch_fit_large(a.as<float2>(), b.as<float2>(), s.as<uint8_t>(), c.as<int>(), thresh, work_w / 2.0, work_h / 2.0,
+                     T.as<double>(), M.as<double>(), fc.as<int>(), 0);
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(T_out, T.p, sizeof(double) * 9, cudaMemcpyDeviceToHost));
+    if (M_out) CK(cudaMemcpy(M_out, M.p, sizeof(double) * 6, cudaMemcpyDeviceToHost));
+    if (counts_out) CK(cudaMemcpy(counts_out, fc.p, sizeof(int) * 2, cudaMemcpyDeviceToHost));
+    return VSTAB_OK;
+}
+
+// The DoG extrema pass of K11 alone, on a caller-made Gaussian pyramid of a rows x cols input (tests: values planted
+// exactly at the contrast threshold).  pyr: the octaves of the plan's geometry (vstab_k_sift_stages' geom) one after the
+// other without padding, each [6][h][w] float32.  cand / counts as vstab_k_sift_stages ({found, capacity}).
+extern "C" vstab_status vstab_k_sift_extrema(int device, const float* pyr, size_t pyr_floats, int rows, int cols, uint64_t* cand,
+                                             int cand_max, int counts[2]) {
+    auto set_err = [&](const std::string& e) { g_err = e; };
+    if (!pyr || !cand || !counts || rows < 1 || cols < 1 || cand_max < 0) return VSTAB_ERR_INVALID_ARGUMENT;
+    if (!device_ok(device, g_err)) return VSTAB_ERR_CUDA;
+    std::unique_ptr<SiftPlan, void (*)(SiftPlan*)> P(sift_plan_create(cols, rows, 0.0, kOrbMaxKp, &g_err), sift_plan_destroy);
+    if (!P) return VSTAB_ERR_CUDA;
+    int w[kSiftMaxOctaves] = {}, h[kSiftMaxOctaves] = {};
+    size_t off[kSiftMaxOctaves] = {}, need = 0;
+    const int n_oct = sift_plan_geometry(P.get(), w, h, off);
+    for (int o = 0; o < n_oct; ++o) need += (size_t)6 * w[o] * h[o];
+    if (pyr_floats != need) { g_err = "vstab_k_sift_extrema: the pyramid has " + std::to_string(need) + " floats"; return VSTAB_ERR_INVALID_ARGUMENT; }
+    size_t src = 0;
+    for (int o = 0; o < n_oct; ++o) {
+        CK(cudaMemcpy(P->pyr + off[o], pyr + src, sizeof(float) * 6 * w[o] * h[o], cudaMemcpyHostToDevice));
+        src += (size_t)6 * w[o] * h[o];
+    }
+    launch_sift_extrema(P.get(), 0);
+    CK(cudaGetLastError());
+    CK(cudaDeviceSynchronize());
+    int n = 0;
+    CK(cudaMemcpy(&n, P->counters, sizeof(int), cudaMemcpyDeviceToHost));
+    counts[0] = n; counts[1] = P->cand_cap;
+    CK(cudaMemcpy(cand, P->cand, 8 * (size_t)std::min(std::min(n, P->cand_cap), cand_max), cudaMemcpyDeviceToHost));
+    return VSTAB_OK;
+}

@@ -175,7 +175,7 @@ void launch_featprep(const uint8_t* frame, size_t pitch, const int* xofs, const 
 
 
 // ---------------------------------------------------------------- CUDA-graph replay of fixed launch sequences
-// The ORB and SIFT front ends are long sequences of small dependent launches (44 / 118 per frame) whose arguments
+// The ORB and SIFT front ends are long sequences of small dependent launches (44 / 119 per frame) whose arguments
 // do not change from call to call in streaming.  The second call with the same arguments captures the sequence on
 // its stream (thread-local capture) and every later one replays the graph: one launch, no per-kernel host cost,
 // back-to-back scheduling on the device.
@@ -271,6 +271,10 @@ struct SiftPlan {
 };
 SiftPlan* sift_plan_create(int w, int h, double size_ratio, int max_keypoints, std::string* err);
 void sift_plan_destroy(SiftPlan* P);
+// octave count; w[o], h[o] and the float offset of Gaussian 0 of octave o in P->pyr (Gaussian i at off[o] + i * w * h)
+int sift_plan_geometry(const SiftPlan* P, int* w, int* h, size_t* off /* or null */);
+// the DoG extrema pass alone on whatever P->pyr holds (tests): candidates in P->cand, their count in P->counters[0]
+void launch_sift_extrema(SiftPlan* P, cudaStream_t st);
 // gray: device u8 w x h.  kps_out[max_kp] {x, y, size, angle, response, packed octave}, desc[max_kp][128] u8
 void launch_sift(SiftPlan* P, const uint8_t* gray, OrbKeypoint* kps_out, uint8_t* desc, int* count, cudaStream_t st);
 

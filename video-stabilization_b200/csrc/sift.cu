@@ -7,8 +7,9 @@
 // refinement steps, contrast and edge tests, 36-bin orientation histogram with extra keypoints for
 // peaks >= 0.8 max, removal of duplicates, retainBest(2500) by response with ties kept, 4x4x8
 // trilinear descriptor, normalise -> clip 0.2 -> normalise -> x512 -> saturate to u8.
-// Floating point, not bit-pinned: parity is stated at the homography level (<= 0.1 px) and by keypoint
-// overlap, as in SURVEY 7.2(3).  The DoG pyramid is never materialised (differences of the Gaussian
+// Floating point, not bit-pinned to cv2: each stage is pinned to a float64 restatement (tests/sift_ref.py,
+// tests/test_gpu_sift.py).  Histograms accumulate in a fixed order, and keypoints leave in KeyPoint_LessThan order, so
+// the output does not depend on scheduling.  The DoG pyramid is never materialised (differences of the Gaussian
 // levels are recomputed where needed: the same float values).
 #include <cub/device/device_radix_sort.cuh>
 #include <cmath>
@@ -386,6 +387,22 @@ VSTAB_D float atan2_deg(float y, float x) {
     return a;
 }
 
+// hist[idx] += v in a fixed order: lanes of the warp that hit the same bin add one after another by lane index (with a
+// float atomic add the hardware picks the order, and a histogram bin could change in its last bit from run to run).
+// Called by every lane of the warp; `on`: this lane has a value.
+VSTAB_D void ordered_add(float* hist, int idx, float v, bool on) {
+    const unsigned act = __ballot_sync(0xffffffffu, on);
+    if (!on) return;
+    const unsigned peers = __match_any_sync(act, idx);
+    const int lane = threadIdx.x & 31;
+    const int rank = __popc(peers & ((1u << lane) - 1u));
+    const int rounds = (int)__reduce_max_sync(act, (unsigned)__popc(peers));
+    for (int s = 0; s < rounds; ++s) {
+        if (rank == s) hist[idx] += v;
+        __syncwarp(act);
+    }
+}
+
 struct SiftKp { float x, y, size, angle, response; int octave; };   // == OrbKeypoint layout
 
 // ---------------------------------------------------------------- refine + orientation, one warp per candidate
@@ -475,18 +492,24 @@ sift_refine_kernel(const float* __restrict__ pyr, SiftOctaves O, const unsigned 
     for (int i = lane; i < 40; i += 32) hist[i] = 0.f;
     __syncwarp();
     const int side = 2 * radius + 1;
-    for (int k = lane; k < side * side; k += 32) {
+    for (int k0 = 0; k0 < side * side; k0 += 32) {           // the whole warp iterates together (ordered_add)
+        const int k = k0 + lane;
         const int i = k / side - radius, j = k - (k / side) * side - radius;
         const int y = r + i, x = c + j;
-        if (y <= 0 || y >= h - 1 || x <= 0 || x >= w - 1) continue;
-        const float dx = img[(size_t)y * w + x + 1] - img[(size_t)y * w + x - 1];
-        const float dy = img[(size_t)(y - 1) * w + x] - img[(size_t)(y + 1) * w + x];
-        const float wgt = expf((i * i + j * j) * expf_scale);
-        const float ori = atan2_deg(dy, dx), mag = sqrtf(dx * dx + dy * dy);
-        int bin = __float2int_rn((36.f / 360.f) * ori);
-        if (bin >= 36) bin -= 36;
-        if (bin < 0) bin += 36;
-        atomicAdd(&hist[2 + bin], wgt * mag);
+        const bool on = k < side * side && y > 0 && y < h - 1 && x > 0 && x < w - 1;
+        int bin = 0;
+        float v = 0.f;
+        if (on) {
+            const float dx = img[(size_t)y * w + x + 1] - img[(size_t)y * w + x - 1];
+            const float dy = img[(size_t)(y - 1) * w + x] - img[(size_t)(y + 1) * w + x];
+            const float wgt = expf((i * i + j * j) * expf_scale);
+            const float ori = atan2_deg(dy, dx), mag = sqrtf(dx * dx + dy * dy);
+            bin = __float2int_rn((36.f / 360.f) * ori);
+            if (bin >= 36) bin -= 36;
+            if (bin < 0) bin += 36;
+            v = wgt * mag;
+        }
+        ordered_add(hist, 2 + bin, v, on);
     }
     __syncwarp();
     if (lane == 0) { hist[0] = hist[2 + 34]; hist[1] = hist[2 + 35]; hist[38] = hist[2]; hist[39] = hist[3]; }
@@ -535,6 +558,34 @@ sift_keys_kernel(const SiftKp* __restrict__ kps, const int* __restrict__ nkp, in
     keys[i] = ((unsigned long long)ord(kps[i].x) << 32) | (unsigned long long)ord(kps[i].y);
 }
 
+// KeyPoint_LessThan after (x, y): size desc, angle asc, response desc, octave desc
+VSTAB_D bool kp_tail_less(const SiftKp& a, const SiftKp& b) {
+    if (a.size != b.size) return a.size > b.size;
+    if (a.angle != b.angle) return a.angle < b.angle;
+    if (a.response != b.response) return a.response > b.response;
+    return a.octave > b.octave;
+}
+
+// after sorting by (x, y): order every run of equal (x, y) by the rest of KeyPoint_LessThan, so the output order does
+// not depend on the order in which the refine kernel's atomics handed out slots.  Runs are short (the extra
+// orientations of one extremum): the first thread of a run insertion-sorts it.
+__global__ void __launch_bounds__(256)
+sift_run_order_kernel(const SiftKp* __restrict__ kps, const int* __restrict__ nkp, int kcap,
+                      const unsigned long long* __restrict__ skeys, int* __restrict__ sidx) {
+    const int n = min(*nkp, kcap);
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n || (i > 0 && skeys[i - 1] == skeys[i])) return;
+    int e = i + 1;
+    while (e < n && skeys[e] == skeys[i]) ++e;
+    for (int a = i + 1; a < e; ++a) {
+        const int v = sidx[a];
+        const SiftKp kv = kps[v];
+        int b = a - 1;
+        while (b >= i && kp_tail_less(kv, kps[sidx[b]])) { sidx[b + 1] = sidx[b]; --b; }
+        sidx[b + 1] = v;
+    }
+}
+
 // after sorting by (x, y): drop a keypoint when an earlier one in its (x, y) run has the same size and
 // angle (KeyPointsFilter::removeDuplicatedSorted); write the response keys of the survivors
 __global__ void __launch_bounds__(256)
@@ -559,7 +610,7 @@ sift_dedupe_kernel(const SiftKp* __restrict__ kps, const int* __restrict__ nkp, 
 __global__ void __launch_bounds__(1024)
 sift_select_kernel(const SiftKp* __restrict__ kps, const int* __restrict__ nkp, int kcap, const int* __restrict__ sidx,
                    const uint8_t* __restrict__ alive, const unsigned int* __restrict__ rsorted /* descending */, int nfeatures,
-                   float max_size, SiftKp* __restrict__ out, int* __restrict__ nout, int max_out) {
+                   float max_size, SiftKp* __restrict__ out, int* __restrict__ nout, int max_out, int* __restrict__ nsel) {
     __shared__ int wsum[32];
     __shared__ int s_base;
     const int n = min(*nkp, kcap);
@@ -594,7 +645,7 @@ sift_select_kernel(const SiftKp* __restrict__ kps, const int* __restrict__ nkp, 
         if (threadIdx.x == 0) { int t = 0; for (int w2 = 0; w2 < 32; ++w2) t += wsum[w2]; s_base += t; }
         __syncthreads();
     }
-    if (threadIdx.x == 0) *nout = min(s_base, max_out);
+    if (threadIdx.x == 0) { *nout = min(s_base, max_out); *nsel = s_base; }   // nsel > max_out: retainBest's ties overflowed
 }
 
 // ---------------------------------------------------------------- descriptor, one CTA of 128 threads per keypoint
@@ -602,7 +653,8 @@ __global__ void __launch_bounds__(128)
 sift_descriptor_kernel(const float* __restrict__ pyr, SiftOctaves O, const SiftKp* __restrict__ kps, const int* __restrict__ nkp,
                        int max_kp, uint8_t* __restrict__ desc) {
     constexpr int d = 4, nb = 8;
-    __shared__ float hist[(d + 2) * (d + 2) * (nb + 2)];
+    constexpr int HL = (d + 2) * (d + 2) * (nb + 2);
+    __shared__ float whist[4][HL];                 // one histogram per warp, summed in warp order at the end
     __shared__ float dst[d * d * nb];
     __shared__ float red[4];
     const int n = min(*nkp, max_kp);
@@ -628,15 +680,21 @@ sift_descriptor_kernel(const float* __restrict__ pyr, SiftOctaves O, const SiftK
     int radius = __float2int_rn(hist_width * 1.4142135623730951f * (d + 1) * 0.5f);
     radius = min(radius, (int)sqrt((double)w * w + (double)h * h));
     cos_t /= hist_width; sin_t /= hist_width;
-    for (int i = threadIdx.x; i < (d + 2) * (d + 2) * (nb + 2); i += 128) hist[i] = 0.f;
+    for (int i = threadIdx.x; i < 4 * HL; i += 128) whist[i / HL][i % HL] = 0.f;
     __syncthreads();
+    float* hist = whist[threadIdx.x >> 5];
     const int side = 2 * radius + 1;
-    for (int k = threadIdx.x; k < side * side; k += 128) {
+    for (int k0 = 0; k0 < side * side; k0 += 128) {          // whole warps iterate together (ordered_add)
+        const int k = k0 + threadIdx.x;
         const int i = k / side - radius, j = k - (k / side) * side - radius;
         const float c_rot = j * cos_t - i * sin_t, r_rot = j * sin_t + i * cos_t;
         float rbin = r_rot + d / 2 - 0.5f, cbin = c_rot + d / 2 - 0.5f;
         const int r = pty + i, c = ptx + j;
-        if (rbin > -1 && rbin < d && cbin > -1 && cbin < d && r > 0 && r < h - 1 && c > 0 && c < w - 1) {
+        const bool on = k < side * side && rbin > -1 && rbin < d && cbin > -1 && cbin < d && r > 0 && r < h - 1 && c > 0 &&
+                        c < w - 1;
+        float v8[8] = {};
+        int idx = 0;
+        if (on) {
             const float dx = img[(size_t)r * w + c + 1] - img[(size_t)r * w + c - 1];
             const float dy = img[(size_t)(r - 1) * w + c] - img[(size_t)(r + 1) * w + c];
             const float wgt = expf((c_rot * c_rot + r_rot * r_rot) * exp_scale);
@@ -654,26 +712,26 @@ sift_descriptor_kernel(const float* __restrict__ pyr, SiftOctaves O, const SiftK
             const float v_rco101 = v_rc10 * obin, v_rco100 = v_rc10 - v_rco101;
             const float v_rco011 = v_rc01 * obin, v_rco010 = v_rc01 - v_rco011;
             const float v_rco001 = v_rc00 * obin, v_rco000 = v_rc00 - v_rco001;
-            const int idx = ((r0 + 1) * (d + 2) + c0 + 1) * (nb + 2) + o0;
-            atomicAdd(&hist[idx], v_rco000);
-            atomicAdd(&hist[idx + 1], v_rco001);
-            atomicAdd(&hist[idx + (nb + 2)], v_rco010);
-            atomicAdd(&hist[idx + (nb + 3)], v_rco011);
-            atomicAdd(&hist[idx + (d + 2) * (nb + 2)], v_rco100);
-            atomicAdd(&hist[idx + (d + 2) * (nb + 2) + 1], v_rco101);
-            atomicAdd(&hist[idx + (d + 3) * (nb + 2)], v_rco110);
-            atomicAdd(&hist[idx + (d + 3) * (nb + 2) + 1], v_rco111);
+            idx = ((r0 + 1) * (d + 2) + c0 + 1) * (nb + 2) + o0;
+            v8[0] = v_rco000; v8[1] = v_rco001; v8[2] = v_rco010; v8[3] = v_rco011;
+            v8[4] = v_rco100; v8[5] = v_rco101; v8[6] = v_rco110; v8[7] = v_rco111;
         }
+        constexpr int kOff[8] = {0, 1, nb + 2, nb + 3, (d + 2) * (nb + 2), (d + 2) * (nb + 2) + 1, (d + 3) * (nb + 2),
+                                 (d + 3) * (nb + 2) + 1};
+#pragma unroll
+        for (int q = 0; q < 8; ++q) ordered_add(hist, idx + kOff[q], v8[q], on);
     }
+    __syncthreads();
+    for (int i = threadIdx.x; i < HL; i += 128) whist[0][i] = ((whist[0][i] + whist[1][i]) + whist[2][i]) + whist[3][i];
     __syncthreads();
     // finalize: fold the circular orientation bins, gather the 4x4x8 core
     {
         const int t = threadIdx.x;                 // 128 = d*d*nb outputs
         const int i = t / (d * nb), j = (t / nb) % d, k = t % nb;
         const int idx = ((i + 1) * (d + 2) + (j + 1)) * (nb + 2);
-        float v = hist[idx + k];
-        if (k == 0) v += hist[idx + nb];
-        if (k == 1) v += hist[idx + nb + 1];
+        float v = whist[0][idx + k];
+        if (k == 0) v += whist[0][idx + nb];
+        if (k == 1) v += whist[0][idx + nb + 1];
         dst[t] = v;
     }
     __syncthreads();
@@ -726,7 +784,10 @@ SiftPlan* sift_plan_create(int w, int h, double size_ratio, int max_keypoints, s
     int cw = bw, ch = bh;
     for (int o = 0; o < nOct; ++o) {
         O.w[o] = cw; O.h[o] = ch; O.off[o] = off;
-        off += (size_t)kGauss * cw * ch;
+        // every octave starts on a 256-byte boundary: the extrema kernel reads rows of an octave whose width is a
+        // multiple of 4 as float4, and 6 w h floats of an octave with odd w and h (41 x 31 at 333 x 250) would leave
+        // the next one only 8-byte aligned
+        off += al256(sizeof(float) * kGauss * cw * ch) / sizeof(float);
         cw /= 2; ch /= 2;
         if (cw < 1 || ch < 1) { O.n = o + 1; break; }
     }
@@ -772,6 +833,12 @@ SiftPlan* sift_plan_create(int w, int h, double size_ratio, int max_keypoints, s
     return P;
 }
 
+int sift_plan_geometry(const SiftPlan* P, int* w, int* h, size_t* off) {
+    const SiftOctaves& O = *(const SiftOctaves*)P->octaves;
+    for (int o = 0; o < O.n; ++o) { w[o] = O.w[o]; h[o] = O.h[o]; if (off) off[o] = O.off[o]; }
+    return O.n;
+}
+
 void sift_plan_destroy(SiftPlan* P) {
     if (!P) return;
     for (auto& a : P->aux) if (a) cudaStreamDestroy(a);
@@ -783,6 +850,23 @@ void sift_plan_destroy(SiftPlan* P) {
 }
 
 static void launch_sift_body(SiftPlan* P, const uint8_t* gray, OrbKeypoint* kps_out, uint8_t* desc, int* count, cudaStream_t st);
+
+// DoG extrema of octave o of P->pyr appended to P->cand / counters[0]; false when the octave has no interior
+static bool launch_extrema(SiftPlan* P, int o, cudaStream_t st) {
+    const SiftOctaves& O = *(const SiftOctaves*)P->octaves;
+    const int w = O.w[o], h = O.h[o];
+    if (w <= 2 * kBorder || h <= 2 * kBorder) return false;
+    const int threshold = (int)std::floor(0.5 * 0.04 / kLayers * 255.0);
+    sift_extrema_tile_kernel<<<dim3((w - 2 * kBorder + EXW - 1) / EXW, (h - 2 * kBorder + EXH - 1) / EXH), 256, 0, st>>>(
+        P->pyr, O, o, threshold, P->cand, P->counters + 0, P->cand_cap);
+    return true;
+}
+
+void launch_sift_extrema(SiftPlan* P, cudaStream_t st) {
+    cudaMemsetAsync(P->counters, 0, sizeof(int), st);
+    const int n = ((const SiftOctaves*)P->octaves)->n;
+    for (int o = 0; o < n; ++o) launch_extrema(P, o, st);
+}
 
 void launch_sift(SiftPlan* P, const uint8_t* gray, OrbKeypoint* kps_out, uint8_t* desc, int* count, cudaStream_t st) {
     // ~120 small dependent launches per frame: replayed as one CUDA graph from the third call with the same buffers on
@@ -819,7 +903,6 @@ static void launch_sift_body(SiftPlan* P, const uint8_t* gray, OrbKeypoint* kps_
     float* scratch = g0 + (size_t)O.w[0] * O.h[0];
     sift_upsample_kernel<<<dim3((P->w + 255) / 256, P->h), 256, 0, st>>>(gray, P->w, P->h, scratch);
     blur(scratch, g0, O.w[0], O.h[0], 0, st);
-    const int threshold = (int)std::floor(0.5 * 0.04 / kLayers * 255.0);
     // Octave o + 1 starts from Gaussian[kLayers] of octave o, so it does not have to wait for the last two blurs and the
     // extrema pass of octave o: octaves >= 1 alternate between two auxiliary streams (fork / join by events; inside a
     // graph capture these become parallel branches).  The small octaves are ~40 launches of a few CTAs each, about
@@ -851,11 +934,7 @@ static void launch_sift_body(SiftPlan* P, const uint8_t* gray, OrbKeypoint* kps_
             ++launches;
             if (i == kLayers && o + 1 < O.n) cudaEventRecord(P->ev_g3[o], q);
         }
-        if (w > 2 * kBorder && h > 2 * kBorder) {
-            sift_extrema_tile_kernel<<<dim3((w - 2 * kBorder + EXW - 1) / EXW, (h - 2 * kBorder + EXH - 1) / EXH), 256, 0, q>>>(
-                P->pyr, O, o, threshold, P->cand, P->counters + 0, P->cand_cap);
-            ++launches;
-        }
+        if (launch_extrema(P, o, q)) ++launches;
     }
     for (int k = 0; k < 2; ++k)
         if (used[k]) { cudaEventRecord(P->ev_join[k], P->aux[k]); cudaStreamWaitEvent(st, P->ev_join[k], 0); }
@@ -866,14 +945,15 @@ static void launch_sift_body(SiftPlan* P, const uint8_t* gray, OrbKeypoint* kps_
     size_t temp = P->cub_bytes;
     cub::DeviceRadixSort::SortPairs(P->cub_temp, temp, (const unsigned long long*)P->keys, P->keys_sorted, (const int*)P->idx,
                                     P->idx_sorted, P->kp_cap, 0, 64, st);
+    sift_run_order_kernel<<<(P->kp_cap + 255) / 256, 256, 0, st>>>(kps, P->counters + 1, P->kp_cap, P->keys_sorted, P->idx_sorted);
     sift_dedupe_kernel<<<(P->kp_cap + 255) / 256, 256, 0, st>>>(kps, P->counters + 1, P->kp_cap, P->keys_sorted, P->idx_sorted,
                                                                P->rkeys, P->alive);
     temp = P->cub_bytes;
     cub::DeviceRadixSort::SortKeysDescending(P->cub_temp, temp, (const unsigned int*)P->rkeys, P->rkeys_sorted, P->kp_cap, 0, 32, st);
     sift_select_kernel<<<1, 1024, 0, st>>>(kps, P->counters + 1, P->kp_cap, P->idx_sorted, P->alive, P->rkeys_sorted, 2500,
-                                          P->max_size, (SiftKp*)kps_out, count, P->max_kp);
+                                          P->max_size, (SiftKp*)kps_out, count, P->max_kp, P->counters + 2);
     sift_descriptor_kernel<<<P->max_kp, 128, 0, st>>>(P->pyr, O, (const SiftKp*)kps_out, count, P->max_kp, desc);
-    count_launch(launches + 6);
+    count_launch(launches + 7);
 }
 
 }  // namespace vstabk

@@ -157,6 +157,11 @@ SYMBOLS = {
     "vstab_k_l2match": (C.c_int, [C.c_int, _vp, C.c_int, _vp, C.c_int, _vp, _vp, _vp]),
     "vstab_k_l2match_batch": (C.c_int, [C.c_int, _vp, C.c_int, _vp, C.POINTER(C.c_int), C.c_int, _vp, _vp, C.c_int, C.POINTER(C.c_float)]),
     "vstab_k_sift": (C.c_int, [C.c_int, _vp, C.c_int, C.c_int, C.c_double, _vp, _vp, C.POINTER(C.c_int), C.c_int]),
+    "vstab_k_sift_stages": (C.c_int, [C.c_int, _vp, C.c_int, C.c_int, C.c_double, C.c_int, _vp, _vp, C.c_size_t, _vp, C.c_int,
+                                      _vp, C.c_int, _vp, _vp, _vp, C.POINTER(C.c_int), C.c_int]),
+    "vstab_k_sift_extrema": (C.c_int, [C.c_int, _vp, C.c_size_t, C.c_int, C.c_int, _vp, C.c_int, _vp]),
+    "vstab_k_fit_large": (C.c_int, [C.c_int, _vp, _vp, _vp, C.c_int, C.c_double, C.c_int, C.c_int, _f64p, _f64p,
+                                    C.POINTER(C.c_int)]),
 }
 
 _lib = None
@@ -466,6 +471,20 @@ def k_fit(prev_pts, next_pts, status, work_w, work_h, thresh=3.0, device: int = 
     return M, T, (cnt[0], cnt[1])
 
 
+def k_fit_large(ref_pts, cur_pts, status, work_w, work_h, thresh=5.0, device: int = 0):
+    """k_fit's estimator instantiated for up to 4096 pairs (the ORB / SIFT registration fit)."""
+    lib = load_library()
+    a = np.ascontiguousarray(ref_pts, np.float32)
+    b = np.ascontiguousarray(cur_pts, np.float32)
+    s = np.ascontiguousarray(status, np.uint8)
+    M = np.zeros((2, 3))
+    T = np.zeros((3, 3))
+    cnt = (C.c_int * 2)()
+    _check(lib.vstab_k_fit_large(device, _ptr(a), _ptr(b), _ptr(s), len(a), thresh, work_w, work_h,
+                                 M.ctypes.data_as(_f64p), T.ctypes.data_as(_f64p), cnt))
+    return M, T, (cnt[0], cnt[1])
+
+
 def k_warp(bgr: np.ndarray, H: np.ndarray, border, device: int = 0):
     lib = load_library()
     bgr = np.ascontiguousarray(bgr)
@@ -590,3 +609,67 @@ def k_sift(gray: np.ndarray, size_ratio: float = 0.0, device: int = 0):
     _check(lib.vstab_k_sift(device, _ptr(gray), gray.shape[0], gray.shape[1], float(size_ratio), _ptr(kps), _ptr(desc),
                             C.byref(n), 4096))
     return kps[:n.value].copy(), desc[:n.value].copy()
+
+
+SIFT_KP_DTYPE = np.dtype([("x", "<f4"), ("y", "<f4"), ("size", "<f4"), ("angle", "<f4"), ("response", "<f4"), ("octave", "<i4")])
+
+
+@dataclass
+class SiftStages:
+    """What vstab_k_sift_stages reads back: `pyr[o]` float32 [6, h, w] per octave, `cand` uint64 DoG extrema
+    (octave << 56 | layer << 48 | row << 24 | col), `kps_pre` SIFT_KP_DTYPE records before duplicate removal and
+    selection, the raw counters and capacities, `n_sel` the keypoints selected (the output keeps the first 4096), and the
+    final keypoints / descriptors as k_sift returns them."""
+    pyr: list
+    cand: np.ndarray
+    n_cand: int
+    cand_cap: int
+    kps_pre: np.ndarray
+    n_kp: int
+    kp_cap: int
+    n_sel: int
+    kps: np.ndarray
+    desc: np.ndarray
+
+
+def k_sift_stages(gray: np.ndarray, size_ratio: float = 0.0, calls: int = 1, device: int = 0) -> SiftStages:
+    """vstab_k_sift_stages: one plan, `calls` runs (graph capture from the second, replay from the third), every stage
+    of the last run."""
+    lib = load_library()
+    gray = np.ascontiguousarray(gray, np.uint8)
+    rows, cols = gray.shape
+    geom = np.zeros(37, np.int32)
+    # bounds: the octaves of the 2x base image hold at most 4/3 of its pixels, 6 Gaussians each, each octave padded
+    # to 64 floats; candidates at most the capacity the plan gives them (base pixels / 16 + 65536, rounded up to 256)
+    pyr = np.zeros(6 * (4 * rows * cols * 4 // 3) + 64 * 12, np.float32)
+    cand_max = 4 * rows * cols // 16 + 65536 + 256
+    cand = np.zeros(cand_max, np.uint64)
+    kp_max = 1 << 18
+    pre = np.zeros(kp_max, SIFT_KP_DTYPE)
+    counts = np.zeros(5, np.int32)
+    kps = np.zeros((4096, 6), np.float32)
+    desc = np.zeros((4096, 128), np.uint8)
+    n = C.c_int(0)
+    _check(lib.vstab_k_sift_stages(device, _ptr(gray), rows, cols, float(size_ratio), int(calls), _ptr(geom), _ptr(pyr),
+                                   pyr.size, _ptr(cand), cand_max, _ptr(pre), kp_max, _ptr(counts), _ptr(kps), _ptr(desc),
+                                   C.byref(n), 4096))
+    levels = []
+    for o in range(int(geom[0])):
+        w, h, off = int(geom[1 + o]), int(geom[13 + o]), int(geom[25 + o])
+        levels.append(pyr[off:off + 6 * w * h].reshape(6, h, w).copy())
+    n_cand, n_kp = int(counts[0]), int(counts[2])
+    return SiftStages(levels, cand[:min(n_cand, int(counts[1]), cand_max)].copy(), n_cand, int(counts[1]),
+                      pre[:min(n_kp, int(counts[3]), kp_max)].copy(), n_kp, int(counts[3]), int(counts[4]),
+                      kps[:n.value].copy(), desc[:n.value].copy())
+
+
+def k_sift_extrema(pyr, rows: int, cols: int, device: int = 0):
+    """The DoG extrema pass alone on a caller-made Gaussian pyramid (list over octaves of float32 [6, h, w] in the
+    geometry of a rows x cols input) -> (candidate words uint64, found, capacity)."""
+    lib = load_library()
+    flat = np.ascontiguousarray(np.concatenate([np.asarray(g, np.float32).ravel() for g in pyr]))
+    cand_max = 4 * rows * cols // 16 + 65536 + 256
+    cand = np.zeros(cand_max, np.uint64)
+    counts = np.zeros(2, np.int32)
+    _check(lib.vstab_k_sift_extrema(device, _ptr(flat), flat.size, rows, cols, _ptr(cand), cand_max, _ptr(counts)))
+    return cand[:min(int(counts[0]), int(counts[1]), cand_max)].copy(), int(counts[0]), int(counts[1])

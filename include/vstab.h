@@ -246,8 +246,11 @@ vstab_status vstab_offline_prepare(vstab_offline_t* o, const double* d_T_all, lo
 /* Whole-clip stabilization with HOST buffers on one GPU (the reference's --file input,
  * src/main_utils.cpp:397-417 feeding stabilizeFrame at :465): `frames` holds n_total BGR frames
  * `frame_stride` bytes apart, `out` receives the outputs of stabilizeFrame calls 0..n_total-1.
- * Uploads, estimation, warping and downloads are pipelined over chunks of max_batch frames on
- * three streams; every frame crosses PCIe once per direction.  Use pinned buffers
+ * This is vstab_offline_run (below) with a HOST source and host_out, as a world of one whatever
+ * communicator the instance has joined: every mode is accepted, uploads, estimation, warping and
+ * downloads are pipelined over chunks of max_batch frames, and device memory is bounded by the
+ * chunk ring of the fused pass, not by the clip length; every frame crosses PCIe once per
+ * direction (ORB / SIFT lock: uploaded twice, like the job's two passes).  Use pinned buffers
  * (vstab_host_alloc) for asynchronous copies.  Synchronous: returns when `out` is complete. */
 vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t* frames, size_t frame_stride,
                                     size_t step, long n_total, int mode, long lock_call,
@@ -303,7 +306,9 @@ uintptr_t vstab_offline_stream(vstab_offline_t* o);
  * window lies inside the rank's own transforms is warped right behind the estimation, out of a ring of the last
  * ceil((F-1)/max_batch) + 3 chunks (source, estimation and warp on three streams) -- a frame is uploaded / rendered
  * once; only the first P-1 and last F-1 calls of a rank in a world > 1 wait for the exchange and fetch their frames
- * again.  The other modes need the global prefix / the broadcast reference and fetch every frame in both passes.
+ * again.  In a world of one the fused pass covers every LK-path mode (ACCUMULATED_FULL_LOCK rescans the prefix of the
+ * transforms estimated so far before each warp step).  The other cases need the global prefix / the broadcast
+ * reference and fetch every frame in both passes.  Outputs for host_out leave on a download stream of their own.
  * Outputs go to host memory and / or are reduced to one 64-bit checksum per call (see vstab_frame_checksum).  With no communicator the
  * instance is a world of one.  Replaces the reference's --file / --simulator loop around stabilizeFrame
  * (src/main_utils.cpp:397-417, 459-493) for clips that are sharded over GPUs. */

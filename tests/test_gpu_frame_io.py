@@ -15,7 +15,7 @@ torch = pytest.importorskip("torch")
 
 W, H, WH, P, F, N, B = 480, 270, 135, 6, 4, 30, 7
 SENTINEL = 0xEE
-MODES = [(vs.GLOBAL_SMOOTHING, 0), (vs.ACCUMULATED_FULL_LOCK, 11)]     # offline_run: the fused pass, then the two passes
+MODES = [(vs.GLOBAL_SMOOTHING, 0), (vs.ACCUMULATED_FULL_LOCK, 11)]     # window average, then the prefix rescanned per chunk
 
 
 def _clip(tex_np, w, h, n):

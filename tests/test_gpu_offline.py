@@ -134,18 +134,22 @@ def test_offline_equals_streaming(texture_small, lock_at, shards):
         assert np.array_equal(got[c], want[c]), c
 
 
-@pytest.mark.parametrize("lock_at", [None, 9])
-def test_run_host_equals_streaming(texture_small, lock_at):
-    """vstab_offline_run_host (pipelined uploads / estimation / warps / downloads over host buffers)
-    returns exactly the frames the streaming calls return."""
-    W, H, wh, P, F = 480, 270, 135, 6, 4
+@pytest.mark.parametrize("mode,lock_at,F", [pytest.param(vs.GLOBAL_SMOOTHING, None, 4, id="None"),
+                                            pytest.param(vs.ACCUMULATED_FULL_LOCK, 9, 4, id="9"),
+                                            pytest.param(vs.ACCUMULATED_FULL_LOCK, 9, 0, id="future0-9"),
+                                            pytest.param(vs.ORB_FULL_LOCK, 9, 4, id="orb-9")])
+def test_run_host_equals_streaming(texture_small, mode, lock_at, F):
+    """vstab_offline_run_host (vstab_offline_run's job on one GPU: uploads / estimation / warps / downloads pipelined over
+    host buffers) returns exactly the frames the streaming calls return: with future 0 (a call presents the frame it
+    receives), and in ORB lock (at the size of the feature-lock test below)."""
+    W, H, wh = (640, 360, 360) if mode == vs.ORB_FULL_LOCK else (480, 270, 135)
+    P = 6
     frames, _ = _dev_clip(texture_small, W, H, 30)
     f_np = np.ascontiguousarray(frames.cpu().numpy())
-    want, _ = _streaming(f_np, P, F, wh, lock_at)
-    mode = vs.GLOBAL_SMOOTHING if lock_at is None else vs.ACCUMULATED_FULL_LOCK
+    want = _streaming_mode(f_np, P, F, wh, mode, lock_at)
     out = np.zeros_like(f_np)
     off = offline.OfflineStabilizer(P, F, wh, H, W, 7)
-    for _ in range(2):                    # second run reuses the instance's device clip buffers
+    for _ in range(2):                    # second run reuses the instance's chunk ring and output chunks
         off.run_host(f_np.ctypes.data, f_np.strides[0], f_np.strides[1], 30, mode, lock_at or 0,
                      out.ctypes.data, out.strides[0], out.strides[1])
         for c in range(30):

@@ -72,7 +72,7 @@ def run_host(vs, host, out, crop):
         off.set_crop(*CROP)
     args = (host.ctypes.data, host.strides[0], host.strides[1], n, vs.GLOBAL_SMOOTHING, 0, out.ctypes.data, out.strides[0],
             out.strides[1])
-    off.run_host(*args)                                            # warm-up: device clip buffers, events
+    off.run_host(*args)                                            # warm-up: chunk ring, output chunks, streams
     t0 = time.perf_counter()
     off.run_host(*args)
     dt = time.perf_counter() - t0

@@ -1291,10 +1291,6 @@ struct vstab_offline {
     const double* acc_T = nullptr;
     int last_ncalls = 0;
     StageTimer timer;
-    // host-clip runner (vstab_offline_run_host): device-resident clip, double-buffered output chunks
-    DevBuf clip, outbuf, clipT, clipSums;
-    size_t clip_frames = 0;
-    cudaStream_t copy_in = nullptr, copy_out = nullptr;
     // ORB / SIFT registration (offline): packed reference set (RefSet) and its mode, gathered registrations
     int ref_mode = -1;
     DevBuf ref_pack;
@@ -1304,16 +1300,16 @@ struct vstab_offline {
     // lanes; lane 0 runs on `stream` (it also captures the reference set), every other one on a stream of its own
     std::vector<std::unique_ptr<RegLane>> lanes;
     cudaEvent_t ev_reg_fork = nullptr;
-    // sharded job (vstab_offline_run): NCCL communicator of this rank, chunk buffers kept between runs
+    // sharded job (vstab_offline_run, vstab_offline_run_host): NCCL communicator of this rank, chunk ring, output chunks and
+    // YUV staging kept between runs; the streams of the fused pass (source: copy_in, warp: copy_out) and of downloads to a
+    // host sink
     void* comm = nullptr;
     int rank = 0, world = 1;
-    DevBuf job_chunk, job_out;
-    size_t job_chunk_frames = 0;
-    std::vector<cudaEvent_t> host_events;         // vstab_offline_run_host: upload / render / download / conversion marks per chunk
-    // YUV layouts of the frames of run_host / run (vstab_offline_set_yuv; none: BGR), and run_host's double-buffered
-    // staging of host YUV frames (2 x max_batch frames each)
+    DevBuf job_chunk, job_out, job_stage;
+    size_t job_chunk_frames = 0, job_out_frames = 0, job_stage_bytes = 0;
+    cudaStream_t copy_in = nullptr, copy_out = nullptr, download = nullptr;
+    // YUV layouts of the frames of run_host / run (vstab_offline_set_yuv; none: BGR)
     std::optional<vstab_yuv_layout> yin, yout;
-    DevBuf ystage_in, ystage_out;
     // auto-crop (vstab_offline_set_crop): every render recomputes the warp parameters of the R calls before its first one
     // (crop_halo) and their needs (crop_need, halo + batch), so no state is carried from one render to the next
     CropArgs crop{1.0, 0.0, 0};
@@ -1477,9 +1473,9 @@ void vstab_offline_destroy(vstab_offline_t* o) {
     if (o->stream) { cudaStreamSynchronize(o->stream); cudaStreamDestroy(o->stream); }
     if (o->copy_in) { cudaStreamSynchronize(o->copy_in); cudaStreamDestroy(o->copy_in); }
     if (o->copy_out) { cudaStreamSynchronize(o->copy_out); cudaStreamDestroy(o->copy_out); }
+    if (o->download) { cudaStreamSynchronize(o->download); cudaStreamDestroy(o->download); }
     if (o->ev_reg_fork) cudaEventDestroy(o->ev_reg_fork);
     if (o->comm) nccl_comm_destroy(o->comm);
-    for (auto e : o->host_events) if (e) cudaEventDestroy(e);
     delete o;
 }
 
@@ -1632,6 +1628,33 @@ extern "C" vstab_status vstab_offline_render(vstab_offline_t* o, const uint8_t* 
                                d_sums, d_out, out_frame_stride, out_step, nullptr);
 }
 
+// o->acc sized for the prefix of n_total transforms (n_total matrices, then the scan's n_total / 256 + 2 block products)
+static vstab_status offline_acc_reserve(vstab_offline_t* o, long n_total) {
+    auto set_err = [&](const std::string& e) { o->err = e; };
+    const size_t mats = (size_t)n_total + (size_t)(n_total / 256 + 2);
+    if (o->acc_capacity < mats) { CK(o->acc.alloc(sizeof(double) * 9 * mats)); o->acc_capacity = mats; }
+    return VSTAB_OK;
+}
+
+// vstab_offline_prepare on stream q
+static vstab_status offline_prepare(vstab_offline_t* o, const double* d_T_all, long n_total, int mode, long lock_call,
+                                    cudaStream_t q) {
+    auto set_err = [&](const std::string& e) { o->err = e; };
+    if (mode != VSTAB_ACCUMULATED_FULL_LOCK) { o->acc_T = nullptr; return VSTAB_OK; }
+    if (lock_call < (long)o->F) {
+        o->err = "ACCUMULATED_FULL_LOCK must be set at a call index >= future (SURVEY B.6)"; return VSTAB_ERR_STATE;
+    }
+    const long anchor = lock_call - (long)o->F;
+    vstab_status st = offline_acc_reserve(o, n_total);
+    if (st != VSTAB_OK) return st;
+    o->timer.begin(ST_ACC, q);
+    launch_acc_scan(d_T_all, n_total, anchor, o->acc.as<double>(), q);
+    o->timer.end(ST_ACC, q);
+    CK(cudaGetLastError());
+    o->acc_T = d_T_all; o->acc_n_total = n_total; o->acc_anchor = anchor;
+    return VSTAB_OK;
+}
+
 // The "segmented prefix/scan over 3x3 transforms" of the north star: accumulated products
 // acc[k] = T[k] * ... * T[anchor+1] for the whole clip, needed by ACCUMULATED_FULL_LOCK
 // (src/stabilizer.cpp:317-338).  Runs every time it is called (no caching of results).
@@ -1640,122 +1663,7 @@ extern "C" vstab_status vstab_offline_prepare(vstab_offline_t* o, const double* 
     if (!o || !d_T_all || n_total < 1) return VSTAB_ERR_INVALID_ARGUMENT;
     auto set_err = [&](const std::string& e) { o->err = e; };
     CK(cudaSetDevice(o->device));
-    if (mode != VSTAB_ACCUMULATED_FULL_LOCK) { o->acc_T = nullptr; return VSTAB_OK; }
-    if (lock_call < (long)o->F) {
-        o->err = "ACCUMULATED_FULL_LOCK must be set at a call index >= future (SURVEY B.6)"; return VSTAB_ERR_STATE;
-    }
-    const long anchor = lock_call - (long)o->F;
-    const size_t mats = (size_t)n_total + (size_t)(n_total / 256 + 2);
-    if (o->acc_capacity < mats) { CK(o->acc.alloc(sizeof(double) * 9 * mats)); o->acc_capacity = mats; }
-    o->timer.begin(ST_ACC, o->stream);
-    launch_acc_scan(d_T_all, n_total, anchor, o->acc.as<double>(), o->stream);
-    o->timer.end(ST_ACC, o->stream);
-    CK(cudaGetLastError());
-    o->acc_T = d_T_all; o->acc_n_total = n_total; o->acc_anchor = anchor;
-    return VSTAB_OK;
-}
-
-// Whole-clip stabilization with HOST buffers on one GPU (the reference's --file mode: decoded
-// frames in host memory in, stabilized frames out).  Produces the outputs of stabilizeFrame calls
-// 0..n_total-1 (call c presents frame max(0, c - future)).  One software pipeline over chunks of
-// max_batch frames on three streams (both PCIe directions busy at the same time):
-//   upload chunk k+1  ||  estimate + smooth + warp chunk k  ||  download chunk k-1
-// Every frame crosses PCIe exactly once in each direction; the clip stays resident in HBM
-// (6.2 MB per 1080p frame: ~29 k frames fit in 180 GB).
-extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t* frames, size_t frame_stride, size_t step,
-                                                long n_total, int mode, long lock_call, uint8_t* out,
-                                                size_t out_frame_stride, size_t out_step) {
-    if (!o || !frames || !out || n_total < 1) return VSTAB_ERR_INVALID_ARGUMENT;
-    auto set_err = [&](const std::string& e) { o->err = e; };
-    Geometry& g = o->g;
-    const FrameFmt in_fmt{true, o->yin ? &*o->yin : nullptr, step, frame_stride};
-    const FrameFmt out_fmt{true, o->yout ? &*o->yout : nullptr, out_step, out_frame_stride};
-    vstab_status st = in_fmt.check(g.rows, g.cols, true, o->err);
-    if (st == VSTAB_OK) st = out_fmt.check(g.rows, g.cols, true, o->err);
-    if (st != VSTAB_OK) return st;
-    CK(cudaSetDevice(o->device));
-    if (!o->copy_in) CK(cudaStreamCreateWithFlags(&o->copy_in, cudaStreamNonBlocking));
-    if (!o->copy_out) CK(cudaStreamCreateWithFlags(&o->copy_out, cudaStreamNonBlocking));
-    const int B = o->max_batch;
-    if (o->clip_frames < (size_t)n_total) {
-        CK(o->clip.alloc(g.frame_bytes * (size_t)n_total + 64));
-        CK(o->outbuf.alloc(g.frame_bytes * (size_t)B * 2 + 64));
-        CK(o->clipT.alloc(sizeof(double) * 9 * (size_t)n_total));
-        CK(o->clipSums.alloc(sizeof(unsigned long long) * 3 * (size_t)n_total));
-        o->clip_frames = (size_t)n_total;
-    }
-    uint8_t* clip = o->clip.as<uint8_t>();
-    double* T = o->clipT.as<double>();
-    unsigned long long* sums = o->clipSums.as<unsigned long long>();
-    // host YUV frames cross the link in staging buffers of two halves of B frames: upload(k) -> convert(k) into the clip,
-    // and render(k) -> convert(k) -> download(k), the halves alternating with k
-    const size_t half_in = in_fmt.staging_bytes(g) * (size_t)B, half_out = out_fmt.staging_bytes(g) * (size_t)B;
-    if (half_in && !o->ystage_in.p) CK(o->ystage_in.alloc(2 * half_in));
-    if (half_out && !o->ystage_out.p) CK(o->ystage_out.alloc(2 * half_out));
-    const long nchunks = (n_total + B - 1) / B;
-    // per-chunk events live in the instance (created once, reused by every call, destroyed with it)
-    std::vector<cudaEvent_t>& ev = o->host_events;
-    while (ev.size() < (size_t)nchunks * 4) {
-        cudaEvent_t e = nullptr;
-        if (cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) { o->err = "cudaEventCreate failed"; return VSTAB_ERR_CUDA; }
-        ev.push_back(e);
-    }
-    cudaEvent_t* ev_up = ev.data();                 // chunk k uploaded
-    cudaEvent_t* ev_rd = ev.data() + nchunks;       // chunk k rendered
-    cudaEvent_t* ev_dn = ev.data() + 2 * nchunks;   // chunk k downloaded
-    cudaEvent_t* ev_cv = ev.data() + 3 * nchunks;   // staged input: chunk k converted (its staging half is free again)
-    // the accumulated-lock prefix is re-scanned after every chunk over the frames seen so far (a few
-    // thousand 3x3 products): size its buffer once so no reallocation happens while kernels are in flight
-    if (mode == VSTAB_ACCUMULATED_FULL_LOCK) {
-        const size_t mats = (size_t)n_total + (size_t)(n_total / 256 + 2);
-        if (o->acc_capacity < mats) { CK(o->acc.alloc(sizeof(double) * 9 * mats)); o->acc_capacity = mats; }
-    }
-    // Call c presents frame max(0, c - future) and needs transforms up to c - 1 only, so the calls of
-    // chunk k can be rendered as soon as chunk k has been estimated:
-    //   upload(k+1)  ||  estimate(k) -> [prefix scan] -> smooth + warp(k)  ||  download(k-1)
-    for (long k = 0; k < nchunks && st == VSTAB_OK; ++k) {
-        const long f0 = k * B, n = (n_total - f0 < B) ? n_total - f0 : B;
-        const long seen = f0 + n;                                       // frames uploaded and estimated so far
-        const uint8_t* src = frames + (size_t)f0 * frame_stride;
-        uint8_t* stg_in = o->ystage_in.as<uint8_t>() + (size_t)(k & 1) * half_in;
-        if (half_in && k >= 2) cudaStreamWaitEvent(o->copy_in, ev_cv[k - 2], 0);
-        if (frames_in_transfer(g, in_fmt, src, n, clip + (size_t)f0 * g.frame_bytes, stg_in, o->copy_in) != cudaSuccess) {
-            o->err = "upload failed"; st = VSTAB_ERR_CUDA; break;
-        }
-        cudaEventRecord(ev_up[k], o->copy_in);
-        cudaStreamWaitEvent(o->stream, ev_up[k], 0);
-        if (frames_in_convert(g, in_fmt, src, n, clip + (size_t)f0 * g.frame_bytes, stg_in, o->stream) != cudaSuccess) {
-            o->err = "CUDA failure in vstab_offline_run_host"; st = VSTAB_ERR_CUDA; break;
-        }
-        if (half_in) cudaEventRecord(ev_cv[k], o->stream);
-        st = vstab_offline_estimate(o, clip + (size_t)f0 * g.frame_bytes, g.frame_bytes, g.pitch, (int)n, f0,
-                                    f0 > 0 ? clip + (size_t)(f0 - 1) * g.frame_bytes : nullptr, T + (size_t)f0 * 9,
-                                    sums + (size_t)f0 * 3);
-        if (st != VSTAB_OK) break;
-        const bool locked = mode == VSTAB_ACCUMULATED_FULL_LOCK && seen > lock_call - (long)o->F;   // anchor frame is in
-        const int rmode = (mode == VSTAB_ACCUMULATED_FULL_LOCK && !locked) ? VSTAB_GLOBAL_SMOOTHING : mode;
-        if (locked) st = vstab_offline_prepare(o, T, seen, mode, lock_call);
-        if (st != VSTAB_OK) break;
-        uint8_t* ob = o->outbuf.as<uint8_t>() + (size_t)(k & 1) * B * g.frame_bytes;
-        if (k >= 2) cudaStreamWaitEvent(o->stream, ev_dn[k - 2], 0);      // output half is free again
-        st = vstab_offline_render(o, clip, g.frame_bytes, g.pitch, 0, (int)n, f0, T, seen, rmode, lock_call, sums, ob,
-                                  g.frame_bytes, g.pitch);
-        if (st != VSTAB_OK) break;
-        uint8_t* dst = out + (size_t)f0 * out_frame_stride;
-        uint8_t* stg_out = o->ystage_out.as<uint8_t>() + (size_t)(k & 1) * half_out;      // free: ev_dn[k - 2] above
-        if (frames_out_convert(g, out_fmt, ob, n, dst, stg_out, o->stream) != cudaSuccess) {
-            o->err = "CUDA failure in vstab_offline_run_host"; st = VSTAB_ERR_CUDA; break;
-        }
-        cudaEventRecord(ev_rd[k], o->stream);
-        cudaStreamWaitEvent(o->copy_out, ev_rd[k], 0);
-        if (frames_out_transfer(g, out_fmt, ob, n, dst, stg_out, o->copy_out) != cudaSuccess) { o->err = "download failed"; st = VSTAB_ERR_CUDA; }
-        cudaEventRecord(ev_dn[k], o->copy_out);
-    }
-    cudaStreamSynchronize(o->copy_in);
-    cudaStreamSynchronize(o->stream);
-    cudaStreamSynchronize(o->copy_out);
-    if (st == VSTAB_OK && cudaGetLastError() != cudaSuccess) { o->err = "CUDA failure in vstab_offline_run_host"; st = VSTAB_ERR_CUDA; }
-    return st;
+    return offline_prepare(o, d_T_all, n_total, mode, lock_call, o->stream);
 }
 
 extern "C" vstab_status vstab_offline_set_yuv(vstab_offline_t* o, const vstab_yuv_layout* in, const vstab_yuv_layout* out) {
@@ -1877,13 +1785,21 @@ NcclApi g_nccl;
 std::mutex g_nccl_mu;
 constexpr int kNcclUint8 = 1, kNcclDouble = 8;
 
-struct PhaseClock {          // device time of the phases of one vstab_offline_run (events on the instance stream)
-    cudaEvent_t ev[2] = {nullptr, nullptr};
+// Device time of the phases of one vstab_offline_run, and the events that order its streams.  Spans are recorded only when a
+// report is asked for (`on`), and only spans carry timestamps: timed events between the copies of a copy stream left the
+// link idle for ~200 us per 16-frame chunk instead of ~50 (1080p run_host, B200 at 1000 W).
+struct PhaseClock {
+    bool on = false;
     std::vector<std::pair<int, std::pair<cudaEvent_t, cudaEvent_t>>> spans;
     std::vector<cudaEvent_t> pool;
-    cudaEvent_t get() { cudaEvent_t e = nullptr; cudaEventCreate(&e); pool.push_back(e); return e; }
-    void begin(int phase, cudaStream_t q) { cudaEvent_t e = get(); cudaEventRecord(e, q); spans.push_back({phase, {e, nullptr}}); }
-    void end(cudaStream_t q) { cudaEvent_t e = get(); cudaEventRecord(e, q); spans.back().second.second = e; }
+    cudaEvent_t get(bool timed = false) {
+        cudaEvent_t e = nullptr;
+        cudaEventCreateWithFlags(&e, timed ? cudaEventDefault : cudaEventDisableTiming);
+        pool.push_back(e);
+        return e;
+    }
+    void begin(int phase, cudaStream_t q) { if (!on) return; cudaEvent_t e = get(true); cudaEventRecord(e, q); spans.push_back({phase, {e, nullptr}}); }
+    void end(cudaStream_t q) { if (!on) return; cudaEvent_t e = get(true); cudaEventRecord(e, q); spans.back().second.second = e; }
     void collect(float* ms4) {
         for (auto& sp : spans) { float ms = 0.f; if (sp.second.second && cudaEventElapsedTime(&ms, sp.second.first, sp.second.second) == cudaSuccess) ms4[sp.first] += ms; }
     }
@@ -1977,7 +1893,8 @@ extern "C" uint64_t vstab_frame_checksum(const uint8_t* bgr, int rows, int cols,
     return sum;
 }
 
-extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offline_cfg* cfg, vstab_offline_report* rep) {
+// vstab_offline_run as rank `rank` of a world of `world` ranks (the instance's communicator carries the exchange when world > 1)
+static vstab_status offline_job(vstab_offline_t* o, const vstab_offline_cfg* cfg, vstab_offline_report* rep, int world, int rank) {
     if (!o || !cfg || cfg->n_total < 1) return VSTAB_ERR_INVALID_ARGUMENT;
     auto set_err = [&](const std::string& e) { o->err = e; };
     Geometry& g = o->g;
@@ -2005,7 +1922,6 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
         o->err = "lock modes must be set at a call index >= future (SURVEY B.6)"; return VSTAB_ERR_STATE;
     }
     CK(cudaSetDevice(o->device));
-    const int world = o->comm ? o->world : 1, rank = o->comm ? o->rank : 0;
     vstab_shard_plan pl;
     vstab_offline_plan(N, world, rank, o->F, &pl);
     if (!sim && pl.first > 0 && !cfg->host_halo) { o->err = "host source: host_halo (frame first-1) required on ranks > 0"; return VSTAB_ERR_INVALID_ARGUMENT; }
@@ -2015,24 +1931,34 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     const long F = (long)o->F;
     cudaStream_t q = o->stream;
     PhaseClock clock;
+    clock.on = rep != nullptr;
     enum { PH_SOURCE = 0, PH_ESTIMATE = 1, PH_EXCHANGE = 2, PH_RENDER = 3 };
 
-    // ---- buffers: one chunk of frames (+ halo), one chunk of outputs, transforms, sums, checksums -----------------
+    // ---- buffers: one chunk of frames (+ halo), one or two chunks of outputs, transforms, sums, checksums -------------
     // GLOBAL_SMOOTHING from a staged source (simulator, host) is ONE pass: the window of call c reads T[c-P-F+1 .. c-1] and
     // nothing else, so the calls whose windows are complete are warped right behind the estimation, from a ring of the last
     // ceil((F-1)/B) + 3 chunks -- every frame is rendered / uploaded once instead of twice.  The calls whose windows reach
     // into a neighbour's shard (the first P-1 and the last F-1 of a rank in a world > 1) wait for the all-gather as before.
-    const bool fused = !resident && mode == VSTAB_GLOBAL_SMOOTHING;
+    // In a world of one every LK-path mode is one pass: the lock modes read the prefix of the transforms estimated so far
+    // (ACCUMULATED_FULL_LOCK) or nothing at all (TRANSLATION_LOCK / ROTATION_LOCK).
+    const bool fused = !resident && (mode == VSTAB_GLOBAL_SMOOTHING || (world == 1 && !feature_lock));
     vstab_fused_plan fp;
     // with auto-crop the matrices of call c come from the windows of calls c - R .. c: a window of past P + R
     vstab_offline_fused_plan(N, world, rank, o->P + (size_t)o->crop.R, o->F, B, &fp);
     const long ring_chunks = fused ? fp.ring_chunks : 1;
     const long ring_frames = ring_chunks * B;                       // + one slot for the halo frame of the first chunk
+    // outputs for a host sink leave on a download stream of their own, out of two halves of the output chunk (and of the
+    // YUV staging): batch i is warped and converted into half i % 2 while the download of batch i - 1 reads the other one
+    const bool split = cfg->host_out != nullptr;
+    const int halves = split ? 2 : 1;
     DevBuf& chunk = o->job_chunk; DevBuf& outc = o->job_out;
     if (!(resident && direct) && o->job_chunk_frames < (size_t)ring_frames + 1) {
         CK(chunk.alloc(g.frame_bytes * ((size_t)ring_frames + 1) + 64));
-        CK(outc.alloc(g.frame_bytes * (size_t)B + 64));
         o->job_chunk_frames = (size_t)ring_frames + 1;
+    }
+    if (!(resident && direct) && o->job_out_frames < (size_t)B * halves) {
+        CK(outc.alloc(g.frame_bytes * (size_t)B * halves + 64));
+        o->job_out_frames = (size_t)B * halves;
     }
     DevBuf T_local, T_gather, T_all, sums, checks, poses_d, rays_d, tex4_d, reg_local, reg_gather, reg_all;
     CK(T_local.alloc(sizeof(double) * 9 * (size_t)L));
@@ -2044,12 +1970,18 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     CK(cudaMemsetAsync(checks.p, 0, sizeof(unsigned long long) * (size_t)(n_calls > 0 ? n_calls : 1), q));
     uint8_t* cb = chunk.as<uint8_t>();
     const size_t fb = g.frame_bytes;
-    // staging of host YUV frames: one upload staging per stream that fetches frames (q, and qs in the fused pass), one
-    // download staging
-    DevBuf ystage_q, ystage_qs, ystage_o;
-    if (in.staging_bytes(g)) { CK(ystage_q.alloc(in.staging_bytes(g) * (size_t)B)); CK(ystage_qs.alloc(in.staging_bytes(g) * (size_t)B)); }
-    if (out.staging_bytes(g)) CK(ystage_o.alloc(out.staging_bytes(g) * (size_t)B));
-    // resident shard: frame f of the clip lives at dframe(f); no staging
+    // staging of host YUV frames: B frames for the fetches on q, two halves of B frames for the source stream of the fused
+    // pass (chunk k uploads into half k % 2, q converts it before E(k), and S(k+2) waits for E(k)), and one download
+    // staging per output half
+    const size_t istage = in.staging_bytes(g) * (size_t)B, ostage = out.staging_bytes(g) * (size_t)B;
+    if (o->job_stage_bytes < 3 * istage + halves * ostage) {
+        CK(o->job_stage.alloc(3 * istage + halves * ostage));
+        o->job_stage_bytes = 3 * istage + halves * ostage;
+    }
+    uint8_t* const ystage_q = o->job_stage.as<uint8_t>();
+    uint8_t* const ystage_qs = ystage_q + istage;
+    uint8_t* const ystage_o = ystage_qs + 2 * istage;
+    // caller frame f of the clip (host or device memory); a resident shard is read there, with no staging
     auto dframe = [&](long f) -> const uint8_t* { return f == pl.first - 1 ? cfg->host_halo : cfg->host_frames + (size_t)(f - pl.first) * cfg->frame_stride; };
     const size_t src_fs = resident ? cfg->frame_stride : fb, src_step = resident ? cfg->step : g.pitch;
     // simulator: poses of the frames this rank may touch (first-1 .. last-1, the anchor frame), as renderer poses
@@ -2065,8 +1997,9 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
         launch_render_tex4(cfg->d_texture, cfg->tex_rows, cfg->tex_cols, tex4_d.as<unsigned>(), q);
         CK(cudaStreamSynchronize(q));                               // hp goes out of scope
     }
-    // frames [f0, f0 + n) of the clip -> chunk slots [slot, slot + n)
-    auto fetch = [&](long f0, long n, int slot, cudaStream_t q) -> vstab_status {
+    // frames [f0, f0 + n) of the clip -> chunk slots [slot, slot + n) on stream q, caller frames through the staging `stg`;
+    // convert = false leaves the conversion of YUV frames (frames_in_convert) to the caller
+    auto fetch = [&](long f0, long n, int slot, cudaStream_t q, uint8_t* stg, bool convert = true) -> vstab_status {
         if (n <= 0 || resident) return VSTAB_OK;
         clock.begin(PH_SOURCE, q);
         if (sim) {
@@ -2074,13 +2007,13 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
                           cb + (size_t)slot * fb, g.pitch, fb, q, rays_d.as<double>(), tex4_d.as<unsigned>());
         } else {
             if (f0 < pl.first - 1 || f0 + n > pl.last) { o->err = "internal: frame outside the rank's shard"; return VSTAB_ERR_STATE; }
-            uint8_t* stg = (q == o->stream ? ystage_q : ystage_qs).as<uint8_t>();
             for (long i = 0; i < n;) {
                 const long f = f0 + i;
-                const bool halo = f == pl.first - 1;
-                const long m = halo ? 1 : n - i;                    // the halo frame alone, then one contiguous run
-                const uint8_t* src = halo ? cfg->host_halo : cfg->host_frames + (size_t)(f - pl.first) * cfg->frame_stride;
-                CK(frames_in(g, in, src, m, cb + (size_t)(slot + i) * fb, stg, q));
+                const long m = f == pl.first - 1 ? 1 : n - i;      // the halo frame alone, then one contiguous run
+                uint8_t* dst = cb + (size_t)(slot + i) * fb;
+                uint8_t* st = stg + (size_t)i * in.staging_bytes(g);
+                CK(frames_in_transfer(g, in, dframe(f), m, dst, st, q));
+                if (convert) CK(frames_in_convert(g, in, dframe(f), m, dst, st, q));
                 i += m;
             }
         }
@@ -2088,7 +2021,7 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
         CK(cudaGetLastError());
         return VSTAB_OK;
     };
-    cudaEvent_t ev_t0 = clock.get(), ev_t1 = clock.get();
+    cudaEvent_t ev_t0 = clock.get(true), ev_t1 = clock.get(true);
     CK(cudaEventRecord(ev_t0, q));
 
     // ---- ORB / SIFT lock: reference set from the anchor frame, broadcast from its owner --------------------------
@@ -2101,7 +2034,7 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
         DevBuf pack;
         CK(pack.alloc(vstab_offline_reference_bytes()));
         if (rank == owner) {
-            if ((st = fetch(anchor, 1, 0, q)) != VSTAB_OK) return st;
+            if ((st = fetch(anchor, 1, 0, q, ystage_q)) != VSTAB_OK) return st;
             if ((st = vstab_offline_reference_capture(o, resident ? dframe(anchor) : cb, src_step, mode)) != VSTAB_OK) return st;
             if ((st = vstab_offline_reference_export(o, pack.p)) != VSTAB_OK) return st;
         }
@@ -2119,25 +2052,40 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
         CK(cudaMemsetAsync(reg_local.p, 0, sizeof(double) * 10 * (size_t)L, q));
     }
 
-    // warps the calls [c0, c1) (at most B per launch) on stream qw; ring > 0: their presentation frames are in the ring already
-    auto render_calls = [&](long c0, long c1, long ring, cudaStream_t qw) -> vstab_status {
-        for (long c = c0; c < c1; c += B) {
+    if (split && !o->download) CK(cudaStreamCreateWithFlags(&o->download, cudaStreamNonBlocking));
+    cudaEvent_t ev_warped = clock.get(), ev_down[2] = {clock.get(), clock.get()};
+    long batches = 0;                                               // batches warped so far
+    // warps the calls [c0, c1) (at most B per launch) on stream qw, in mode `rmode` over the transforms T_all[0 .. nT);
+    // ring > 0: their presentation frames are in the ring already
+    auto render_calls = [&](long c0, long c1, long ring, int rmode, long nT, cudaStream_t qw) -> vstab_status {
+        for (long c = c0; c < c1; c += B, ++batches) {
             const long n = c1 - c < B ? c1 - c : B;
             const long p_lo = c - F > 0 ? c - F : 0, p_hi = c + n - 1 - F > 0 ? c + n - 1 - F : 0;
             vstab_status s2;
-            if (ring == 0 && (s2 = fetch(p_lo, p_hi - p_lo + 1, 0, qw)) != VSTAB_OK) return s2;
+            if (ring == 0 && (s2 = fetch(p_lo, p_hi - p_lo + 1, 0, qw, ystage_q)) != VSTAB_OK) return s2;
+            const int h = (int)(batches % halves);
+            if (split && batches >= 2) CK(cudaStreamWaitEvent(qw, ev_down[h], 0));   // the download of batch - 2 read half h
+            uint8_t* ob = outc.as<uint8_t>() + (size_t)h * B * fb;
+            uint8_t* stg = ystage_o + (size_t)h * ostage;
             clock.begin(PH_RENDER, qw);
-            uint8_t* dst = direct ? cfg->d_out + (size_t)(c - pl.call_first) * cfg->out_frame_stride : outc.as<uint8_t>();
+            uint8_t* dst = direct ? cfg->d_out + (size_t)(c - pl.call_first) * cfg->out_frame_stride : ob;
             const long base = ring > 0 ? pl.first : p_lo;          // frame held by slot 0 (ring: modulo `ring`)
-            s2 = offline_render_impl(o, resident ? dframe(p_lo) : cb, src_fs, src_step, base, (int)n, c, T_all.as<double>(), N, mode,
+            s2 = offline_render_impl(o, resident ? dframe(p_lo) : cb, src_fs, src_step, base, (int)n, c, T_all.as<double>(), nT, rmode,
                                      cfg->lock_call, sums.as<unsigned long long>() + (size_t)(base - pl.first) * 3, dst,
                                      direct ? cfg->out_frame_stride : fb, direct ? cfg->out_step : g.pitch,
                                      cfg->checksums ? checks.as<unsigned long long>() + (c - pl.call_first) : nullptr, ring, qw);
             clock.end(qw);
             if (s2 != VSTAB_OK) return s2;
-            if (sink && !direct)
-                CK(frames_out(g, out, outc.as<uint8_t>(), n, sink + (size_t)(c - pl.call_first) * cfg->out_frame_stride,
-                              ystage_o.as<uint8_t>(), qw));
+            if (sink && !direct) {
+                uint8_t* to = sink + (size_t)(c - pl.call_first) * cfg->out_frame_stride;
+                CK(frames_out_convert(g, out, ob, n, to, stg, qw));
+                if (split) {
+                    CK(cudaEventRecord(ev_warped, qw));
+                    CK(cudaStreamWaitEvent(o->download, ev_warped, 0));
+                }
+                CK(frames_out_transfer(g, out, ob, n, to, stg, split ? o->download : qw));
+                if (split) CK(cudaEventRecord(ev_down[h], o->download));
+            }
         }
         return VSTAB_OK;
     };
@@ -2157,19 +2105,21 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
         cudaEvent_t evS[kEv], evE[kEv], evW[kEv];
         for (int i = 0; i < kEv; ++i) { evS[i] = clock.get(); evE[i] = clock.get(); evW[i] = clock.get(); }
         CK(cudaMemsetAsync(T_all.p, 0, sizeof(double) * 9 * (size_t)N, q));
+        if (mode == VSTAB_ACCUMULATED_FULL_LOCK && (st = offline_acc_reserve(o, N)) != VSTAB_OK) return st;   // no reallocation in flight
         cudaEvent_t ev_ready = clock.get();                        // the job's buffers are reset (q) before qs / qw touch them
         CK(cudaEventRecord(ev_ready, q));
         CK(cudaStreamWaitEvent(qs, ev_ready, 0));
         CK(cudaStreamWaitEvent(qw, ev_ready, 0));
         c_head = c_tail = fp.fused_first;
         const long nchunks = (n_local + B - 1) / B;
+        auto stg_qs = [&](long k) { return ystage_qs + (size_t)(k % 2) * istage; };
         auto source = [&](long k) -> vstab_status {               // S(k)
             const long f0 = pl.first + k * B, n = pl.last - f0 < B ? pl.last - f0 : B;
             if (k >= 3) CK(cudaStreamWaitEvent(qs, evW[(k - 3) % kEv], 0));
             if (k >= 2) CK(cudaStreamWaitEvent(qs, evE[(k - 2) % kEv], 0));
             vstab_status s2;
-            if (k == 0 && f0 > 0 && (s2 = fetch(f0 - 1, 1, (int)ring_frames, qs)) != VSTAB_OK) return s2;
-            if ((s2 = fetch(f0, n, (int)((k % ring_chunks) * B), qs)) != VSTAB_OK) return s2;
+            if (k == 0 && f0 > 0 && (s2 = fetch(f0 - 1, 1, (int)ring_frames, qs, stg_qs(k))) != VSTAB_OK) return s2;
+            if ((s2 = fetch(f0, n, (int)((k % ring_chunks) * B), qs, stg_qs(k), false)) != VSTAB_OK) return s2;
             CK(cudaEventRecord(evS[k % kEv], qs));
             return VSTAB_OK;
         };
@@ -2182,6 +2132,11 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
             if (k == 0) { if (f0 > 0) hl = cb + (size_t)ring_frames * fb; }
             else hl = cb + (size_t)(((k - 1) % ring_chunks) * B + B - 1) * fb;      // the previous chunk's last frame, still in the ring
             CK(cudaStreamWaitEvent(q, evS[k % kEv], 0));
+            if (in.yuv) {                                           // YUV frames staged (or left in place) by S(k)
+                clock.begin(PH_SOURCE, q);
+                CK(frames_in_convert(g, in, dframe(f0), n, cb + (size_t)slot0 * fb, stg_qs(k), q));
+                clock.end(q);
+            }
             clock.begin(PH_ESTIMATE, q);
             st = vstab_offline_estimate(o, cb + (size_t)slot0 * fb, src_fs, src_step, (int)n, f0, hl, T_all.as<double>() + (size_t)f0 * 9,
                                         sums.as<unsigned long long>() + (size_t)(f0 - pl.first) * 3);
@@ -2189,13 +2144,22 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
             if (st != VSTAB_OK) return st;
             CK(cudaEventRecord(evE[k % kEv], q));
             if (k + 2 < nchunks && (st = source(k + 2)) != VSTAB_OK) return st;
-            // W(k): call c reads transforms up to T[c - 1]
+            // W(k): call c reads transforms up to T[c - 1] and presents frame c - F (future 0: T[c] and frame c)
             CK(cudaStreamWaitEvent(qw, evE[k % kEv], 0));
-            const long c_ok = f0 + n + 1 < fp.fused_last ? f0 + n + 1 : fp.fused_last;
+            const long c_end = f0 + n + (F > 0 ? 1 : 0);
+            const long c_ok = c_end < fp.fused_last ? c_end : fp.fused_last;
             if (c_ok > c_tail) {
                 const long p_lo = c_tail - F > 0 ? c_tail - F : 0;
                 if (p_lo < pl.first || p_lo - pl.first < (k - (ring_chunks - 3)) * B) { o->err = "internal: presentation frame left the ring"; return VSTAB_ERR_STATE; }
-                if ((st = render_calls(c_tail, c_ok, ring_frames, qw)) != VSTAB_OK) return st;
+                // ACCUMULATED_FULL_LOCK (world of one): the prefix over the frames estimated so far, rescanned on qw because
+                // W(k-1) reads the one it replaces; until the anchor frame is in, every call is before the lock call
+                int rmode = mode;
+                const long seen = f0 + n, nT = mode == VSTAB_ACCUMULATED_FULL_LOCK ? seen : N;
+                if (mode == VSTAB_ACCUMULATED_FULL_LOCK) {
+                    if (seen <= cfg->lock_call - F) rmode = VSTAB_GLOBAL_SMOOTHING;
+                    else if ((st = offline_prepare(o, T_all.as<double>(), seen, mode, cfg->lock_call, qw)) != VSTAB_OK) return st;
+                }
+                if ((st = render_calls(c_tail, c_ok, ring_frames, rmode, nT, qw)) != VSTAB_OK) return st;
                 c_tail = c_ok;
             }
             CK(cudaEventRecord(evW[k % kEv], qw));
@@ -2211,12 +2175,12 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
         const long n = pl.last - f0 < B ? pl.last - f0 : B;
         if (!resident) {
             if (f0 == pl.first) {
-                if (f0 > 0 && (st = fetch(f0 - 1, 1, 0, q)) != VSTAB_OK) return st;     // halo frame
+                if (f0 > 0 && (st = fetch(f0 - 1, 1, 0, q, ystage_q)) != VSTAB_OK) return st;     // halo frame
             } else {
                 // the last frame of the previous chunk is this chunk's halo
                 CK(cudaMemcpyAsync(cb, cb + (size_t)B * fb, fb, cudaMemcpyDeviceToDevice, q));
             }
-            if ((st = fetch(f0, n, 1, q)) != VSTAB_OK) return st;
+            if ((st = fetch(f0, n, 1, q, ystage_q)) != VSTAB_OK) return st;
         }
         const uint8_t* fr = resident ? dframe(f0) : cb + fb;
         const uint8_t* hl = f0 > 0 ? (resident ? dframe(f0 - 1) : cb) : nullptr;
@@ -2252,12 +2216,14 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
         if ((st = gather(reg_local, reg_gather, reg_all, 10)) != VSTAB_OK) return st;
         if ((st = vstab_offline_set_registrations(o, reg_all.as<double>(), N)) != VSTAB_OK) return st;
     }
-    if ((st = vstab_offline_prepare(o, T_all.as<double>(), N, mode, cfg->lock_call)) != VSTAB_OK) return st;
+    const bool pass2 = c_head > pl.call_first || c_tail < pl.call_last;
+    if (pass2 && (st = offline_prepare(o, T_all.as<double>(), N, mode, cfg->lock_call, q)) != VSTAB_OK) return st;
     clock.end(q);
 
     // ---- pass 2: the calls whose presentation frame this rank owns (all of them, or what the fused pass left) ----------
-    if ((st = render_calls(pl.call_first, c_head, 0, q)) != VSTAB_OK) return st;
-    if ((st = render_calls(c_tail, pl.call_last, 0, q)) != VSTAB_OK) return st;
+    if ((st = render_calls(pl.call_first, c_head, 0, mode, N, q)) != VSTAB_OK) return st;
+    if ((st = render_calls(c_tail, pl.call_last, 0, mode, N, q)) != VSTAB_OK) return st;
+    if (split && batches > 0) CK(cudaStreamWaitEvent(q, ev_down[(batches - 1) % 2], 0));
     if (cfg->checksums && n_calls > 0)
         CK(cudaMemcpyAsync(cfg->checksums, checks.p, sizeof(unsigned long long) * (size_t)n_calls, cudaMemcpyDeviceToHost, q));
     if (cfg->T_all) CK(cudaMemcpyAsync(cfg->T_all, T_all.p, sizeof(double) * 9 * (size_t)N, cudaMemcpyDeviceToHost, q));
@@ -2275,6 +2241,23 @@ extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offlin
     }
     CK(cudaGetLastError());
     return VSTAB_OK;
+}
+
+extern "C" vstab_status vstab_offline_run(vstab_offline_t* o, const vstab_offline_cfg* cfg, vstab_offline_report* rep) {
+    if (!o) return VSTAB_ERR_INVALID_ARGUMENT;
+    return offline_job(o, cfg, rep, o->comm ? o->world : 1, o->comm ? o->rank : 0);
+}
+
+// the job of vstab_offline_run in a world of one (whatever communicator the instance has joined), host frames in and out
+extern "C" vstab_status vstab_offline_run_host(vstab_offline_t* o, const uint8_t* frames, size_t frame_stride, size_t step,
+                                                long n_total, int mode, long lock_call, uint8_t* out,
+                                                size_t out_frame_stride, size_t out_step) {
+    if (!o || !frames || !out || n_total < 1) return VSTAB_ERR_INVALID_ARGUMENT;
+    vstab_offline_cfg cfg{};
+    cfg.n_total = n_total; cfg.mode = mode; cfg.lock_call = lock_call; cfg.source = VSTAB_SRC_HOST;
+    cfg.host_frames = frames; cfg.frame_stride = frame_stride; cfg.step = step;
+    cfg.host_out = out; cfg.out_frame_stride = out_frame_stride; cfg.out_step = out_step;
+    return offline_job(o, &cfg, nullptr, 1, 0);
 }
 
 // =====================================================================================
